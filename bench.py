@@ -86,6 +86,42 @@ def load_peaks():
     return {"hbm": 6650.0, "tc_burst": 1590.0, "tc_sustained": 1400.0, "src": "fallback"}
 
 
+DUMP_BYTES = 60 << 20            # --dump-outputs: data bytes of all files together (< 64 MB with the .npy headers)
+
+
+def _flat_outputs(outputs, prefix=""):
+    for k, v in outputs.items():
+        if isinstance(v, dict):
+            yield from _flat_outputs(v, f"{prefix}{k}.")
+        else:
+            yield prefix + k, v
+
+
+def dump_outputs(path, outputs, budget=DUMP_BYTES, seed=0):
+    """Write every tensor of `outputs` (nested dicts: names joined by '.') as `path/<name>.npy`: float64 for float64 and
+    integer tensors (exact), float32 otherwise.  Within `budget` bytes in all: the smaller arrays are written whole, and
+    each array above the byte cap that leaves becomes a 1-D sample of its flattened elements at sorted indices drawn
+    with `seed`, the same indices on every run (and for every array of the same size), so that the files of two builds
+    compare element for element."""
+    import numpy as np
+    arrays = [(n, t.detach(), np.float64 if t.dtype == torch.float64 or not t.is_floating_point() else np.float32)
+              for n, t in _flat_outputs(outputs)]
+    sizes = sorted(t.numel() * np.dtype(d).itemsize for _, t, d in arrays)
+    cap, left = None, budget
+    for i, s in enumerate(sizes):
+        if s * (len(sizes) - i) > left:
+            cap = left // (len(sizes) - i)
+            break
+        left -= s
+    os.makedirs(path, exist_ok=True)
+    for name, t, dtype in arrays:
+        keep = t.numel() if cap is None else min(t.numel(), cap // np.dtype(dtype).itemsize)
+        if keep < t.numel():
+            idx = np.sort(np.random.default_rng(seed).choice(t.numel(), keep, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(path, name + ".npy"), t.cpu().numpy().astype(dtype))
+
+
 def synth_latents(B, h, w, seed=1234, pin=False):
     """SURVEY §8d 'direct' synthetic inputs: y = 4 randn, latents = randn."""
     g = torch.Generator().manual_seed(seed)
@@ -401,35 +437,37 @@ def run_training(args):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            out = fn()
         e1.record()
         torch.cuda.synchronize()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         barrier()
-        return float(ms) / steps
+        return float(ms) / steps, out
 
     sampler = ClockSampler(local) if rank == 0 and not args.no_clock_sampler else None
     for _ in range(max(args.warmup, 3)):
         step()
     if sampler:
         sampler.mark()
-    ms_step = timed(lambda: step(copy=False), args.steps)          # inputs resident
+    ms_step, loss = timed(lambda: step(copy=False), args.steps)    # inputs resident
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"loss": loss, "params": dict(model.named_parameters())})
     launches = model.engine[0].last_launches
     t0 = time.perf_counter()
     barrier()
-    ms_e2e = timed(step, args.steps)                               # H2D of the batch + D2H of the loss inside
+    ms_e2e, _ = timed(step, args.steps)                            # H2D of the batch + D2H of the loss inside
     loss_value = float(host_loss[0])
-    ms_nosync = timed(lambda: step(sync=False, copy=False), args.steps) if world > 1 else ms_step
+    ms_nosync = timed(lambda: step(sync=False, copy=False), args.steps)[0] if world > 1 else ms_step
     # the gradient all-reduce alone: one flat fp32 buffer of all hot-path gradients
     ar_ms = None
     if world > 1:
         flat = torch.zeros(n_params, device=dev)
         for _ in range(3):
             dist.all_reduce(flat)
-        ar_ms = timed(lambda: dist.all_reduce(flat), 10)
+        ar_ms = timed(lambda: dist.all_reduce(flat), 10)[0]
         del flat
     # where the step goes on one rank: forward (kernels), backward (recompute + autograd), optimizer + repack
     def phase_times():
@@ -579,14 +617,14 @@ def run_codec(args):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            out = fn()
         e1.record()
         torch.cuda.synchronize()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         barrier()
-        return float(ms) / steps
+        return float(ms) / steps, out
 
     sampler = ClockSampler(local) if rank == 0 and not args.no_clock_sampler else None
     warm = max(args.warmup, 3)
@@ -598,9 +636,12 @@ def run_codec(args):
         n_warm += 1
     if sampler:
         sampler.mark()
-    ms_step = timed(step_resident, args.steps)
+    ms_step, out = timed(step_resident, args.steps)
     clocks = sampler.stop() if sampler else None
-    ms_e2e = timed(step_e2e, args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)
+    del out                                     # held, it would make the first e2e step allocate a second output set
+    ms_e2e, _ = timed(step_e2e, args.steps)
 
     # launches of one step: the library's counter restarts when the slice loop loads its inputs, so read it on both sides
     torch.cuda.synchronize()
@@ -716,7 +757,15 @@ def main():
     ap.add_argument("--no-clock-sampler", action="store_true", help="diagnostic: do not poll NVML during the timed region")
     ap.add_argument("--gc-micro-mb", type=int, default=1024, help="footprint of the kernel-3 HBM microbenchmark")
     ap.add_argument("--no-whole-codec", action="store_true", help="skip the secondary whole-model figure of the default line")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed on rank 0 (the outputs; for --config 4 the loss "
+                         "and the updated parameters) as DIR/<name>.npy, float32 / float64, under 64 MB in all: a larger "
+                         "array becomes a fixed seeded sample (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what this library computes: not with --impl reference")
     if args.mode:
         CONFIGS[args.config] = dict(CONFIGS[args.config], mode=args.mode)
     if args.impl == "reference":
@@ -809,6 +858,8 @@ def main():
         sampler.mark()
     ms_step, out = timed(step_resident, args.steps)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)
     launches = eng.last_launches
     run_e2e(3)
     barrier()
