@@ -68,9 +68,10 @@ __global__ void __launch_bounds__(256) gelu_kernel(const float* __restrict__ x, 
 // Each thread owns 4 channels of DX horizontally adjacent tokens: a 3 x (DX + 2) input patch is read
 // once (4.5 float4 loads per output at DX = 4 instead of 9), consecutive threads take consecutive channel
 // groups so every load/store is a coalesced 16-byte access.  DX = 4 (72 registers) measured 8 % / 23 % faster than
-// DX = 8 (104 registers, 25 % occupancy) on the 640- / 1280-channel GLU launch, DX = 2 slower again (DCAE_DW_X).
+// DX = 8 (104 registers, 25 % occupancy) on the 640- / 1280-channel GLU launch, DX = 2 slower again.
 // ---------------------------------------------------------------------------------------------
-constexpr int DW_ROWS = 4;      // token rows per block; the tokens per thread (DX) are a template parameter: 4 by default, DCAE_DW_X = 2 / 8 for A/B
+constexpr int DW_ROWS = 4;      // token rows per block
+constexpr int DX = 4;           // tokens per thread
 
 // grid = (ceil(C4 / 32), ceil(h / DW_ROWS), B * ceil(w / DX)); block = 32 channel groups x DW_ROWS token rows, so the
 // three input rows a thread needs are shared with its neighbours in the block through L1.
@@ -79,7 +80,7 @@ constexpr int DW_ROWS = 4;      // token rows per block; the tokens per thread (
 // All element offsets are 32-bit (the host checks that every tensor spans < 2^32 elements): one IMAD per access and one
 // IMAD.WIDE onto the 64-bit base, instead of the 64-bit multiply chains that made integer work 45 % of the kernel
 // (round 1: 69 instructions per output element, 16 of them FFMA).
-template <int ACT, int DX>
+template <int ACT>
 __global__ void __launch_bounds__(32 * DW_ROWS) dwconv3x3_kernel(const float* __restrict__ x, uint32_t x_ld,
                                                         const float* __restrict__ wt, const float* __restrict__ bias,
                                                         int C4, int B, int h, int w,
@@ -398,15 +399,12 @@ extern "C" int dcae_op_dwconv3x3(const float* x, int64_t x_ld, const float* wt, 
     DCAE_REQUIRE(T * x_ld < lim && T * out_ld < lim && T * gate_ld < lim && T * o16.ld < lim && x_ld < lim && out_ld < lim && gate_ld < lim,
                  "dcae_op_dwconv3x3: tensors of 2^32 elements or more are not supported (32-bit offsets)");
   }
-  static const int dw_x = [] { const char* v = getenv("DCAE_DW_X"); const int x = v ? atoi(v) : 4; return (x == 2 || x == 4 || x == 8) ? x : 4; }();
-  const int xg = (w + dw_x - 1) / dw_x;
+  const int xg = (w + DX - 1) / DX;
   DCAE_REQUIRE((int64_t)B * xg <= 65535 && (h + DW_ROWS - 1) / DW_ROWS <= 65535, "dcae_op_dwconv3x3: token grid too large");
   dim3 grid((unsigned)((C / 4 + 31) / 32), (unsigned)((h + DW_ROWS - 1) / DW_ROWS), (unsigned)(B * xg));
   const int variant = act == DCAE_ACT_NONE ? 0 : (out == nullptr ? 2 : 1);
-#define DW_LAUNCH(A, X) dwconv3x3_kernel<A, X><<<grid, 32 * DW_ROWS, 0, (cudaStream_t)stream>>>(x, (uint32_t)x_ld, wt, bias, C / 4, B, h, w, gate, (uint32_t)gate_ld, out, (uint32_t)out_ld, o16)
-  if (dw_x == 4) { if (variant == 0) DW_LAUNCH(0, 4); else if (variant == 1) DW_LAUNCH(1, 4); else DW_LAUNCH(2, 4); }
-  else if (dw_x == 2) { if (variant == 0) DW_LAUNCH(0, 2); else if (variant == 1) DW_LAUNCH(1, 2); else DW_LAUNCH(2, 2); }
-  else { if (variant == 0) DW_LAUNCH(0, 8); else if (variant == 1) DW_LAUNCH(1, 8); else DW_LAUNCH(2, 8); }
+#define DW_LAUNCH(A) dwconv3x3_kernel<A><<<grid, 32 * DW_ROWS, 0, (cudaStream_t)stream>>>(x, (uint32_t)x_ld, wt, bias, C / 4, B, h, w, gate, (uint32_t)gate_ld, out, (uint32_t)out_ld, o16)
+  if (variant == 0) DW_LAUNCH(0); else if (variant == 1) DW_LAUNCH(1); else DW_LAUNCH(2);
 #undef DW_LAUNCH
   DCAE_LAUNCH_CHECK();
   return DCAE_OK;

@@ -18,8 +18,6 @@
 // Every mbarrier wait is bounded: a protocol bug traps instead of hanging the GPU.
 #include <cuda.h>
 
-#include <stdlib.h>
-
 #include <mutex>
 
 #include "common.cuh"
@@ -49,17 +47,9 @@ struct TcParams {
   int taps;
   int B, h, w, TH, TW, tw_shift, tiles_x, tiles_y;
   int BN, stages, tmem_cols;
-  int n_tiles_n, total_tiles, chunk_kb, dbg_epi;
-  int dbg_nosplit, dbg_nostore;   // tuning experiments only (env DCAE_TC_NOSPLIT / DCAE_TC_NOSTORE): wrong results
+  int n_tiles_n, total_tiles, chunk_kb;
   uint32_t stage_bytes, b_bytes;
 };
-
-__device__ __forceinline__ float act_apply(float v, int act) {
-  if (act == DCAE_ACT_GELU) return gelu_erf(v);
-  if (act == DCAE_ACT_HALF_TANH) return 0.5f * tanhf(v);
-  if (act == DCAE_ACT_RELU) return fmaxf(v, 0.f);
-  return v;
-}
 
 // Persistent kernel: grid = min(#tiles, #SMs); each CTA walks tiles t = blockIdx.x + i * gridDim.x in
 // (token-tile major, n-tile minor) order so that CTAs running together share A tiles through L2.
@@ -168,7 +158,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
           const uint32_t tmem_acc = tmem_base + buf * (uint32_t)p.BN;
           const int kb_end = min(p.KB, (ck + 1) * p.chunk_kb);
           for (int kb = ck * p.chunk_kb; kb < kb_end; ++kb) {
-            mbar_wait(smem_u32((PASSES == 3 && !p.dbg_nosplit) ? &ready_bar[stage] : &full_bar[stage]), phase);
+            mbar_wait(smem_u32(PASSES == 3 ? &ready_bar[stage] : &full_bar[stage]), phase);
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
             const uint32_t sbase = smem0 + stage * p.stage_bytes;
             const uint32_t first = (kb == ck * p.chunk_kb) ? 0u : 1u;
@@ -200,7 +190,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
     }
   } else if (warp < 8) {
     asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(REGS_SPLIT));
-    if (PASSES == 3 && !p.dbg_nosplit) {
+    if (PASSES == 3) {
       // ===================== split warps: a -> (a_hi in place, a_lo) =====================
       const int st = threadIdx.x - 128;   // 0..127
       int stage = 0;
@@ -235,7 +225,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
     for (int t = blockIdx.x; t < p.total_tiles; t += gridDim.x) {
       EpiTile et;
       tile_coords(t, et.b, et.y0, et.x0, et.n0);
-      et.B = p.B; et.h = p.h; et.w = p.w; et.tw_shift = p.tw_shift; et.N = p.N; et.BN = p.BN; et.dbg = p.dbg_epi;
+      et.B = p.B; et.h = p.h; et.w = p.w; et.tw_shift = p.tw_shift; et.N = p.N; et.BN = p.BN;
       float acc[EPI_BLOCKS * 32];
       for (int ck = 0; ck < n_chunks; ++ck, ++gchunk) {
         const uint32_t buf = gchunk & 1;
@@ -246,7 +236,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
         mbar_arrive(smem_u32(&tmem_empty_bar[buf]));   // the MMA warp may start the next chain in this buffer
       }
       // ---- epilogue of this tile (overlaps the next tile's mainloop) ----
-      if (!p.dbg_nostore) epilogue_store(acc, p.e, et, quarter, half, lane);
+      epilogue_store(acc, p.e, et, quarter, half, lane);
     }
   }
 
@@ -272,10 +262,6 @@ void pick_tile(int h, int w, int* TH, int* TW) {
 }
 
 int pick_bn(int N) {
-  if (const char* env = getenv("DCAE_TC_BN")) {   // tuning override (tools/gemm_bench.py)
-    const int bn = atoi(env);
-    if (bn >= 32 && bn <= 256 && bn % 32 == 0 && N % bn == 0) return bn;
-  }
   for (int bn = 256; bn >= 32; bn -= 32)
     if (N % bn == 0) return bn;
   return 0;
@@ -289,16 +275,11 @@ int gemm_tcgen05(const dcae_operand* a, const dcae_weight* w, const dcae_epilogu
   DCAE_REQUIRE(e->act_cols <= 0 || e->act_cols >= w->N || e->act_cols % 32 == 0, "gemm(tcgen05): act_cols must be a multiple of 32");
   const int64_t T = (int64_t)a->B * a->h * a->w;
   if (T == 0) return DCAE_OK;
-  {
-    // thread-block-pair kernel (gemm_tcgen05_2cta.cu); DCAE_TC_2CTA=0 forces the single-CTA kernel below
-    // Measured (profiles/r01/gemm_ab_v3.jsonl): the pair kernel wins on long-K 3-pass layers (cc1: K = 8640..10944,
-    // +8 %) and loses on short K, where the extra cross-CTA handshakes are not amortised.  -1 = that heuristic.
-    static const int pair_mode = [] { const char* v = getenv("DCAE_TC_2CTA"); return v ? atoi(v) : -1; }();
-    const bool use_pair = pair_mode == 1 || (pair_mode == -1 && passes == 3 && w->K >= 4096);
-    if (use_pair) {
-      const int rc = gemm_tcgen05_2cta(a, w, e, passes, pick_bn(w->N), s);
-      if (rc != 1) return rc;
-    }
+  // thread-block-pair kernel (gemm_tcgen05_2cta.cu).  Measured (profiles/r01/gemm_ab_v3.jsonl): it wins on long-K
+  // 3-pass layers (cc1: K = 8640..10944, +8 %) and loses on short K, where the extra cross-CTA handshakes are not amortised.
+  if (passes == 3 && w->K >= 4096) {
+    const int rc = gemm_tcgen05_2cta(a, w, e, passes, pick_bn(w->N), s);
+    if (rc != 1) return rc;
   }
   TcParams p;
   p.e = *e;
@@ -323,11 +304,6 @@ int gemm_tcgen05(const dcae_operand* a, const dcae_weight* w, const dcae_epilogu
   p.stage_bytes = (passes == 3) ? (2 * A_BYTES + 2 * p.b_bytes) : (A_BYTES + p.b_bytes);
   p.stages = (int)((SMEM_LIMIT - 2048) / p.stage_bytes);
   if (p.stages > MAX_STAGES) p.stages = MAX_STAGES;
-  if (const char* env = getenv("DCAE_TC_STAGES")) { const int v = atoi(env); if (v >= 1 && v < p.stages) p.stages = v; }
-  p.dbg_nosplit = getenv("DCAE_TC_NOSPLIT") != nullptr;
-  p.dbg_nostore = getenv("DCAE_TC_NOSTORE") != nullptr;
-  if (const char* env = getenv("DCAE_TC_CHUNK")) { const int v = atoi(env); if (v >= 1) p.chunk_kb = v; }
-  p.dbg_epi = getenv("DCAE_TC_EPI") ? atoi(getenv("DCAE_TC_EPI")) : 0;
   if (p.stages > p.KB) p.stages = p.KB;
   DCAE_REQUIRE(p.stages >= 1, "gemm(tcgen05): tile does not fit in shared memory");
   const size_t smem = (size_t)p.stages * p.stage_bytes + 1024;

@@ -14,8 +14,6 @@
 // Barriers (S stages): a_full[S] local (x3: the CTA's own A tile landed), b_full[S] in the leader (weights of
 // both CTAs; x1: A tiles too), ready[S] in the leader (256 split threads of both CTAs), empty[S] and
 // tmem_full[2] in both CTAs (multicast tcgen05.commit), tmem_empty[2] in the leader (512 drain threads).
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "tc_common.cuh"
 
@@ -36,16 +34,9 @@ struct Tc2Params {
   int N, KB, cblk_per_tap, col0, k0, col1, taps;
   int B, h, w, TH, TW, tw_shift, tiles_x, tiles_y;
   int BN, stages, tmem_cols;
-  int n_tiles_n, m_tiles, total_pair_tiles, chunk_kb, dbg_epi;
+  int n_tiles_n, m_tiles, total_pair_tiles, chunk_kb;
   uint32_t stage_bytes, bh_bytes;   // bh_bytes = (BN/2) rows x 128 B: this CTA's half of a weight tile
 };
-
-__device__ __forceinline__ float act2(float v, int act) {
-  if (act == DCAE_ACT_GELU) return gelu_erf(v);
-  if (act == DCAE_ACT_HALF_TANH) return 0.5f * tanhf(v);
-  if (act == DCAE_ACT_RELU) return fmaxf(v, 0.f);
-  return v;
-}
 
 // wait with cluster-scope acquire: the data guarded by the barrier was written by the peer CTA
 __device__ __forceinline__ void mbar_wait_cluster(uint32_t bar, uint32_t parity) {
@@ -246,7 +237,7 @@ gemm_tcgen05_2cta_kernel(const __grid_constant__ CUtensorMap map_a, const __grid
     for (int pt = pair; pt < p.total_pair_tiles; pt += npairs) {
       EpiTile et;
       tile_coords(pt, et.b, et.y0, et.x0, et.n0);
-      et.B = p.B; et.h = p.h; et.w = p.w; et.tw_shift = p.tw_shift; et.N = p.N; et.BN = p.BN; et.dbg = p.dbg_epi;
+      et.B = p.B; et.h = p.h; et.w = p.w; et.tw_shift = p.tw_shift; et.N = p.N; et.BN = p.BN;
       float acc[EPI_BLOCKS * 32];
       for (int ck = 0; ck < n_chunks; ++ck, ++gchunk) {
         const uint32_t buf = gchunk & 1;
@@ -303,13 +294,10 @@ int gemm_tcgen05_2cta(const dcae_operand* a, const dcae_weight* w, const dcae_ep
   p.n_tiles_n = w->N / p.BN;
   p.total_pair_tiles = p.n_tiles_n * ((p.m_tiles + 1) / 2);
   p.chunk_kb = (passes == 3) ? CHUNK_MMAS / 12 : p.KB;
-  if (const char* env = getenv("DCAE_TC_CHUNK")) { const int v = atoi(env); if (v >= 1) p.chunk_kb = v; }
-  p.dbg_epi = getenv("DCAE_TC_EPI") ? atoi(getenv("DCAE_TC_EPI")) : 0;
   p.bh_bytes = (uint32_t)(p.BN / 2) * BK * 4;
   p.stage_bytes = (passes == 3) ? (2 * A_BYTES + 2 * p.bh_bytes) : (A_BYTES + p.bh_bytes);
   p.stages = (int)((SMEM_LIMIT - 2048) / p.stage_bytes);
   if (p.stages > MAX_STAGES) p.stages = MAX_STAGES;
-  if (const char* env = getenv("DCAE_TC_STAGES")) { const int v = atoi(env); if (v >= 1 && v < p.stages) p.stages = v; }
   if (p.stages > p.KB) p.stages = p.KB;
   const size_t smem = (size_t)p.stages * p.stage_bytes + 1024;
 

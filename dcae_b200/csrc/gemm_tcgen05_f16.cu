@@ -49,9 +49,7 @@ struct F16Params {
   int BN, stages, tmem_cols;
   int n_tiles_n, total_tiles, chunk_kb;
   float descale;
-  int dbg_nostore;
   int has_o32, has_o16, has_o16a;
-  int pdl;                   // launched with programmatic stream serialization: see griddepcontrol below
   int fuse_b;                // single CTA, BN <= 128: one N = 2 BN MMA covers a_hi x [b_hi; b_lo], see the MMA issuer
   int passes;                // 3 = hi/lo error-compensated (fp32-level accuracy); 1 = DCAE_MATH_F16: a_hi x b_hi only, lo planes never loaded
   uint32_t stage_bytes, b_bytes;
@@ -315,15 +313,6 @@ __device__ __forceinline__ void gemm_f16x3_body(const CUtensorMap& map_ah, const
   if (PAIR) cluster_sync_all();     // the peer's barriers exist before anything signals them
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
   const uint32_t tmem_base = tmem_base_slot;
-  // Programmatic dependent launch: this grid may have become resident while the previous kernel of the stream was
-  // still draining (its CTAs leave one by one: 8-10 us of exit skew); barrier init, TMEM allocation and the
-  // tensor-map prefetch above overlapped with that tail.  Nothing before this line touches global memory a
-  // predecessor writes; from here on the predecessor has completed and its writes are visible.  Our own successor
-  // may be scheduled as soon as every CTA has passed this point.
-  if (p.pdl) {
-    asm volatile("griddepcontrol.wait;" ::: "memory");
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-  }
 
   // per-stage smem: [A_hi | A_lo | B_hi | B_lo] (single pass: [A_hi | B_hi]); the two epilogue staging buffers follow the stages
   const uint32_t off_al = A16_BYTES, off_bh = (p.passes == 3 ? 2 : 1) * A16_BYTES, off_bl = off_bh + p.b_bytes;
@@ -460,7 +449,7 @@ __device__ __forceinline__ void gemm_f16x3_body(const CUtensorMap& map_ah, const
     for (int t = unit; t < p.total_tiles; t += nunits) {
       EpiTile et;
       tile_coords(t, et.b, et.y0, et.x0, et.n0);
-      et.B = p.B; et.h = p.h; et.w = p.w; et.tw_shift = p.tw_shift; et.N = p.N; et.BN = p.BN; et.dbg = 0;
+      et.B = p.B; et.h = p.h; et.w = p.w; et.tw_shift = p.tw_shift; et.N = p.N; et.BN = p.BN;
       float acc[NB * 32];
       float bias_l[NB], rs_l[NB];          // column (block g, lane) of bias / res_scale, see finalize_block
 #pragma unroll
@@ -482,7 +471,6 @@ __device__ __forceinline__ void gemm_f16x3_body(const CUtensorMap& map_ah, const
         if (DBG) t_drain += clock64() - td0;
       }
       const long long te0 = DBG ? clock64() : 0;
-      if (p.dbg_nostore) continue;
       // ---- epilogue: registers -> swizzled staging -> TMA tensor store, one 32-column block at a time ----
       // A ROLLED loop with one copy of the body.  Fully unrolled (4 blocks x 3 activations x 3 outputs) the kernel was
       // 350 KB of straight-line SASS that each warp runs once per tile: instruction fetch, not arithmetic, set the
@@ -661,35 +649,27 @@ int gemm_tcgen05_f16x3(const dcae_operand* a, const dcae_weight* w, const dcae_e
   p.tiles_x = (a->w + p.TW - 1) / p.TW;
   p.tiles_y = (a->h + p.TH - 1) / p.TH;
   const int m_tiles = p.tiles_x * p.tiles_y * a->B;
-  // thread-block pairs (cta_group::2): DCAE_F16_PAIR = 1 / 0 forces it on / off, default = heuristic below
-  static const int pair_mode = [] { const char* v = getenv("DCAE_F16_PAIR"); return v ? atoi(v) : -1; }();
-  static const int fuse_mode = [] { const char* v = getenv("DCAE_F16_FUSEB"); return v ? atoi(v) : 1; }();
   // A/B sweeps (profiles/r01/gemm_f16_pair_ab.jsonl, layer_times_bn_pair_sweep3.log): pairs win where the mainloop is
   // long or wide (cc1, proj, fc1, the K = 2 016 conv layers); everything else runs single-CTA with BN <= 128 so that
   // the fused [b_hi; b_lo] MMA applies (N = 320 -> 128 + 128 + 64 ragged beats 2 x 160 by 20 %, N = 224 likewise).
   // single pass: the mainloop moves a third of the flops per operand byte less... per k-block a 128 x 128 tile is 256 tensor
   // cycles against 32 KB of operands (128 B/clk, twice what the L2 -> SM path feeds), so every layer that can takes
   // M = 256 pairs with the widest N tile (each CTA loads half of the weight rows: 62 B/clk at BN = 256)
-  const bool pair_heur = passes == 1 ? w->N >= 128 : ((int64_t)a->taps * Kp >= 2048 || w->N >= 2048);
   // The arithmetic (fused or three-MMA accumulation order) follows want_pair, a function of the layer shape only, so
   // that a result never depends on the batch size (a 1-tile problem cannot pair but keeps the pair path's order).
-  const bool want_pair = pair_mode == 1 || (pair_mode == -1 && pair_heur);
+  const bool want_pair = passes == 1 ? w->N >= 128 : ((int64_t)a->taps * Kp >= 2048 || w->N >= 2048);
   const bool pair = want_pair && m_tiles >= 2;
   p.BN = 0;
-  if (const char* env = getenv("DCAE_TC_BN")) {        // tuning override; BN need not divide N (ragged last tile)
-    const int bn = atoi(env);
-    if (bn >= 32 && bn <= 256 && bn % 32 == 0) p.BN = bn;
-  }
   p.passes = passes;
-  if (p.BN == 0 && passes == 1 && want_pair) {     // least padded work, then the widest tile (N = 640 -> 4 x 160, 672 -> 3 x 224)
+  if (!want_pair) {
+    p.BN = w->N >= 128 ? 128 : w->N;
+  } else if (passes == 1) {              // least padded work, then the widest tile (N = 640 -> 4 x 160, 672 -> 3 x 224)
     int best = 1 << 30;
     for (int bn = 256; bn >= 128; bn -= 32) {
       const int padded = (w->N + bn - 1) / bn * bn;
       if (padded < best) { best = padded; p.BN = bn; }
     }
-  }
-  if (p.BN == 0 && !want_pair && fuse_mode != 0) p.BN = w->N >= 128 ? 128 : w->N;
-  if (p.BN == 0) {
+  } else {
     // 256 and 128 first: with the 32 KB of epilogue staging, 128 keeps three 64 KB stages in flight; then the largest
     // divisor (672 -> 224).  profiles/r01/gemm_f16_sweep.jsonl
     static const int order[] = {256, 128, 224, 192, 160, 96, 64, 32};
@@ -698,21 +678,18 @@ int gemm_tcgen05_f16x3(const dcae_operand* a, const dcae_weight* w, const dcae_e
   }
   DCAE_REQUIRE(p.BN > 0 && p.BN % 32 == 0, "gemm(f16x3): N=%d must be a multiple of 32", w->N);
   p.n_tiles_n = (w->N + p.BN - 1) / p.BN;      // a ragged last tile reads zero-filled weight rows and stores clipped
-  p.fuse_b = (fuse_mode != 0 && !want_pair && p.BN <= 128 && passes == 3) ? 1 : 0;
+  p.fuse_b = (!want_pair && p.BN <= 128 && passes == 3) ? 1 : 0;
   const int acc_cols = 2 * (p.fuse_b ? 2 * p.BN : p.BN);          // two chunk buffers
   p.tmem_cols = acc_cols <= 64 ? 64 : acc_cols <= 128 ? 128 : acc_cols <= 256 ? 256 : 512;
   p.total_tiles = p.n_tiles_n * (pair ? (m_tiles + 1) / 2 : m_tiles);
   p.chunk_kb = CHUNK_MMAS / (passes == 1 ? 4 : p.fuse_b ? 8 : 12);      // accumulation chain per column: 1, 2 (fused) or 3 MMAs per K = 16 step, 4 steps per k-block
-  if (const char* env = getenv("DCAE_TC_CHUNK")) { const int v = atoi(env); if (v >= 1) p.chunk_kb = v; }
   p.descale = w->descale;
-  p.dbg_nostore = getenv("DCAE_TC_NOSTORE") != nullptr;
   static const bool dbg_on = getenv("DCAE_F16_DBG") != nullptr;
   p.dbg = nullptr;
   p.b_bytes = (uint32_t)(pair ? p.BN / 2 : p.BN) * BK16 * 2;     // a pair's CTA holds half of the weight rows
   p.stage_bytes = (passes == 3 ? 2 : 1) * (A16_BYTES + p.b_bytes);
   p.stages = (int)((SMEM_LIMIT - 2048 - 2 * STG_BYTES) / p.stage_bytes);
   if (p.stages > MAX_STAGES) p.stages = MAX_STAGES;
-  if (const char* env = getenv("DCAE_TC_STAGES")) { const int v = atoi(env); if (v >= 1 && v < p.stages) p.stages = v; }
   if (p.stages > p.KB) p.stages = p.KB;
   DCAE_REQUIRE(p.stages >= 1, "gemm(f16x3): tile does not fit in shared memory");
   const size_t smem = (size_t)p.stages * p.stage_bytes + 2 * STG_BYTES + 1024;
@@ -779,39 +756,14 @@ int gemm_tcgen05_f16x3(const dcae_operand* a, const dcae_weight* w, const dcae_e
     DCAE_CUDA(cudaMalloc(&p.dbg, (size_t)n_ctas * 24 * sizeof(unsigned long long)));
     DCAE_CUDA(cudaMemsetAsync(p.dbg, 0, (size_t)n_ctas * 24 * sizeof(unsigned long long), s));
   }
-  // Opt-in (DCAE_F16_PDL=1).  Measured at config #2 (tools/lanes_ab.py, medians of 8 x 10 steps): one lane 13.67 ->
-  // 13.58 ms, two lanes 13.60 -> 13.74 ms -- the early-resident CTAs of the successor hold SMs the other lane's
-  // kernels would have used, and the chip is power-capped either way.
-  static const int pdl_mode = [] { const char* v = getenv("DCAE_F16_PDL"); return v ? atoi(v) : 0; }();
-  p.pdl = (pdl_mode != 0 && !dbg_on) ? 1 : 0;
-  cudaLaunchConfig_t cfg = {};
-  cfg.blockDim = dim3(NTHREADS);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = s;
-  cudaLaunchAttribute pdl_attr[1];
-  pdl_attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  pdl_attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = pdl_attr;
-  cfg.numAttrs = p.pdl ? 1 : 0;
-  if (pair) {
-    const int max_pairs = num_sms() / 2;
-    const int pairs = p.total_tiles < max_pairs ? p.total_tiles : max_pairs;
-#define F16_LAUNCH_ONE(KERNEL, GRID) DCAE_CUDA(cudaLaunchKernelEx(&cfg, KERNEL, map_ah, map_al, map_bh, map_bl, map_o32, map_oh, map_ol, map_oha, map_ola, p))
-#define F16_LAUNCH(KERNEL, GRID)                                                                                      \
-  do {                                                                                                                \
-    cfg.gridDim = dim3((unsigned)(GRID));                                                                             \
-    if (dbg_on && p.BN <= 128) F16_LAUNCH_ONE((KERNEL<true, 2>), GRID);                                               \
-    else if (dbg_on) F16_LAUNCH_ONE((KERNEL<true, 4>), GRID);                                                         \
-    else if (p.BN <= 128) F16_LAUNCH_ONE((KERNEL<false, 2>), GRID);                                                   \
-    else F16_LAUNCH_ONE((KERNEL<false, 4>), GRID);                                                                    \
-  } while (0)
-    F16_LAUNCH(gemm_f16x3_pair_kernel, 2 * pairs);
-  } else {
-    const int ctas = p.total_tiles < num_sms() ? p.total_tiles : num_sms();
-    F16_LAUNCH(gemm_f16x3_kernel, ctas);
-#undef F16_LAUNCH
-#undef F16_LAUNCH_ONE
-  }
+  // the pair kernel's cluster shape is fixed at compile time (__cluster_dims__)
+  const bool nb2 = p.BN <= 128;
+  decltype(&gemm_f16x3_kernel<false, 2>) kernel;
+  if (pair) kernel = dbg_on ? (nb2 ? gemm_f16x3_pair_kernel<true, 2> : gemm_f16x3_pair_kernel<true, 4>)
+                            : (nb2 ? gemm_f16x3_pair_kernel<false, 2> : gemm_f16x3_pair_kernel<false, 4>);
+  else kernel = dbg_on ? (nb2 ? gemm_f16x3_kernel<true, 2> : gemm_f16x3_kernel<true, 4>)
+                       : (nb2 ? gemm_f16x3_kernel<false, 2> : gemm_f16x3_kernel<false, 4>);
+  kernel<<<n_ctas, NTHREADS, smem, s>>>(map_ah, map_al, map_bh, map_bl, map_o32, map_oh, map_ol, map_oha, map_ola, p);
   DCAE_LAUNCH_CHECK();
   if (dbg_on) {
     std::vector<unsigned long long> hbuf((size_t)n_ctas * 24);

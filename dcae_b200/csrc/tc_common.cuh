@@ -213,13 +213,6 @@ __device__ __forceinline__ void warp_transpose32(float* r, int lane) {
   }
 }
 
-__device__ __forceinline__ float epi_act(float v, int act) {
-  if (act == DCAE_ACT_GELU) return gelu_erf(v);
-  if (act == DCAE_ACT_HALF_TANH) return 0.5f * tanhf(v);
-  if (act == DCAE_ACT_RELU) return fmaxf(v, 0.f);
-  return v;
-}
-
 // acc (+)= the chain partial sitting in TMEM at taddr (this warp's lane quarter, start of the chain buffer).
 // Both tcgen05.ld of a 32-column block are in flight per wait (more would spill next to the 128 running sums).
 template <int NB = EPI_BLOCKS>
@@ -254,7 +247,6 @@ __device__ __forceinline__ void drain_chunk(float* acc, uint32_t taddr, int half
 struct EpiTile {
   int b, y0, x0, n0;        // image, tile origin on the token grid, first output column
   int B, h, w, tw_shift, N, BN;
-  int dbg;                  // tuning experiments (env DCAE_TC_EPI): 1 = skip transpose, 2 = skip global stores
 };
 
 // Row-per-lane epilogue of one 32-column block held in r[0..32): bias / addend / activation / scaled residual, eight

@@ -9,7 +9,6 @@
 //     GEMM (kernel 2) unchanged.
 // All HBM-bound, fp32 in / fp32 (+ optional fp16 hi/lo planes) out, no atomics, deterministic.
 #include <math.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 
@@ -523,16 +522,15 @@ extern "C" int dcae_op_window_attention(const float* qkv, int64_t ld, int32_t q_
   a.out = out; a.out_ld = out_ld; a.o16 = o16;
   const dim3 grid((unsigned)(a.nwx * a.nwy), (unsigned)B);
   cudaStream_t s = (cudaStream_t)stream;
-  // 8x8 windows: the warp-MMA kernel (3 x TF32); DCAE_WIN_MMA = 0 selects the fp32 FFMA kernel (the cross-check); 4x4 windows: FFMA
-  static const int use_mma = [] { const char* v = getenv("DCAE_WIN_MMA"); return v ? atoi(v) : 1; }();
-  if (window == 8 && use_mma) {
+  // 8x8 windows: the warp-MMA kernel (3 x TF32); 4x4 windows: the FFMA kernel
+  if (window == 8) {
     if (head_dim == 8) window_attention_mma_kernel<8><<<grid, 128, 0, s>>>(a, C);
     else if (head_dim == 16) window_attention_mma_kernel<16><<<grid, 128, 0, s>>>(a, C);
     else window_attention_mma_kernel<32><<<grid, 128, 0, s>>>(a, C);
   } else {
-#define WIN_CASE(HD, P) if (head_dim == HD && window == P) window_attention_kernel<HD, P><<<grid, 2 * P * P, 0, s>>>(a);
-    WIN_CASE(8, 4) WIN_CASE(16, 4) WIN_CASE(32, 4) WIN_CASE(8, 8) WIN_CASE(16, 8) WIN_CASE(32, 8)
-#undef WIN_CASE
+    if (head_dim == 8) window_attention_kernel<8, 4><<<grid, 32, 0, s>>>(a);
+    else if (head_dim == 16) window_attention_kernel<16, 4><<<grid, 32, 0, s>>>(a);
+    else window_attention_kernel<32, 4><<<grid, 32, 0, s>>>(a);
   }
   DCAE_LAUNCH_CHECK();
   return DCAE_OK;

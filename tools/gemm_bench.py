@@ -12,11 +12,7 @@ lib = _lib.load()
 dev = torch.device("cuda:0")
 
 
-def bench(Kd, N, math, taps=1, bn=None, reps=10):
-    if bn:
-        os.environ["DCAE_TC_BN"] = str(bn)
-    else:
-        os.environ.pop("DCAE_TC_BN", None)
+def bench(Kd, N, math, taps=1, reps=10):
     C = Kd // taps
     buf = torch.randn(T, C, device=dev)
     wt = torch.randn(N, Kd, device=dev) * 0.02
@@ -35,12 +31,10 @@ def bench(Kd, N, math, taps=1, bn=None, reps=10):
     e1.record(); torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / reps
     tf = 2.0 * T * N * Kd / (ms * 1e-3) / 1e12
-    print(json.dumps({"K": Kd, "N": N, "taps": taps, "math": math, "bn": bn, "ms": round(ms, 4), "algo_TFLOPs": round(tf, 1),
+    print(json.dumps({"K": Kd, "N": N, "taps": taps, "math": math, "ms": round(ms, 4), "algo_TFLOPs": round(tf, 1),
                       "mma_TFLOPs": round(tf * (3 if math == "tf32x3" else 1), 1)}), flush=True)
 
 
 for math in ("tf32x3", "tf32"):
-    for Kd, N, taps, bns in [(640, 640, 1, [64, 128, 160]), (2560, 640, 1, [64, 128, 160]), (640, 2560, 1, [128, 256]),
-                             (8640, 672, 9, [96, 224]), (2016, 128, 9, [64, 128]), (1152, 64, 9, [32, 64])]:
-        for bn in bns:
-            bench(Kd, N, math, taps, bn)
+    for Kd, N, taps in [(640, 640, 1), (2560, 640, 1), (640, 2560, 1), (8640, 672, 9), (2016, 128, 9), (1152, 64, 9)]:
+        bench(Kd, N, math, taps)
