@@ -9,7 +9,10 @@ Public surface (mirrors the reference's operator interface for this path only):
   EntropyModel, SliceLoopFunction -- the training form (autograd: kernels forward, torch-graph recompute backward)
   ans.BufferedRansEncoder / RansDecoder -- the native range coder with compressai.ans' interface
   init_entropy_params   -- deterministic random-init weights with the reference's state-dict keys
-  TransformStack, accelerate_transforms, init_transform_params -- g_a / g_s / h_a / h_z_s1 / h_z_s2 on the library (dcae_b200/transforms.py)
+  TransformStack, accelerate_transforms, init_transform_params -- g_a / g_s / h_a / h_z_s1 / h_z_s2 on the library (dcae_b200/transforms.py);
+                        accelerate_transforms also trains: under autograd each stack call is a recompute node
+  TransformModel        -- one transform stack as a trainable module (kernels forward, recompute backward with the
+                           window-attention backward kernel; dcae_b200/training.py)
   DCAECodec             -- the whole model (forward / compress / decompress / update, image <-> .bin container) from a reference state dict
   container             -- the reference's bitstream container and image padding (compress_and_decompress.py:48-148)
 """
@@ -27,7 +30,7 @@ def __getattr__(name):
     if name in ("accelerate", "DictCrossAttention", "ConvStack"):
         from . import modules
         return getattr(modules, name)
-    if name in ("EntropyModel", "SliceLoopFunction", "GaussianLikelihoodFunction", "rate_distortion_loss"):
+    if name in ("EntropyModel", "SliceLoopFunction", "GaussianLikelihoodFunction", "rate_distortion_loss", "TransformModel"):
         from . import training
         return getattr(training, name)
     if name == "EntropyBottleneck":

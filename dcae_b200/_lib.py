@@ -143,7 +143,10 @@ SIGNATURES = {
     "dcae_op_spatial_gate_ln": (C.c_int, [_P, _I64, _P, _I64, _P, _P, _I32, _I32, _I32, _I32, _P, _P, _I64, _P, _P, C.POINTER(Planes), _P]),
     "dcae_op_dict_attention": (C.c_int, [_P, _I64, C.POINTER(Planes), C.POINTER(DictKV), _I64, _P, _I64, C.POINTER(Planes), C.c_int, _P]),
     "dcae_op_window_attention": (C.c_int, [_P, _I64, _I32, _I32, _I32, _I32, _I32, _I32, _I32, _P, _I32, _I32, _I32, _P, _I64, C.POINTER(Planes), _P]),
-    "dcae_op_space_to_depth": (C.c_int, [_P, _I64, _I32, _I32, _I32, _I32, _I32, _P, _I64, C.POINTER(Planes), _P]),
+    "dcae_window_attention_backward_scratch_bytes": (C.c_size_t, [_I32, _I32, _I32, _I32, _I32, _I32]),
+    "dcae_op_window_attention_backward": (C.c_int, [_P, _I64, _I32, _I32, _I32, _I32, _I32, _I32, _I32, _P, _I32, _I32, _I32, _P, _I64, _P, _I64,
+                                                    _P, _P, C.c_size_t, _P]),
+    "dcae_op_space_to_depth":(C.c_int, [_P, _I64, _I32, _I32, _I32, _I32, _I32, _P, _I64, C.POINTER(Planes), _P]),
     "dcae_op_depth_to_space": (C.c_int, [_P, _I64, _I32, _I32, _I32, _I32, _I32, _I32, _P, _I64, C.POINTER(Planes), _P]),
     "dcae_op_nchw_to_tokens": (C.c_int, [_P, _I32, _I32, _I64, _P, _I64, C.POINTER(Planes), _P]),
     "dcae_op_tokens_to_nchw": (C.c_int, [_P, _I64, _I32, _I32, _I64, _P, _P]),

@@ -407,6 +407,337 @@ __global__ void __launch_bounds__(128) window_attention_mma_kernel(const WinArgs
 }
 
 // ---------------------------------------------------------------------------------------------
+// Backward of the window attention.  Per window and head, s = 1 / sqrt(hd): S and P recomputed as the forward does (same
+// bias, SW mask, max-subtracted exponentials); dP = dO V^T; D_i = sum_j P_ij dP_ij; dS = P o (dP - D); dQ = s dS K,
+// dK = s dS^T Q, dV = P^T dO; drel[e, dy, dx] = sum of dS over the (query, key) pairs at that offset.
+// Determinism without atomics: every token belongs to one window, so each dq / dk / dv element has one writer; block b walks
+// heads in order and, per head, the windows b, b + gridDim.x, ... (flattened over the batch) in order, accumulates its drel
+// bins in registers (thread tid owns bins tid, tid + NT, ...) and writes them to part[b][e][bin]; a second launch adds the
+// partials in block order.  The grid depends on the shape only (wattn_bwd_blocks).
+// ---------------------------------------------------------------------------------------------
+constexpr int WATTN_BWD_MAX_BLOCKS = 1184;         // 148 SMs x 8
+
+inline int64_t wattn_bwd_blocks(int64_t n_windows) { return n_windows < WATTN_BWD_MAX_BLOCKS ? n_windows : WATTN_BWD_MAX_BLOCKS; }
+
+struct WinBwdArgs {
+  const float* qkv; int64_t ld; int q_col, k_col, v_col;
+  int n_heads, shift, h, w, nwx, nwy;
+  int64_t n_win;               // B * nwx * nwy
+  const float* rel;            // [n_heads, 2P-1, 2P-1]
+  float scale;
+  const float* dout; int64_t dout_ld;
+  float* dqkv; int64_t dqkv_ld;
+  float* part;                 // [gridDim.x, n_heads, (2P-1)^2]
+};
+
+// window `win` (flattened b, wy, wx) -> its tokens (rolled by the SW shift) into stok, and (wy, wx)
+template <int P>
+__device__ __forceinline__ void window_tokens(const WinBwdArgs& a, int64_t win, int64_t* stok, int& wy, int& wx) {
+  const int64_t nw = (int64_t)a.nwx * a.nwy;
+  const int b = (int)(win / nw), wi = (int)(win - b * nw);
+  wx = wi % a.nwx; wy = wi / a.nwx;
+  for (int p = threadIdx.x; p < P * P; p += blockDim.x) {
+    int yy = wy * P + p / P + a.shift; if (yy >= a.h) yy -= a.h;
+    int xx = wx * P + p % P + a.shift; if (xx >= a.w) xx -= a.w;
+    stok[p] = ((int64_t)b * a.h + yy) * a.w + xx;
+  }
+}
+
+// sum of dS over the pairs at bin = (dy + P - 1) * R + (dx + P - 1): query (py, px), key (py - dy, px - dx); dS(i, j) = ds[j * ld + i]
+template <int P>
+__device__ __forceinline__ float rel_bin_sum(const float* dsT, int ld, int bin) {
+  constexpr int R = 2 * P - 1;
+  const int dy = bin / R - (P - 1), dx = bin % R - (P - 1);
+  float s = 0.f;
+  for (int py = dy > 0 ? dy : 0; py < (dy < 0 ? P + dy : P); ++py)
+    for (int px = dx > 0 ? dx : 0; px < (dx < 0 ? P + dx : P); ++px)
+      s += dsT[((py - dy) * P + (px - dx)) * ld + py * P + px];
+  return s;
+}
+
+// 4x4 windows (the hyper path): FFMA, one window of PP = 16 tokens per block iteration, everything in shared memory
+template <int HD, int P>
+__global__ void __launch_bounds__(128) window_attention_bwd_kernel(const WinBwdArgs a) {
+  constexpr int PP = P * P, R = 2 * P - 1, NT = 128, LD = HD + 1, LP = PP + 1, NB = (R * R + NT - 1) / NT;
+  __shared__ float sq[PP * LD], sk[PP * LD], sv[PP * LD], sdo[PP * LD];
+  __shared__ float sp[PP * LP], sdsT[PP * LP];        // P[i][j] at i * LP + j; dS transposed: dS[i][j] at j * LP + i
+  __shared__ float sdp[PP * LP];
+  __shared__ float sbias[R * R];
+  __shared__ int64_t stok[PP];
+  const int tid = threadIdx.x, sp_edge = P - a.shift;
+  for (int e = 0; e < a.n_heads; ++e) {
+    float acc[NB];
+#pragma unroll
+    for (int r = 0; r < NB; ++r) acc[r] = 0.f;
+    for (int64_t win = blockIdx.x; win < a.n_win; win += gridDim.x) {
+      __syncthreads();                     // the previous window is done with shared memory
+      int wy, wx;
+      window_tokens<P>(a, win, stok, wy, wx);
+      for (int i = tid; i < R * R; i += NT) sbias[i] = __ldg(a.rel + (int64_t)e * R * R + i);
+      __syncthreads();
+      for (int idx = tid; idx < PP * HD; idx += NT) {
+        const int t = idx / HD, d = idx - t * HD;
+        const float* row = a.qkv + stok[t] * a.ld + e * HD + d;
+        sq[t * LD + d] = __ldg(row + a.q_col);
+        sk[t * LD + d] = __ldg(row + a.k_col);
+        sv[t * LD + d] = __ldg(row + a.v_col);
+        sdo[t * LD + d] = __ldg(a.dout + stok[t] * a.dout_ld + e * HD + d);
+      }
+      __syncthreads();
+      const bool last_row = a.shift > 0 && wy == a.nwy - 1, last_col = a.shift > 0 && wx == a.nwx - 1;
+      for (int pr = tid; pr < PP * PP; pr += NT) {
+        const int i = pr / PP, j = pr - i * PP;
+        float s = 0.f, dp = 0.f;
+#pragma unroll
+        for (int d = 0; d < HD; ++d) {
+          s = fmaf(sq[i * LD + d], sk[j * LD + d], s);
+          dp = fmaf(sdo[i * LD + d], sv[j * LD + d], dp);
+        }
+        const int py = i / P, px = i % P, qy = j / P, qx = j % P;
+        const bool masked = (last_row && ((py < sp_edge) != (qy < sp_edge))) || (last_col && ((px < sp_edge) != (qx < sp_edge)));
+        sp[i * LP + j] = masked ? -INFINITY : s * a.scale + sbias[(py - qy + P - 1) * R + (px - qx + P - 1)];
+        sdp[i * LP + j] = dp;
+      }
+      __syncthreads();
+      if (tid < PP) {                      // softmax, D and dS of query row tid
+        const int i = tid;
+        float m = -INFINITY;
+        for (int j = 0; j < PP; ++j) m = fmaxf(m, sp[i * LP + j]);
+        float sum = 0.f;
+        for (int j = 0; j < PP; ++j) { const float v = expf(sp[i * LP + j] - m); sp[i * LP + j] = v; sum += v; }
+        const float inv = 1.0f / sum;
+        float D = 0.f;
+        for (int j = 0; j < PP; ++j) { sp[i * LP + j] *= inv; D = fmaf(sp[i * LP + j], sdp[i * LP + j], D); }
+        for (int j = 0; j < PP; ++j) sdsT[j * LP + i] = sp[i * LP + j] * (sdp[i * LP + j] - D);
+      }
+      __syncthreads();
+      for (int idx = tid; idx < PP * HD; idx += NT) {
+        const int t = idx / HD, d = idx - t * HD;
+        float gq = 0.f, gk = 0.f, gv = 0.f;
+#pragma unroll
+        for (int j = 0; j < PP; ++j) {
+          gq = fmaf(sdsT[j * LP + t], sk[j * LD + d], gq);
+          gk = fmaf(sdsT[t * LP + j], sq[j * LD + d], gk);
+          gv = fmaf(sp[j * LP + t], sdo[j * LD + d], gv);
+        }
+        float* o = a.dqkv + stok[t] * a.dqkv_ld + e * HD + d;
+        o[a.q_col] = gq * a.scale;
+        o[a.k_col] = gk * a.scale;
+        o[a.v_col] = gv;
+      }
+#pragma unroll
+      for (int r = 0; r < NB; ++r)
+        if (tid + r * NT < R * R) acc[r] += rel_bin_sum<P>(sdsT, LP, tid + r * NT);
+    }
+#pragma unroll
+    for (int r = 0; r < NB; ++r)
+      if (tid + r * NT < R * R) a.part[((int64_t)blockIdx.x * a.n_heads + e) * R * R + tid + r * NT] = acc[r];
+  }
+}
+
+// 8x8 windows: the products on m16n8k8 TF32 MMAs with the 3-pass hi/lo split, like window_attention_mma_kernel.  4 warps;
+// warp w owns query rows [16 w, 16 w + 16) for S, dP, dS and dQ (P, dP, D and dS never leave registers: the C fragment of
+// dP = dO V^T has the layout of S, and dS is then the A fragment of dS K with the forward's key-slot order), and key rows
+// [16 w, 16 w + 16) for dK = dS^T Q and dV = P^T dO, whose A operands go through shared memory transposed.  Q, K, V, dO
+// of the head sit in shared memory as fp32 (split into hi / lo at fragment load).
+template <int HD>
+__host__ __device__ constexpr int wattn_bwd_mma_smem_floats() { return 4 * 64 * (HD + 4) + 2 * 64 * 72 + 228; }
+
+__device__ __forceinline__ void split_tf32(float v, float& hi, float& lo) { hi = to_tf32(v); lo = to_tf32(v - hi); }
+
+// d += a b, 3 passes (a_lo b_hi + a_hi b_lo + a_hi b_hi)
+__device__ __forceinline__ void mma3_tf32(float (&d)[4], const float (&ah)[4], const float (&al)[4], float b0, float b1) {
+  float bh0, bl0, bh1, bl1;
+  split_tf32(b0, bh0, bl0);
+  split_tf32(b1, bh1, bl1);
+  mma_tf32_16x8x8(d, al, bh0, bh1);
+  mma_tf32_16x8x8(d, ah, bl0, bl1);
+  mma_tf32_16x8x8(d, ah, bh0, bh1);
+}
+
+template <int HD>
+__global__ void __launch_bounds__(128) window_attention_bwd_mma_kernel(const WinBwdArgs a) {
+  constexpr int P = 8, PP = 64, R = 2 * P - 1, LDS = HD + 4, LDT = 72, KSTEPS = HD / 8, NT = 128;
+  extern __shared__ __align__(16) float smem[];
+  float* sq = smem;
+  float* sk = sq + PP * LDS;
+  float* sv = sk + PP * LDS;
+  float* sdo = sv + PP * LDS;
+  float* spT = sdo + PP * LDS;             // P transposed: P[i][j] at j * LDT + i
+  float* sdsT = spT + PP * LDT;            // dS transposed
+  float* sbias = sdsT + PP * LDT;          // R * R (228 floats keep stok 16-byte aligned)
+  int64_t* stok = reinterpret_cast<int64_t*>(sbias + 228);
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, t = lane & 3;
+  const int r0 = 16 * warp + g, r1 = r0 + 8;          // this thread's query rows (and key rows in the dK / dV phase)
+  const int py0 = 2 * warp, px = g, sp_edge = P - a.shift;
+  for (int e = 0; e < a.n_heads; ++e) {
+    float acc[2] = {0.f, 0.f};
+    for (int64_t win = blockIdx.x; win < a.n_win; win += gridDim.x) {
+      __syncthreads();
+      int wy, wx;
+      window_tokens<P>(a, win, stok, wy, wx);
+      for (int i = tid; i < R * R; i += NT) sbias[i] = __ldg(a.rel + (int64_t)e * R * R + i);
+      __syncthreads();
+      for (int idx = tid; idx < PP * (HD / 4); idx += NT) {
+        const int tk = idx / (HD / 4), d4 = idx - tk * (HD / 4);
+        const float* row = a.qkv + stok[tk] * a.ld + e * HD + 4 * d4;
+        *reinterpret_cast<float4*>(sq + tk * LDS + 4 * d4) = __ldg(reinterpret_cast<const float4*>(row + a.q_col));
+        *reinterpret_cast<float4*>(sk + tk * LDS + 4 * d4) = __ldg(reinterpret_cast<const float4*>(row + a.k_col));
+        *reinterpret_cast<float4*>(sv + tk * LDS + 4 * d4) = __ldg(reinterpret_cast<const float4*>(row + a.v_col));
+        *reinterpret_cast<float4*>(sdo + tk * LDS + 4 * d4) =
+            __ldg(reinterpret_cast<const float4*>(a.dout + stok[tk] * a.dout_ld + e * HD + 4 * d4));
+      }
+      __syncthreads();
+      // S = Q K^T and dP = dO V^T (C fragment: c0 = (g, 2t), c1 = (g, 2t + 1), c2 = (g + 8, 2t), c3 = (g + 8, 2t + 1) of key tile nt)
+      float sc[8][4], dp[8][4];
+#pragma unroll
+      for (int nt = 0; nt < 8; ++nt) {
+#pragma unroll
+        for (int i = 0; i < 4; ++i) { sc[nt][i] = 0.f; dp[nt][i] = 0.f; }
+      }
+#pragma unroll
+      for (int ks = 0; ks < KSTEPS; ++ks) {
+        float qh[4], ql[4], oh[4], ol[4];
+        const int c = 8 * ks + t;
+        const float qa[4] = {sq[r0 * LDS + c], sq[r1 * LDS + c], sq[r0 * LDS + c + 4], sq[r1 * LDS + c + 4]};
+        const float oa[4] = {sdo[r0 * LDS + c], sdo[r1 * LDS + c], sdo[r0 * LDS + c + 4], sdo[r1 * LDS + c + 4]};
+#pragma unroll
+        for (int i = 0; i < 4; ++i) { split_tf32(qa[i], qh[i], ql[i]); split_tf32(oa[i], oh[i], ol[i]); }
+#pragma unroll
+        for (int nt = 0; nt < 8; ++nt) {
+          const int o = (8 * nt + g) * LDS + c;
+          mma3_tf32(sc[nt], qh, ql, sk[o], sk[o + 4]);
+          mma3_tf32(dp[nt], oh, ol, sv[o], sv[o + 4]);
+        }
+      }
+      const bool last_row = a.shift > 0 && wy == a.nwy - 1, last_col = a.shift > 0 && wx == a.nwx - 1;
+      float m0 = -INFINITY, m1 = -INFINITY;
+#pragma unroll
+      for (int nt = 0; nt < 8; ++nt) {
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+          const int r = i >> 1, qx = 2 * t + (i & 1), py = py0 + r, qy = nt;
+          const float v = sc[nt][i] * a.scale + sbias[(py - qy + P - 1) * R + (px - qx + P - 1)];
+          const bool masked = (last_row && ((py < sp_edge) != (qy < sp_edge))) || (last_col && ((px < sp_edge) != (qx < sp_edge)));
+          sc[nt][i] = masked ? -INFINITY : v;
+        }
+        m0 = fmaxf(m0, fmaxf(sc[nt][0], sc[nt][1]));
+        m1 = fmaxf(m1, fmaxf(sc[nt][2], sc[nt][3]));
+      }
+      m0 = fmaxf(m0, __shfl_xor_sync(0xffffffffu, m0, 1)); m0 = fmaxf(m0, __shfl_xor_sync(0xffffffffu, m0, 2));
+      m1 = fmaxf(m1, __shfl_xor_sync(0xffffffffu, m1, 1)); m1 = fmaxf(m1, __shfl_xor_sync(0xffffffffu, m1, 2));
+      float s0 = 0.f, s1 = 0.f;
+#pragma unroll
+      for (int nt = 0; nt < 8; ++nt) {
+        sc[nt][0] = expf(sc[nt][0] - m0); sc[nt][1] = expf(sc[nt][1] - m0);
+        sc[nt][2] = expf(sc[nt][2] - m1); sc[nt][3] = expf(sc[nt][3] - m1);
+        s0 += sc[nt][0] + sc[nt][1];
+        s1 += sc[nt][2] + sc[nt][3];
+      }
+      s0 += __shfl_xor_sync(0xffffffffu, s0, 1); s0 += __shfl_xor_sync(0xffffffffu, s0, 2);
+      s1 += __shfl_xor_sync(0xffffffffu, s1, 1); s1 += __shfl_xor_sync(0xffffffffu, s1, 2);
+      const float i0 = 1.0f / s0, i1 = 1.0f / s1;
+      float D0 = 0.f, D1 = 0.f;
+#pragma unroll
+      for (int nt = 0; nt < 8; ++nt) {
+        sc[nt][0] *= i0; sc[nt][1] *= i0; sc[nt][2] *= i1; sc[nt][3] *= i1;
+        D0 = fmaf(sc[nt][0], dp[nt][0], fmaf(sc[nt][1], dp[nt][1], D0));
+        D1 = fmaf(sc[nt][2], dp[nt][2], fmaf(sc[nt][3], dp[nt][3], D1));
+      }
+      D0 += __shfl_xor_sync(0xffffffffu, D0, 1); D0 += __shfl_xor_sync(0xffffffffu, D0, 2);
+      D1 += __shfl_xor_sync(0xffffffffu, D1, 1); D1 += __shfl_xor_sync(0xffffffffu, D1, 2);
+#pragma unroll
+      for (int nt = 0; nt < 8; ++nt) {
+        dp[nt][0] = sc[nt][0] * (dp[nt][0] - D0); dp[nt][1] = sc[nt][1] * (dp[nt][1] - D0);
+        dp[nt][2] = sc[nt][2] * (dp[nt][2] - D1); dp[nt][3] = sc[nt][3] * (dp[nt][3] - D1);
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+          const int key = 8 * nt + 2 * t + (i & 1), q = (i >> 1) ? r1 : r0;
+          spT[key * LDT + q] = sc[nt][i];
+          sdsT[key * LDT + q] = dp[nt][i];
+        }
+      }
+      // dQ = s dS K: k-step j = key tile j, slot t <-> key 8j + 2t, slot t + 4 <-> key 8j + 2t + 1 (A = (c0, c2, c1, c3) of dS)
+      {
+        float gq[KSTEPS][4];
+#pragma unroll
+        for (int nd = 0; nd < KSTEPS; ++nd) {
+#pragma unroll
+          for (int i = 0; i < 4; ++i) gq[nd][i] = 0.f;
+        }
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+          const float av[4] = {dp[j][0], dp[j][2], dp[j][1], dp[j][3]};
+          float ah[4], al[4];
+#pragma unroll
+          for (int i = 0; i < 4; ++i) split_tf32(av[i], ah[i], al[i]);
+#pragma unroll
+          for (int nd = 0; nd < KSTEPS; ++nd) {
+            const int o = (8 * j + 2 * t) * LDS + 8 * nd + g;
+            mma3_tf32(gq[nd], ah, al, sk[o], sk[o + LDS]);
+          }
+        }
+#pragma unroll
+        for (int nd = 0; nd < KSTEPS; ++nd) {
+          const int col = a.q_col + e * HD + 8 * nd + 2 * t;
+          *reinterpret_cast<float2*>(a.dqkv + stok[r0] * a.dqkv_ld + col) = make_float2(gq[nd][0] * a.scale, gq[nd][1] * a.scale);
+          *reinterpret_cast<float2*>(a.dqkv + stok[r1] * a.dqkv_ld + col) = make_float2(gq[nd][2] * a.scale, gq[nd][3] * a.scale);
+        }
+      }
+      __syncthreads();                     // P^T and dS^T complete
+      // dV = P^T dO and dK = s dS^T Q for key rows r0 / r1: k-step ks over queries, slot t <-> query 8ks + 2t, t + 4 <-> 8ks + 2t + 1
+      {
+        float gk[KSTEPS][4], gv[KSTEPS][4];
+#pragma unroll
+        for (int nd = 0; nd < KSTEPS; ++nd) {
+#pragma unroll
+          for (int i = 0; i < 4; ++i) { gk[nd][i] = 0.f; gv[nd][i] = 0.f; }
+        }
+#pragma unroll 2
+        for (int ks = 0; ks < 8; ++ks) {
+          const int c = 8 * ks + 2 * t;
+          const float pa[4] = {spT[r0 * LDT + c], spT[r1 * LDT + c], spT[r0 * LDT + c + 1], spT[r1 * LDT + c + 1]};
+          const float da[4] = {sdsT[r0 * LDT + c], sdsT[r1 * LDT + c], sdsT[r0 * LDT + c + 1], sdsT[r1 * LDT + c + 1]};
+          float ph[4], pl[4], dh[4], dl[4];
+#pragma unroll
+          for (int i = 0; i < 4; ++i) { split_tf32(pa[i], ph[i], pl[i]); split_tf32(da[i], dh[i], dl[i]); }
+#pragma unroll
+          for (int nd = 0; nd < KSTEPS; ++nd) {
+            const int o = c * LDS + 8 * nd + g;
+            mma3_tf32(gv[nd], ph, pl, sdo[o], sdo[o + LDS]);
+            mma3_tf32(gk[nd], dh, dl, sq[o], sq[o + LDS]);
+          }
+        }
+#pragma unroll
+        for (int nd = 0; nd < KSTEPS; ++nd) {
+          const int cd = e * HD + 8 * nd + 2 * t;
+          float* o0 = a.dqkv + stok[r0] * a.dqkv_ld + cd;
+          float* o1 = a.dqkv + stok[r1] * a.dqkv_ld + cd;
+          *reinterpret_cast<float2*>(o0 + a.k_col) = make_float2(gk[nd][0] * a.scale, gk[nd][1] * a.scale);
+          *reinterpret_cast<float2*>(o1 + a.k_col) = make_float2(gk[nd][2] * a.scale, gk[nd][3] * a.scale);
+          *reinterpret_cast<float2*>(o0 + a.v_col) = make_float2(gv[nd][0], gv[nd][1]);
+          *reinterpret_cast<float2*>(o1 + a.v_col) = make_float2(gv[nd][2], gv[nd][3]);
+        }
+      }
+      acc[0] += rel_bin_sum<P>(sdsT, LDT, tid);
+      if (tid + NT < R * R) acc[1] += rel_bin_sum<P>(sdsT, LDT, tid + NT);
+    }
+    float* part = a.part + ((int64_t)blockIdx.x * a.n_heads + e) * R * R;
+    part[tid] = acc[0];
+    if (tid + NT < R * R) part[tid + NT] = acc[1];
+  }
+}
+
+// drel[i] = sum over blocks b in order of part[b][i]
+__global__ void __launch_bounds__(256) rel_partials_reduce_kernel(const float* __restrict__ part, int n_blocks, int n, float* __restrict__ drel) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  float s = 0.f;
+  for (int b = 0; b < n_blocks; ++b) s += part[(int64_t)b * n + i];
+  drel[i] = s;
+}
+
+// ---------------------------------------------------------------------------------------------
 // space-to-depth: out[(b, y', x'), (sy*2 + sx) * Cs + c] = x[(b, 2y' + sy, 2x' + sx), c]  (0 outside / for c >= C)
 // depth-to-space: out[(b, 2y + py, 2x + px), c] = x[(b, y, x), (py*2 + px) * Cs + c]     (0 for C <= c < Cpad)
 // one thread per output float4 (scalar variant when a channel count is not a multiple of 4)
@@ -532,6 +863,70 @@ extern "C" int dcae_op_window_attention(const float* qkv, int64_t ld, int32_t q_
     else if (head_dim == 16) window_attention_kernel<16, 4><<<grid, 32, 0, s>>>(a);
     else window_attention_kernel<32, 4><<<grid, 32, 0, s>>>(a);
   }
+  DCAE_LAUNCH_CHECK();
+  return DCAE_OK;
+}
+
+extern "C" size_t dcae_window_attention_backward_scratch_bytes(int32_t B, int32_t h, int32_t w, int32_t C, int32_t head_dim, int32_t window) {
+  if (B <= 0 || window <= 0 || head_dim <= 0 || C <= 0 || h < window || w < window) return 0;
+  const int64_t n_win = (int64_t)B * (h / window) * (w / window);
+  const int64_t R = 2 * window - 1;
+  return (size_t)(wattn_bwd_blocks(n_win) * (C / head_dim) * R * R * (int64_t)sizeof(float));
+}
+
+extern "C" int dcae_op_window_attention_backward(const float* qkv, int64_t ld, int32_t q_col, int32_t k_col, int32_t v_col, int32_t C,
+                                                 int32_t head_dim, int32_t window, int32_t shift, const float* rel_bias, int32_t B, int32_t h,
+                                                 int32_t w, const float* dout, int64_t dout_ld, float* dqkv, int64_t dqkv_ld, float* drel,
+                                                 void* scratch, size_t scratch_bytes, void* stream) {
+  ProfileScope prof(DCAE_PROF_ATTN, 10.0 * B * h * w * (double)window * window * (double)C, stream);
+  DCAE_REQUIRE(qkv && rel_bias && dout && dqkv && drel, "dcae_op_window_attention_backward: null pointer");
+  DCAE_REQUIRE((window == 4 || window == 8) && (head_dim == 8 || head_dim == 16 || head_dim == 32),
+               "dcae_op_window_attention_backward: window %d / head_dim %d not supported (window 4 or 8, head_dim 8, 16 or 32)", window, head_dim);
+  DCAE_REQUIRE(C > 0 && C % head_dim == 0, "dcae_op_window_attention_backward: C=%d is not a multiple of head_dim=%d", C, head_dim);
+  DCAE_REQUIRE(B >= 0 && h > 0 && w > 0 && h % window == 0 && w % window == 0,
+               "dcae_op_window_attention_backward: the token grid %dx%d must be a multiple of the window %d", h, w, window);
+  DCAE_REQUIRE(shift == 0 || shift == window / 2, "dcae_op_window_attention_backward: shift must be 0 (W) or window/2 (SW)");
+  DCAE_REQUIRE(q_col >= 0 && k_col >= 0 && v_col >= 0 && q_col + C <= ld && k_col + C <= ld && v_col + C <= ld && q_col + C <= dqkv_ld &&
+                   k_col + C <= dqkv_ld && v_col + C <= dqkv_ld && dout_ld >= C,
+               "dcae_op_window_attention_backward: column windows exceed the leading dimension");
+  DCAE_REQUIRE(abs(q_col - k_col) >= C && abs(q_col - v_col) >= C && abs(k_col - v_col) >= C,
+               "dcae_op_window_attention_backward: the q / k / v column windows overlap");
+  DCAE_REQUIRE(aligned16(qkv) && aligned16(dout) && aligned16(dqkv) && ld % 4 == 0 && dout_ld % 4 == 0 && dqkv_ld % 4 == 0 && q_col % 4 == 0 &&
+                   k_col % 4 == 0 && v_col % 4 == 0,
+               "dcae_op_window_attention_backward: qkv / dout / dqkv must be 16-byte aligned with ld and column offsets multiples of 4");
+  DCAE_REQUIRE((int64_t)B * h * w < (1ll << 31), "dcae_op_window_attention_backward: too many tokens");
+  if (B == 0) return DCAE_OK;
+  const size_t need = dcae_window_attention_backward_scratch_bytes(B, h, w, C, head_dim, window);
+  DCAE_REQUIRE(scratch && scratch_bytes >= need && aligned16(scratch),
+               "dcae_op_window_attention_backward: scratch of %zu bytes (16-byte aligned) needed, %zu given", need, scratch ? scratch_bytes : (size_t)0);
+  WinBwdArgs a;
+  a.qkv = qkv; a.ld = ld; a.q_col = q_col; a.k_col = k_col; a.v_col = v_col;
+  a.n_heads = C / head_dim; a.shift = shift; a.h = h; a.w = w; a.nwx = w / window; a.nwy = h / window;
+  a.n_win = (int64_t)B * a.nwx * a.nwy;
+  a.rel = rel_bias; a.scale = 1.0f / sqrtf((float)head_dim);
+  a.dout = dout; a.dout_ld = dout_ld; a.dqkv = dqkv; a.dqkv_ld = dqkv_ld;
+  a.part = static_cast<float*>(scratch);
+  const int blocks = (int)wattn_bwd_blocks(a.n_win);
+  cudaStream_t s = (cudaStream_t)stream;
+  if (window == 8) {
+#define WBWD_MMA(HD)                                                                                                     \
+  {                                                                                                                      \
+    constexpr int bytes = wattn_bwd_mma_smem_floats<HD>() * 4 + 64 * 8;                                                  \
+    DCAE_CUDA(cudaFuncSetAttribute(window_attention_bwd_mma_kernel<HD>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes)); \
+    window_attention_bwd_mma_kernel<HD><<<blocks, 128, bytes, s>>>(a);                                                   \
+  }
+    if (head_dim == 8) WBWD_MMA(8)
+    else if (head_dim == 16) WBWD_MMA(16)
+    else WBWD_MMA(32)
+#undef WBWD_MMA
+  } else {
+    if (head_dim == 8) window_attention_bwd_kernel<8, 4><<<blocks, 128, 0, s>>>(a);
+    else if (head_dim == 16) window_attention_bwd_kernel<16, 4><<<blocks, 128, 0, s>>>(a);
+    else window_attention_bwd_kernel<32, 4><<<blocks, 128, 0, s>>>(a);
+  }
+  DCAE_LAUNCH_CHECK();
+  const int n = a.n_heads * (2 * window - 1) * (2 * window - 1);
+  rel_partials_reduce_kernel<<<(n + 255) / 256, 256, 0, s>>>(a.part, blocks, n, drel);
   DCAE_LAUNCH_CHECK();
   return DCAE_OK;
 }

@@ -9,6 +9,13 @@ differentiated analytically on the device (`dcae_gc_backward`).  Three entry poi
   EntropyModel                 nn.Module owning the hot-path parameters under the reference's keys; what DDP wraps
                                (train.py:413-426) when only the entropy model trains or is benchmarked
 
+and the same pattern for the transform stacks g_a / g_s / h_a / h_z_s1 / h_z_s2 (`dcae_b200.transform_graph` is their
+recompute graph; the windowed attention core keeps a kernel backward, `dcae_op_window_attention_backward`):
+
+  WindowAttentionFunction      the WMSA core with the library's forward and backward kernels
+  TransformStackFunction       one stack call as one autograd node (forward = `TransformStack.forward`)
+  TransformModel               nn.Module owning one stack's parameters, the transform counterpart of EntropyModel
+
 Gradients are the exact gradients of the fp32 graph (the forward values agree with it to 1e-5, tests/test_gpu_training.py
 pins gradient parity against the reference's own modules under torch autograd).
 """
@@ -19,9 +26,10 @@ from typing import Dict, Optional
 import torch
 import torch.nn as nn
 
-from . import _lib, torch_graph
+from . import _lib, torch_graph, transform_graph
 from .entropy_model import EntropySliceLoop
 from .params import init_entropy_params
+from .transforms import TransformStack, init_transform_params, transform_param_shapes
 
 
 def _rows(t: torch.Tensor):
@@ -170,6 +178,108 @@ class EntropyModel(nn.Module):
             return {k: out[k] for k in ("y_hat", "means", "scales", "likelihoods")}
         y_hat, mu, sc, lik = SliceLoopFunction.apply(self.engine[0], self.keys, noise, y, latent_scales, latent_means, *self.plist)
         return {"y_hat": y_hat, "means": mu, "scales": sc, "likelihoods": lik}
+
+
+class WindowAttentionFunction(torch.autograd.Function):
+    """out [B, h, w, C] = WMSA core of qkv [B, h, w, 3C] ('(threeh c)' columns) with relative position bias rel
+    [n_heads, 2 window - 1, 2 window - 1]: forward dcae_op_window_attention (fp32 output), backward
+    dcae_op_window_attention_backward (dq / dk / dv and drel).  The signature of `transform_graph.window_attention`."""
+
+    @staticmethod
+    def forward(ctx, qkv, head_dim: int, window: int, shift: int, rel):
+        lib = _lib.load()
+        qkv, rel = qkv.contiguous(), rel.contiguous()
+        B, h, w, C3 = qkv.shape
+        C = C3 // 3
+        out = qkv.new_empty(B, h, w, C)
+        with torch.cuda.device(qkv.device):
+            _lib.check(lib.dcae_op_window_attention(qkv.data_ptr(), C3, 0, C, 2 * C, C, head_dim, window, shift, rel.data_ptr(), B, h, w,
+                                                    out.data_ptr(), C, None, _lib.current_stream(qkv.device)), "dcae_op_window_attention")
+        ctx.save_for_backward(qkv, rel)
+        ctx.cfg = (head_dim, window, shift)
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        qkv, rel = ctx.saved_tensors
+        head_dim, window, shift = ctx.cfg
+        lib = _lib.load()
+        g = g.contiguous()
+        B, h, w, C3 = qkv.shape
+        C = C3 // 3
+        dqkv, drel = torch.empty_like(qkv), torch.empty_like(rel)
+        n = int(lib.dcae_window_attention_backward_scratch_bytes(B, h, w, C, head_dim, window))
+        scratch = torch.empty(max(n, 16), dtype=torch.uint8, device=qkv.device)
+        with torch.cuda.device(qkv.device):
+            _lib.check(lib.dcae_op_window_attention_backward(qkv.data_ptr(), C3, 0, C, 2 * C, C, head_dim, window, shift, rel.data_ptr(), B, h, w,
+                                                             g.data_ptr(), C, dqkv.data_ptr(), C3, drel.data_ptr(), scratch.data_ptr(), n,
+                                                             _lib.current_stream(qkv.device)), "dcae_op_window_attention_backward")
+        return dqkv, None, None, None, drel
+
+
+def window_attention(qkv, head_dim: int, window: int, shift: int, rel):
+    return WindowAttentionFunction.apply(qkv, head_dim, window, shift, rel)
+
+
+class TransformStackFunction(torch.autograd.Function):
+    """y = stack(x; params) as ONE autograd node: forward = `TransformStack.forward` (the kernels, in the stack's math mode),
+    backward = recompute `transform_graph.stack` on the saved input with `WindowAttentionFunction` + torch.autograd.grad.
+    `keys`: the state-dict key of each parameter, with or without the stack prefix.  The recompute's dense layers and
+    convolutions are torch ops and follow torch's TF32 settings."""
+
+    @staticmethod
+    def forward(ctx, engine: TransformStack, keys, x, *params):
+        ctx.engine, ctx.keys = engine, [k[len(engine.stack) + 1:] if k.startswith(engine.stack + ".") else k for k in keys]
+        ctx.save_for_backward(x, *params)
+        return engine.forward(x)
+
+    @staticmethod
+    def backward(ctx, g):
+        x, *params = ctx.saved_tensors
+        with torch.enable_grad():
+            leaf = x.detach().requires_grad_(True)
+            plist = [p.detach().requires_grad_(True) for p in params]
+            out = transform_graph.stack(ctx.engine.stack, dict(zip(ctx.keys, plist)), leaf, attn=window_attention)
+            grads = torch.autograd.grad(out, [leaf] + plist, g, allow_unused=True)
+        return (None, None) + tuple(grads)
+
+
+class TransformModel(nn.Module):
+    """One transform stack (g_a / g_s / h_a / h_z_s1 / h_z_s2) as a trainable module: parameters in a ParameterList, `keys`
+    holds the reference's state-dict key of each ('g_a.0.conv.weight'; `reference_state_dict()` gives the mapping back),
+    forward(x NCHW) = the stack.  No-grad calls run the kernels only (the bits of `TransformStack.forward`); calls under
+    autograd go through `TransformStackFunction`.  The packed device weights follow the parameters (repacked when their
+    version counters or addresses change, i.e. after an optimizer step or load)."""
+
+    def __init__(self, stack: str, params: Optional[Dict[str, torch.Tensor]] = None, device="cuda:0", math: str = "f16x3", seed: int = 0):
+        super().__init__()
+        params = params if params is not None else init_transform_params(seed, (stack,))
+        self.stack = stack
+        self.keys = [f"{stack}.{k}" for k in transform_param_shapes(stack)]
+        vals = [params.get(k, params.get(k[len(stack) + 1:])) for k in self.keys]
+        missing = [k for k, v in zip(self.keys, vals) if v is None]
+        if missing:
+            raise KeyError(f"{stack}: missing parameters {missing[:3]}")
+        self.plist = nn.ParameterList([nn.Parameter(v.detach().clone().to(device, torch.float32)) for v in vals])
+        self.engine = [TransformStack(stack, self.reference_state_dict(), device=device, math=math)]
+        self._sig = self._signature()
+
+    def _signature(self):
+        return tuple((p.data_ptr(), p._version) for p in self.plist)
+
+    def reference_state_dict(self) -> Dict[str, torch.Tensor]:
+        return {k: p.detach() for k, p in zip(self.keys, self.plist)}
+
+    def sync(self) -> None:
+        if self._signature() != self._sig:
+            self.engine[0].refresh(self.reference_state_dict())
+            self._sig = self._signature()
+
+    def forward(self, x: torch.Tensor) -> torch.Tensor:
+        self.sync()
+        if torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in self.plist)):
+            return TransformStackFunction.apply(self.engine[0], self.keys, x, *self.plist)
+        return self.engine[0].forward(x)
 
 
 def rate_distortion_loss(likelihoods: torch.Tensor, y_hat: torch.Tensor, target: torch.Tensor, num_pixels: int, lmbda: float = 0.013):

@@ -558,6 +558,13 @@ class TransformStack:
             raise ValueError(f"unknown stack {stack!r}; one of {STACKS}")
         self.stack = stack
         self.K = kernels if kernels is not None else LibKernels(device, math)
+        self._pack(params)
+        first, last = ARCH[stack][0], ARCH[stack][-1]
+        self.c_in = first[1]
+        self.c_out = last[2]
+
+    def _pack(self, params: Dict[str, torch.Tensor]) -> None:
+        stack = self.stack
         P = {}
         for key, shape in transform_param_shapes(stack).items():
             t = params.get(key, params.get(f"{stack}.{key}"))
@@ -567,30 +574,35 @@ class TransformStack:
                 raise ValueError(f"{stack}.{key}: expected shape {shape}, got {tuple(t.shape)}")
             P[key] = t.detach().to(torch.float32)
         K = self.K
-        self.blocks: list = []
+        blocks: list = []
         for idx, spec in enumerate(ARCH[stack]):
             p = f"{idx}."
             kind = spec[0]
             if kind == "rbws":
                 _, cin, cout = spec
-                self.blocks.append(("conv", _ConvS2(K, P[p + "conv.weight"], P[p + "conv.bias"], cin, cout)))
-                self.blocks += [("rbb", _ResidualBottleneck(K, P, p + f"res{r}.", cout)) for r in (1, 2, 3)]
+                blocks.append(("conv", _ConvS2(K, P[p + "conv.weight"], P[p + "conv.bias"], cin, cout)))
+                blocks += [("rbb", _ResidualBottleneck(K, P, p + f"res{r}.", cout)) for r in (1, 2, 3)]
             elif kind == "rbwu":
                 _, cin, cout = spec
-                self.blocks += [("rbb", _ResidualBottleneck(K, P, p + f"res{r}.", cin)) for r in (1, 2, 3)]
-                self.blocks.append(("deconv", _DeconvS2(K, P[p + "conv.weight"], P[p + "conv.bias"], cin, cout)))
+                blocks += [("rbb", _ResidualBottleneck(K, P, p + f"res{r}.", cin)) for r in (1, 2, 3)]
+                blocks.append(("deconv", _DeconvS2(K, P[p + "conv.weight"], P[p + "conv.bias"], cin, cout)))
             elif kind == "conv_s2":
                 _, cin, cout, _k = spec
-                self.blocks.append(("conv", _ConvS2(K, P[p + "weight"], P[p + "bias"], cin, cout)))
+                blocks.append(("conv", _ConvS2(K, P[p + "weight"], P[p + "bias"], cin, cout)))
             elif kind == "deconv_s2":
                 _, cin, cout, _k = spec
-                self.blocks.append(("deconv", _DeconvS2(K, P[p + "weight"], P[p + "bias"], cin, cout)))
+                blocks.append(("deconv", _DeconvS2(K, P[p + "weight"], P[p + "bias"], cin, cout)))
             elif kind == "swin":
                 _, c, hd, win, n = spec
-                self.blocks.append(("swin", _Swin(K, P, p, c, hd, win, n)))
-        first, last = ARCH[stack][0], ARCH[stack][-1]
-        self.c_in = first[1]
-        self.c_out = last[2]
+                blocks.append(("swin", _Swin(K, P, p, c, hd, win, n)))
+        self.blocks = blocks
+
+    def refresh(self, params: Dict[str, torch.Tensor]) -> None:
+        """Repack the weights in place from a new state dict (same keys as the constructor takes), e.g. after an optimizer
+        step or `load_state_dict`.  The previous packed tensors are released once no queued launch uses them."""
+        if isinstance(self.K, LibKernels):
+            torch.cuda.synchronize(self.K.device)
+        self._pack(params)
 
     # widest intermediate of a stack, in fp32 elements per input position (tokens of the finest level x its widest buffer,
     # the fc1 output of 4 C columns): the element-wise kernels address with 32-bit offsets, so one call must stay below 2^32
@@ -625,16 +637,25 @@ class TransformStack:
 
 def accelerate_transforms(net: torch.nn.Module, device="cuda:0", math: str = "f16x3", stacks: Sequence[str] = STACKS) -> Dict[str, TransformStack]:
     """Redirect `net.g_a / g_s / h_a / h_z_s1 / h_z_s2` of a reference `DCAE` instance to the CUDA library, in place
-    (instance-level `forward`, the modules and their parameters stay where they are, like `accelerate`).  Inference only:
-    the weights are packed once from the module's current parameters; call again after they change."""
+    (instance-level `forward`, the modules and their parameters stay where they are, like `accelerate`).  The packed
+    weights follow the module's parameters: they are repacked when a parameter's version counter or address changed
+    (an optimizer step, `load_state_dict`).  Under autograd a call becomes one `training.TransformStackFunction` node
+    over the module's own parameters -- kernels forward, recompute backward -- so gradients land in `net.parameters()`."""
     out = {}
     for name in stacks:
         mod = getattr(net, name)
+        tracked = dict(list(mod.named_parameters()) + list(mod.named_buffers()))
         ts = TransformStack(name, {k: v.detach() for k, v in mod.state_dict().items()}, device=device, math=math)
+        sig = [tuple((t.data_ptr(), t._version) for t in tracked.values())]
 
-        def fwd(x, ts=ts):
-            if torch.is_grad_enabled() and x.requires_grad:
-                raise _lib.DcaeError("dcae_b200 transform stacks are forward-only: wrap the call in torch.no_grad()")
+        def fwd(x, ts=ts, tracked=tracked, sig=sig):
+            now = tuple((t.data_ptr(), t._version) for t in tracked.values())
+            if now != sig[0]:
+                ts.refresh({k: v.detach() for k, v in tracked.items()})
+                sig[0] = now
+            if torch.is_grad_enabled() and (x.requires_grad or any(t.requires_grad for t in tracked.values())):
+                from .training import TransformStackFunction
+                return TransformStackFunction.apply(ts, list(tracked), x, *tracked.values())
             return ts.forward(x)
 
         mod.forward = fwd

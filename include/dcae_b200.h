@@ -285,6 +285,23 @@ int dcae_op_nchw_to_tokens_i32(const int32_t* src, int32_t B, int32_t C, int64_t
 int dcae_op_window_attention(const float* qkv, int64_t ld, int32_t q_col, int32_t k_col, int32_t v_col, int32_t C,
                              int32_t head_dim, int32_t window, int32_t shift, const float* rel_bias, int32_t B, int32_t h,
                              int32_t w, float* out, int64_t out_ld, const dcae_planes* out16, void* stream);
+/* Backward of dcae_op_window_attention, same qkv / window / head_dim / shift / rel_bias arguments, plus the output
+ * cotangent dout [T, dout_ld] (columns e*hd.. of head e).  Per window and head, s = 1/sqrt(hd), with S and P recomputed
+ * exactly as the forward computes them:
+ *   dP = dO V^T;  D_i = sum_j P_ij dP_ij;  dS = P o (dP - D);  dQ = s dS K;  dK = s dS^T Q;  dV = P^T dO
+ *   drel[e, dy, dx] = sum of dS over every (query, key) pair at that offset, in every window and image (masked pairs add 0)
+ * dq / dk / dv are written into the q_col / k_col / v_col column windows of dqkv [T, dqkv_ld] (the three windows must not
+ * overlap; other columns are left untouched); drel [n_heads, 2*window-1, 2*window-1] is overwritten.  dqkv must not alias
+ * qkv or dout.  scratch: device memory of at least dcae_window_attention_backward_scratch_bytes() bytes (16-byte aligned),
+ * per-block partial sums of drel; its size does not grow with the image beyond a fixed number of blocks.  Deterministic, no
+ * atomics: every dqkv element has one writer, drel is summed in a fixed order that depends on the shape only, and the dqkv
+ * rows of an image do not depend on the rest of the batch.  8x8 windows run on warp-level TF32 MMAs with the 3-pass split,
+ * 4x4 windows on FFMA.  Work booked: 10 T window^2 C flop. */
+size_t dcae_window_attention_backward_scratch_bytes(int32_t B, int32_t h, int32_t w, int32_t C, int32_t head_dim, int32_t window);
+int dcae_op_window_attention_backward(const float* qkv, int64_t ld, int32_t q_col, int32_t k_col, int32_t v_col, int32_t C,
+                                      int32_t head_dim, int32_t window, int32_t shift, const float* rel_bias,
+                                      int32_t B, int32_t h, int32_t w, const float* dout, int64_t dout_ld,
+                                      float* dqkv, int64_t dqkv_ld, float* drel, void* scratch, size_t scratch_bytes, void* stream);
 /* out[(b, y', x'), (sy*2 + sx)*Cs + c] = x[(b, 2y' + sy, 2x' + sx), c] for c < C, 0 elsewhere (c >= C, odd edge);
  * output grid ceil(h/2) x ceil(w/2), 4*Cs columns.  With the weights re-indexed at pack time a stride-2 k x k
  * convolution (conv(), dcae.py:35-42) becomes a stride-1 3x3 convolution over this image (dcae_op_gemm, taps = 9). */
