@@ -13,6 +13,8 @@ Public surface (mirrors the reference's operator interface for this path only):
                         accelerate_transforms also trains: under autograd each stack call is a recompute node
   TransformModel        -- one transform stack as a trainable module (kernels forward, recompute backward with the
                            window-attention backward kernel; dcae_b200/training.py)
+  EntropyBottleneckModel, DCAEModel, dcae_rate_distortion_loss -- the trainable bottleneck (backward kernel
+                           dcae_eb_backward) and the whole DCAE as one trainable module (dcae_b200/training.py)
   DCAECodec             -- the whole model (forward / compress / decompress / update, image <-> .bin container) from a reference state dict
   container             -- the reference's bitstream container and image padding (compress_and_decompress.py:48-148)
 """
@@ -30,7 +32,8 @@ def __getattr__(name):
     if name in ("accelerate", "DictCrossAttention", "ConvStack"):
         from . import modules
         return getattr(modules, name)
-    if name in ("EntropyModel", "SliceLoopFunction", "GaussianLikelihoodFunction", "rate_distortion_loss", "TransformModel"):
+    if name in ("EntropyModel", "SliceLoopFunction", "GaussianLikelihoodFunction", "rate_distortion_loss", "TransformModel",
+                "EntropyBottleneckFunction", "EntropyBottleneckModel", "DCAEModel", "dcae_rate_distortion_loss"):
         from . import training
         return getattr(training, name)
     if name == "EntropyBottleneck":

@@ -60,6 +60,12 @@ class EbArgs(C.Structure):
                 ("z_hat", c_f32p), ("lik", c_f32p), ("sym", c_i32p)]
 
 
+class EbBwdArgs(C.Structure):
+    _fields_ = [("z", c_f32p), ("noise", c_f32p), ("params", c_f32p), ("medians", c_f32p), ("grad_lik", c_f32p),
+                ("mode", C.c_int32), ("B", C.c_int32), ("C", C.c_int32), ("HW", C.c_int64), ("lik_bound", C.c_float),
+                ("grad_z", c_f32p), ("grad_params", c_f32p)]
+
+
 class Operand(C.Structure):
     _fields_ = [("base", c_f32p), ("ld", C.c_int64), ("col0", C.c_int32), ("k0", C.c_int32),
                 ("col1", C.c_int32), ("k1", C.c_int32), ("taps", C.c_int32),
@@ -130,6 +136,7 @@ SIGNATURES = {
     "dcae_gc_fused": (C.c_int, [C.POINTER(GcArgs), _P]),
     "dcae_gc_backward": (C.c_int, [C.POINTER(GcBwdArgs), _P]),
     "dcae_eb_fused": (C.c_int, [C.POINTER(EbArgs), _P]),
+    "dcae_eb_backward": (C.c_int, [C.POINTER(EbBwdArgs), _P]),
     "dcae_gc_num_partials": (_I64, [_I64, _I64]),
     "dcae_reduce_partials": (C.c_int, [_P, _I64, _P, _P]),
     "dcae_op_gemm": (C.c_int, [C.POINTER(Operand), C.POINTER(Weight), C.POINTER(Epilogue), C.c_int, _P]),

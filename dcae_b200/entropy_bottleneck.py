@@ -65,12 +65,16 @@ class EntropyBottleneck(nn.Module):
     def _get_medians(self) -> torch.Tensor:
         return self.quantiles[:, :, 1:2]
 
-    def _logits_cumulative(self, inputs: torch.Tensor) -> torch.Tensor:
+    def _logits_cumulative(self, inputs: torch.Tensor, stop_gradient: bool = False) -> torch.Tensor:
+        """stop_gradient (compressai's keyword): the density parameters enter detached, so only `inputs` is differentiated."""
+        def param(name):
+            t = getattr(self, name)
+            return t.detach() if stop_gradient else t
         logits = inputs
         for i in range(len(self.filters) + 1):
-            logits = torch.matmul(F.softplus(getattr(self, f"_matrix{i}")), logits) + getattr(self, f"_bias{i}")
+            logits = torch.matmul(F.softplus(param(f"_matrix{i}")), logits) + param(f"_bias{i}")
             if i < len(self.filters):
-                logits = logits + torch.tanh(getattr(self, f"_factor{i}")) * torch.tanh(logits)
+                logits = logits + torch.tanh(param(f"_factor{i}")) * torch.tanh(logits)
         return logits
 
     def loss(self) -> torch.Tensor:

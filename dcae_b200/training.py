@@ -16,20 +16,32 @@ recompute graph; the windowed attention core keeps a kernel backward, `dcae_op_w
   TransformStackFunction       one stack call as one autograd node (forward = `TransformStack.forward`)
   TransformModel               nn.Module owning one stack's parameters, the transform counterpart of EntropyModel
 
+and for the hyper-latent entropy bottleneck and the whole model:
+
+  EntropyBottleneckFunction    the bottleneck's likelihood with the library's forward and backward kernels
+                               (`dcae_eb_fused`, `dcae_eb_backward`)
+  EntropyBottleneckModel       `EntropyBottleneck` that trains (same keys); aux loss with compressai's stop_gradient
+  DCAEModel                    the whole DCAE (dcae.py:623-677) as one trainable nn.Module over the reference's keys
+
 Gradients are the exact gradients of the fp32 graph (the forward values agree with it to 1e-5, tests/test_gpu_training.py
 pins gradient parity against the reference's own modules under torch autograd).
 """
 from __future__ import annotations
 
+import math as _math
 from typing import Dict, Optional
 
 import torch
 import torch.nn as nn
+import torch.nn.functional as F
 
 from . import _lib, torch_graph, transform_graph
-from .entropy_model import EntropySliceLoop
+from .entropy_bottleneck import EntropyBottleneck
+from .entropy_model import EntropySliceLoop, get_scale_table
+from .gaussian_conditional import GaussianConditional
+from .modules import HOT_PREFIXES
 from .params import init_entropy_params
-from .transforms import TransformStack, init_transform_params, transform_param_shapes
+from .transforms import STACKS, TransformStack, init_transform_params, transform_param_shapes
 
 
 def _rows(t: torch.Tensor):
@@ -290,3 +302,194 @@ def rate_distortion_loss(likelihoods: torch.Tensor, y_hat: torch.Tensor, target:
     bpp = torch.log(likelihoods).sum() / (-math.log(2) * num_pixels)
     mse = torch.mean((y_hat - target) ** 2)
     return lmbda * 255 ** 2 * mse + bpp, bpp, mse
+
+
+def dcae_rate_distortion_loss(out: dict, target: torch.Tensor, lmbda: float = 0.013):
+    """train.py:82-88 with type='mse' for the whole model: bpp = sum over BOTH likelihood tensors (y and z) of
+    sum(log lik) / (-ln 2 * pixels), pixels = N * H * W of the image; loss = lmbda * 255^2 * mse(x_hat, target) + bpp.
+    -> (loss, bpp, mse)."""
+    N, _, H, W = target.shape
+    pixels = N * H * W
+    bpp = sum(torch.log(lik).sum() / (-_math.log(2) * pixels) for lik in out["likelihoods"].values())
+    mse = F.mse_loss(out["x_hat"], target)
+    return lmbda * 255 ** 2 * mse + bpp, bpp, mse
+
+
+# ---- the hyper-latent entropy bottleneck ---------------------------------------------------------------------------------
+
+class EntropyBottleneckFunction(torch.autograd.Function):
+    """(lik, z_hat) = compressai EntropyBottleneck likelihood of z [B, C, h, w] (dcae.py:630) with the packed density
+    `params` [C, 58] (softplus(_matrix*) | _bias* | tanh(_factor*), as `EntropyBottleneck._pack` lays them out) and
+    `medians` [C] (no gradient, compressai detaches them).  noise given: training mode, out = z + noise; None: eval mode,
+    out = round(z - median) + median.  Forward dcae_eb_fused, backward dcae_eb_backward; the packed tensor is built under
+    autograd by the caller, so torch chains its gradient back to _matrix* / _bias* / _factor*.  z_hat = round(z - median)
+    + median in both modes, not differentiable (the caller attaches the straight-through gradient)."""
+
+    @staticmethod
+    def forward(ctx, z, noise, params, medians, lik_bound: float):
+        z, params, medians = z.contiguous().float(), params.contiguous().float(), medians.contiguous().float()
+        noise = noise.contiguous().float() if noise is not None else None
+        B, C, h, w = z.shape
+        lik, z_hat = torch.empty_like(z), torch.empty_like(z)
+        a = _lib.EbArgs()
+        a.z, a.params, a.medians = z.data_ptr(), params.data_ptr(), medians.data_ptr()
+        a.mode = _lib.GC_NOISE if noise is not None else _lib.GC_EVAL
+        if noise is not None:
+            a.noise = noise.data_ptr()
+        a.B, a.C, a.HW, a.lik_bound = B, C, h * w, lik_bound
+        a.z_hat, a.lik = z_hat.data_ptr(), lik.data_ptr()
+        if z.numel():
+            with torch.cuda.device(z.device):
+                _lib.check(_lib.load().dcae_eb_fused(a, _lib.current_stream(z.device)), "dcae_eb_fused")
+        ctx.save_for_backward(z, noise if noise is not None else z.new_empty(0), params, medians)
+        ctx.lik_bound = lik_bound
+        ctx.mark_non_differentiable(z_hat)
+        return lik, z_hat
+
+    @staticmethod
+    def backward(ctx, g_lik, _g_zhat):
+        z, noise, params, medians = ctx.saved_tensors
+        noisy = noise.numel() > 0
+        B, C, h, w = z.shape
+        g_lik = g_lik.contiguous().float()
+        gz, gp = torch.empty_like(z), torch.empty_like(params)
+        a = _lib.EbBwdArgs()
+        a.z, a.params, a.medians, a.grad_lik = z.data_ptr(), params.data_ptr(), medians.data_ptr(), g_lik.data_ptr()
+        a.mode = _lib.GC_NOISE if noisy else _lib.GC_EVAL
+        if noisy:
+            a.noise = noise.data_ptr()
+        a.B, a.C, a.HW, a.lik_bound = B, C, h * w, ctx.lik_bound
+        a.grad_z, a.grad_params = gz.data_ptr(), gp.data_ptr()
+        with torch.cuda.device(z.device):
+            _lib.check(_lib.load().dcae_eb_backward(a, _lib.current_stream(z.device)), "dcae_eb_backward")
+        return gz, None, gp, None, None
+
+
+class EntropyBottleneckModel(EntropyBottleneck):
+    """`dcae_b200.EntropyBottleneck` that trains: the same parameter and buffer names (state dicts move either way between
+    it, `EntropyBottleneck` and `DCAECodec`).  Calls under autograd go through `EntropyBottleneckFunction` with the packed
+    density built differentiably; calls without autograd are `EntropyBottleneck.forward`'s launch, bit for bit.
+    `loss()` is compressai's aux loss: stop_gradient=True, so its gradient reaches `quantiles` only."""
+
+    def _pack_graph(self, device) -> torch.Tensor:
+        """[C, 58] as `_pack` builds it, under autograd."""
+        parts = [F.softplus(getattr(self, f"_matrix{i}")).reshape(self.channels, -1) for i in range(5)]
+        parts += [getattr(self, f"_bias{i}").reshape(self.channels, -1) for i in range(5)]
+        parts += [torch.tanh(getattr(self, f"_factor{i}")).reshape(self.channels, -1) for i in range(4)]
+        return torch.cat(parts, dim=1).to(device, torch.float32)
+
+    def forward_parts(self, x: torch.Tensor, training: Optional[bool] = None, noise: Optional[torch.Tensor] = None):
+        """-> (outputs, likelihood, z_hat): outputs as compressai's forward returns them (x + noise in training mode,
+        round(x - median) + median otherwise) and z_hat = round(x - median) + median, the value dcae.py:631-633 passes on."""
+        if training is None:
+            training = self.training
+        if training and noise is None:
+            noise = torch.empty_like(x).uniform_(-0.5, 0.5)
+        if not training:
+            noise = None
+        if not x.is_cuda:
+            raise _lib.DcaeError("dcae_b200.EntropyBottleneckModel runs on CUDA tensors only (no CPU fallback)")
+        if len(x.shape) != 4 or x.shape[1] != self.channels:
+            raise ValueError(f"expected [B, {self.channels}, h, w], got {tuple(x.shape)}")
+        if not (torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in self.parameters()))):
+            o = self._run(_lib.GC_NOISE if noise is not None else _lib.GC_EVAL, x, noise=noise, want=("z_hat", "lik"))
+            return (x + noise if noise is not None else o["z_hat"]), o["lik"], o["z_hat"]
+        med = self.quantiles[:, 0, 1].detach().to(x.device, torch.float32)
+        lik, z_hat = EntropyBottleneckFunction.apply(x, noise, self._pack_graph(x.device), med, self.likelihood_bound)
+        return (x + noise if noise is not None else z_hat), lik, z_hat
+
+    def forward(self, x: torch.Tensor, training: Optional[bool] = None, noise: Optional[torch.Tensor] = None):
+        """-> (outputs, likelihood) like compressai (dcae.py:630)."""
+        out, lik, _ = self.forward_parts(x, training, noise)
+        return out, lik
+
+    def loss(self) -> torch.Tensor:
+        """aux loss (train.py:177) as compressai computes it: sum |logits_cumulative(quantiles) - target| with the density
+        parameters detached."""
+        return torch.abs(self._logits_cumulative(self.quantiles, stop_gradient=True) - self.target).sum()
+
+
+def init_entropy_bottleneck_params(seed: int = 0, channels: int = 192) -> Dict[str, torch.Tensor]:
+    """compressai's EntropyBottleneck initialisation (matrices log(expm1(1 / scale / fan)), biases U(-1/2, 1/2), factors 0,
+    quantiles [-10, 0, 10]) from a fixed seed, under the reference's `entropy_bottleneck.` keys (parameters only)."""
+    with torch.random.fork_rng(devices=[]):
+        torch.manual_seed(seed)
+        eb = EntropyBottleneck(channels)
+    return {f"entropy_bottleneck.{k}": v.detach() for k, v in eb.named_parameters()}
+
+
+# ---- the whole model ---------------------------------------------------------------------------------------------------
+
+class DCAEModel(nn.Module):
+    """The whole DCAE as one trainable module (dcae.py:623-677): five `TransformModel`s (g_a, g_s, h_a, h_z_s1, h_z_s2), the
+    slice loop as an `EntropyModel` (one lane), an `EntropyBottleneckModel(192)` and a `GaussianConditional` holding the
+    scale table.  `params`: a reference state dict (the keys `DCAECodec` takes); missing -> seeded initialisation.
+    Every hot path runs on the library's kernels forward; backward is the kernels' backward (likelihoods, window attention)
+    and torch recompute elsewhere.  `reference_state_dict()` loads into `DCAECodec` (compress / decompress) and back."""
+
+    def __init__(self, params: Optional[Dict[str, torch.Tensor]] = None, device="cuda:0", math: str = "f16x3", seed: int = 0,
+                 likelihood_math: str = "fast"):
+        super().__init__()
+        if params is None:
+            params = dict(init_entropy_params(seed))
+            params.update(init_transform_params(seed))
+            params.update(init_entropy_bottleneck_params(seed))
+        for name in STACKS:
+            self.add_module(name, TransformModel(name, params, device=device, math=math))
+        hot = {k: v for k, v in params.items() if k.split(".")[0] in HOT_PREFIXES}
+        self.entropy = EntropyModel(hot, device=device, math=math, lanes=1, likelihood_math=likelihood_math)
+        self.entropy_bottleneck = EntropyBottleneckModel(192)
+        eb = {k[len("entropy_bottleneck."):]: v for k, v in params.items() if k.startswith("entropy_bottleneck.")}
+        if eb:
+            self.entropy_bottleneck.load_state_dict(eb, strict=False)
+        self.entropy_bottleneck.to(device)
+        table = params.get("gaussian_conditional.scale_table")
+        table = table if table is not None and table.numel() else get_scale_table()
+        self.gaussian_conditional = GaussianConditional(table.tolist(), likelihood_math=likelihood_math)
+        gc = {k[len("gaussian_conditional."):]: v for k, v in params.items() if k.startswith("gaussian_conditional.")}
+        if gc:
+            self.gaussian_conditional.load_state_dict(gc, strict=False)
+        self.gaussian_conditional.to(device)
+
+    def forward(self, x: torch.Tensor, y_noise: Optional[torch.Tensor] = None, z_noise: Optional[torch.Tensor] = None) -> dict:
+        """-> {"x_hat", "likelihoods": {"y", "z"}, "para": {"means", "scales", "y"}} (dcae.py:623-677).  A given noise tensor
+        (U(-1/2, 1/2), shaped like y / z) selects the training-mode likelihood for its part; in train() mode missing
+        noise is drawn, in eval() mode the latents are rounded."""
+        y = self.g_a(x)
+        z = self.h_a(y)
+        if self.training and z_noise is None:
+            z_noise = torch.empty_like(z).uniform_(-0.5, 0.5)
+        _, z_lik, z_hat = self.entropy_bottleneck.forward_parts(z, training=z_noise is not None, noise=z_noise)
+        if torch.is_grad_enabled() and z.requires_grad:
+            z_hat = z_hat + (z - z.detach())           # ste_round(z - median) + median: the value round() gives, gradient 1
+        latent_scales, latent_means = self.h_z_s1(z_hat), self.h_z_s2(z_hat)
+        o = self.entropy(y, latent_scales, latent_means, noise=y_noise)
+        x_hat = self.g_s(o["y_hat"])
+        return {"x_hat": x_hat, "likelihoods": {"y": o["likelihoods"], "z": z_lik},
+                "para": {"means": o["means"], "scales": o["scales"], "y": y}}
+
+    def aux_loss(self) -> torch.Tensor:
+        """train.py:177: the bottleneck's aux loss (gradient to `quantiles` only)."""
+        return self.entropy_bottleneck.loss()
+
+    def parameter_groups(self):
+        """-> (main, aux): the optimizer split of train.py -- every `*.quantiles` in aux, everything else in main."""
+        named = list(self.named_parameters())
+        return ([p for n, p in named if not n.endswith(".quantiles")], [p for n, p in named if n.endswith(".quantiles")])
+
+    def reference_state_dict(self) -> Dict[str, torch.Tensor]:
+        """Every parameter under the reference's key, plus the entropy bottleneck's and the Gaussian conditional's buffers:
+        what `DCAECodec` consumes, and what this class's constructor takes back."""
+        sd: Dict[str, torch.Tensor] = {}
+        for name in STACKS:
+            sd.update(getattr(self, name).reference_state_dict())
+        sd.update(self.entropy.reference_state_dict())
+        sd.update({f"entropy_bottleneck.{k}": v.detach() for k, v in self.entropy_bottleneck.state_dict().items()})
+        sd.update({f"gaussian_conditional.{k}": v.detach() for k, v in self.gaussian_conditional.state_dict().items()})
+        return sd
+
+    def update(self, force: bool = False) -> bool:
+        """compressai's update(): the coder tables of both entropy models (dcae.py:616-621)."""
+        updated = self.gaussian_conditional.update_scale_table(self.gaussian_conditional.scale_table, force=force)
+        updated |= self.entropy_bottleneck.update(force=force)
+        return updated

@@ -154,6 +154,24 @@ typedef struct {
   float* z_hat; float* lik; int32_t* sym;
 } dcae_eb_args;
 int dcae_eb_fused(const dcae_eb_args* a, void* stream);
+/* Backward of dcae_eb_fused's likelihood for the training step (train.py:165-179 differentiates the rate of z through
+ * compressai's EntropyBottleneck.forward).  Given dL/dlik [B, C, HW] it overwrites
+ *   grad_z [B, C, HW]    dL/dz through out = z + noise (NOISE); all zeros in EVAL mode, where round() passes no gradient
+ *   grad_params [C, 58]  dL/d of the PACKED values softplus(_matrix*), _bias*, tanh(_factor*) in dcae_eb_fused's layout
+ * with compressai's LowerBound rule for the likelihood floor (the gradient passes where lik >= lik_bound or where it is
+ * negative).  The medians get no gradient (compressai detaches them).  mode: DCAE_GC_EVAL or DCAE_GC_NOISE.
+ * Deterministic, no atomics: one block per channel sums the channel's B*HW elements in an order fixed by the shape, and
+ * every grad_z element depends on its own element only (an image's rows do not depend on the rest of the batch). */
+typedef struct {
+  const float* z; const float* noise;
+  const float* params; const float* medians;
+  const float* grad_lik;
+  int32_t mode;            /* DCAE_GC_EVAL / DCAE_GC_NOISE */
+  int32_t B, C; int64_t HW;
+  float lik_bound;
+  float* grad_z; float* grad_params;
+} dcae_eb_bwd_args;
+int dcae_eb_backward(const dcae_eb_bwd_args* a, void* stream);
 
 /* --------------------------------------------------------------------------------------------
  * Elementary token-major operators (each replaces one torch dispatch chain of dcae.py:300-509).
