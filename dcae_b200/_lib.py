@@ -66,6 +66,26 @@ class EbBwdArgs(C.Structure):
                 ("grad_z", c_f32p), ("grad_params", c_f32p)]
 
 
+class CoderTables(C.Structure):
+    _fields_ = [("cdfs", C.c_void_p), ("cdf_stride", C.c_int32), ("cdf_sizes", C.c_void_p), ("offsets", C.c_void_p),
+                ("n_cdfs", C.c_int32)]
+
+
+class IlvEncArgs(C.Structure):
+    _fields_ = [("symbols", c_i32p), ("indexes", c_i32p), ("B", C.c_int32), ("h", C.c_int32), ("w", C.c_int32),
+                ("lanes", C.c_int32), ("tables", CoderTables), ("scratch", C.c_void_p), ("scratch_bytes", C.c_size_t),
+                ("sizes", C.c_void_p), ("out", C.c_void_p), ("out_capacity", C.c_int64), ("status", c_i32p)]
+
+
+class IlvDecArgs(C.Structure):
+    _fields_ = [("strings", C.c_void_p), ("bounds", C.c_void_p), ("indexes", c_i32p), ("slice", C.c_int32),
+                ("B", C.c_int32), ("h", C.c_int32), ("w", C.c_int32), ("tables", CoderTables), ("symbols", c_i32p),
+                ("status", c_i32p)]
+
+
+ILV_STATUS = {1: "malformed header", 2: "corrupt stream", 3: "index outside the coder tables", 4: "unusable coder table row"}
+
+
 class Operand(C.Structure):
     _fields_ = [("base", c_f32p), ("ld", C.c_int64), ("col0", C.c_int32), ("k0", C.c_int32),
                 ("col1", C.c_int32), ("k1", C.c_int32), ("taps", C.c_int32),
@@ -159,6 +179,10 @@ SIGNATURES = {
     "dcae_op_tokens_to_nchw": (C.c_int, [_P, _I64, _I32, _I32, _I64, _P, _P]),
     "dcae_op_tokens_to_nchw_i32": (C.c_int, [_P, _I64, _I32, _I32, _I64, _P, _P]),
     "dcae_op_nchw_to_tokens_i32": (C.c_int, [_P, _I32, _I32, _I64, _P, _I64, _P]),
+    "dcae_ilv_encode_scratch_bytes": (C.c_size_t, [_I32, _I32, _I32, _I32]),
+    "dcae_ilv_encode_max_bytes": (_I64, [_I32, _I32, _I32, _I32]),
+    "dcae_ilv_encode": (C.c_int, [C.POINTER(IlvEncArgs), _P]),
+    "dcae_ilv_decode": (C.c_int, [C.POINTER(IlvDecArgs), _P]),
     "dcae_slice_loop_workspace_bytes": (C.c_size_t, [_I32, _I32, _I32]),
     "dcae_slice_loop_create": (C.c_int, [C.POINTER(_P), _I32, _I32, _I32, C.POINTER(SliceWeights), _P, _I32, _P, C.c_size_t, C.c_int]),
     "dcae_slice_loop_check_f16_range": (C.c_int, [_P, _I32, C.POINTER(C.c_ulonglong)]),

@@ -40,6 +40,9 @@ SIGNATURES = {
     "dcae_rans_decoder_set_stream": (C.c_int, [_P, C.c_char_p, _I64]),
     "dcae_rans_decoder_decode_stream": (C.c_int, [_P, _P, _I32, _I64, C.POINTER(RansTables), _P]),
     "dcae_pmf_to_quantized_cdf": (C.c_int, [_P, _I32, _I32, _P]),
+    "dcae_rans_ilv_max_bytes": (_I64, [_I64, _I32]),
+    "dcae_rans_ilv_encode": (_I64, [_P, _P, _I64, _I32, C.POINTER(RansTables), _P, _I64]),
+    "dcae_rans_ilv_decode": (C.c_int, [C.c_char_p, _I64, _P, _I64, C.POINTER(RansTables), _P]),
 }
 
 _lib = None
@@ -161,6 +164,46 @@ class RansDecoder:
     def decode_stream(self, indexes, cdf, cdf_lengths, offsets) -> Sequence[int]:
         """The reference's call (dcae.py:893): returns a list, as compressai does."""
         return self.decode_array(indexes, cdf, cdf_lengths, offsets).tolist()
+
+
+ILV_SLICES = 5
+ILV_LANES = (1, 2, 4, 8, 16, 32)
+
+
+def _slices(x, what) -> np.ndarray:
+    a = _array(x, allow=(np.int32,))
+    if a.size % ILV_SLICES:
+        raise RansError(f"{what}: expected {ILV_SLICES} slices of equal length, got {a.size} values")
+    return a
+
+
+def encode_interleaved(symbols, indexes, cdf, cdf_lengths, offsets, lanes: int = 32) -> bytes:
+    """The ilv1 string of one image (include/dcae_rans.h): symbols / indexes [5, n] (the image's five slices, each in
+    coder order), coded on `lanes` interleaved rANS states.  The host reference of the sm_100a encoder."""
+    s, i = _slices(symbols, "symbols"), _slices(indexes, "indexes")
+    if s.size != i.size:
+        raise RansError("symbols and indexes differ in length")
+    n = s.size // ILV_SLICES
+    tab = _Tables()                              # owns the arrays the struct points at until the call returns
+    t = tab.get(cdf, cdf_lengths, offsets)
+    cap = int(load().dcae_rans_ilv_max_bytes(n, lanes))
+    _check(cap, "ilv_max_bytes")
+    out = np.empty(cap, dtype=np.uint8)
+    size = int(load().dcae_rans_ilv_encode(s.ctypes.data, i.ctypes.data, n, lanes, C.byref(t), out.ctypes.data, cap))
+    _check(size, "ilv_encode")
+    return out[:size].tobytes()
+
+
+def decode_interleaved(data: bytes, indexes, cdf, cdf_lengths, offsets) -> np.ndarray:
+    """ilv1 string + indexes [5, n] -> int32 symbols [5, n]; raises RansError on a malformed or corrupt string."""
+    i = _slices(indexes, "indexes")
+    out = np.empty(i.size, dtype=np.int32)
+    tab = _Tables()
+    t = tab.get(cdf, cdf_lengths, offsets)
+    data = bytes(data)
+    _check(load().dcae_rans_ilv_decode(data, len(data), i.ctypes.data, i.size // ILV_SLICES, C.byref(t), out.ctypes.data),
+           "ilv_decode")
+    return out.reshape(ILV_SLICES, -1)
 
 
 def pmf_to_quantized_cdf(pmf, precision: int = 16):

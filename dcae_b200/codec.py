@@ -87,41 +87,64 @@ class DCAECodec:
         self._graphs = getattr(self, "_graphs", []) + [graph]        # the graph owns the memory `out` lives in
         return graph.replay, out
 
+    CODERS = ("reference", "interleaved")
+
+    @classmethod
+    def _check_coder(cls, coder):
+        if coder not in cls.CODERS:
+            raise ValueError(f"coder must be one of {cls.CODERS} (got {coder!r})")
+
     @torch.no_grad()
-    def compress(self, x: torch.Tensor) -> dict:
-        """dcae.py:698-761 -> {"strings": [[y_string], z_strings], "shape": z.shape[-2:]} (one y stream for the batch in the
-        reference's coder order, one z stream per image)."""
+    def compress(self, x: torch.Tensor, coder: str = "reference", lanes: int = 32) -> dict:
+        """dcae.py:698-761 -> {"strings": [y_strings, z_strings], "shape": z.shape[-2:]}, one z stream per image.
+        coder="reference" (default): y_strings = [one y stream for the batch in the reference's coder order], coded on
+        the host.  coder="interleaved": y_strings = one ilv1 string per image (include/dcae_rans.h), coded on the GPU
+        on `lanes` interleaved states; it decodes only with decompress(..., coder="interleaved")."""
+        self._check_coder(coder)
         y, z = self._latents(x)
         z_strings = self.entropy_bottleneck.compress(z)
         z_hat = self.entropy_bottleneck.decompress(z_strings, z.shape[-2:])
         latent_scales, latent_means = self.stacks["h_z_s1"](z_hat), self.stacks["h_z_s2"](z_hat)
+        if coder == "interleaved":
+            enc = self.loop.compress_to_strings_interleaved(y, latent_scales, latent_means, self.gaussian_conditional, lanes=lanes)
+            return {"strings": [enc["y_strings"], z_strings], "shape": tuple(z.shape[-2:])}
         enc = self.loop.compress_to_string(y, latent_scales, latent_means, self.gaussian_conditional)
         return {"strings": [[enc["y_string"]], z_strings], "shape": tuple(z.shape[-2:])}
 
     @torch.no_grad()
-    def decompress(self, strings, shape) -> dict:
-        """dcae.py:859-910 -> {"x_hat"} (clamped to [0, 1])."""
+    def decompress(self, strings, shape, coder: str = "reference") -> dict:
+        """dcae.py:859-910 -> {"x_hat"} (clamped to [0, 1]).  `coder` names the format `compress` wrote."""
+        self._check_coder(coder)
         z_hat = self.entropy_bottleneck.decompress(strings[1], shape)
         latent_scales, latent_means = self.stacks["h_z_s1"](z_hat), self.stacks["h_z_s2"](z_hat)
-        dec = self.loop.decompress_from_string(strings[0][0], latent_scales, latent_means, self.gaussian_conditional)
+        if coder == "interleaved":
+            dec = self.loop.decompress_from_strings_interleaved(strings[0], latent_scales, latent_means, self.gaussian_conditional)
+        else:
+            dec = self.loop.decompress_from_string(strings[0][0], latent_scales, latent_means, self.gaussian_conditional)
         return {"x_hat": self.stacks["g_s"](dec["y_hat"]).clamp_(0, 1)}
 
     # ---- image <-> container (compress_and_decompress.py:150-215: pad to multiples of 128, compress, save_bin / read_bin,
     # decompress, crop, clamp); one image per container like the reference
-    def encode_image(self, x: torch.Tensor) -> bytes:
-        """x [1, 3, H, W] in [0, 1] (any H, W >= 1 whose padded size is >= 256) -> the reference's .bin container bytes."""
+    def encode_image(self, x: torch.Tensor, coder: str = "reference") -> bytes:
+        """x [1, 3, H, W] in [0, 1] (any H, W >= 1 whose padded size is >= 256) -> container bytes: the reference's .bin
+        (coder="reference") or the DCI1 container of the ilv1 format (coder="interleaved", `container.pack_ilv`)."""
         from . import container
+        self._check_coder(coder)
         if x.dim() != 4 or x.size(0) != 1:
             raise ValueError("the container holds one image: expected [1, 3, H, W]")
         xp, _ = container.pad(x.to(self.device, torch.float32))
-        enc = self.compress(xp)
-        return container.pack_bin(enc["strings"], x.shape[-2:])
+        enc = self.compress(xp, coder=coder)
+        pack = container.pack_ilv if coder == "interleaved" else container.pack_bin
+        return pack(enc["strings"], x.shape[-2:])
 
-    def decode_image(self, blob: bytes) -> torch.Tensor:
-        """-> x_hat [1, 3, H, W] in [0, 1], cropped back to the size stored in the container."""
+    def decode_image(self, blob: bytes, coder: str = "reference") -> torch.Tensor:
+        """-> x_hat [1, 3, H, W] in [0, 1], cropped back to the size stored in the container.  `coder` names the
+        container's format; it is never guessed from the bytes."""
         from . import container
-        strings, z_shape, padding, _ = container.unpack_bin(blob)
-        out = self.decompress(strings, z_shape)
+        self._check_coder(coder)
+        unpack = container.unpack_ilv if coder == "interleaved" else container.unpack_bin
+        strings, z_shape, padding, _ = unpack(blob)
+        out = self.decompress(strings, z_shape, coder=coder)
         return container.crop(out["x_hat"], padding).clamp_(0, 1)
 
 

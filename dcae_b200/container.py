@@ -63,6 +63,29 @@ def unpack_bin(blob: bytes):
     return [[y], [z]], [padded[0] // 64, padded[1] // 64], padding, (h, w)
 
 
+ILV_MAGIC = b"DCI1"
+
+
+def pack_ilv(strings: Sequence[Sequence[bytes]], size: Sequence[int]) -> bytes:
+    """The container of the interleaved y format (`DCAECodec.compress(..., coder="interleaved")`), one image per file:
+
+        b"DCI1"  >H height  >H width  >I len(y_string)  y_string  >I len(z_string)  z_string
+
+    y_string is the image's ilv1 string (include/dcae_rans.h), z_string the same z stream as in `pack_bin`.  Its own
+    magic keeps it apart from the reference's `.bin`, which the reference's `read_bin` cannot decode."""
+    return ILV_MAGIC + pack_bin(strings, size)
+
+
+def unpack_ilv(blob: bytes):
+    """-> (strings [[y], [z]], z_shape, padding, (H, W)), like `unpack_bin`."""
+    if blob[:4] != ILV_MAGIC:
+        raise ValueError("not a DCI1 container")
+    strings, z_shape, padding, size = unpack_bin(blob[4:])
+    if 16 + len(strings[0][0]) + len(strings[1][0]) != len(blob):
+        raise ValueError("DCI1 container: trailing bytes")
+    return strings, z_shape, padding, size
+
+
 def save_bin(strings, size, path: str) -> None:
     with open(path, "wb") as f:
         f.write(pack_bin(strings, size))
@@ -74,4 +97,4 @@ def read_bin(path: str):
     return strings, z_shape, padding
 
 
-__all__ = ["calculate_padding", "pad", "crop", "pack_bin", "unpack_bin", "save_bin", "read_bin"]
+__all__ = ["calculate_padding", "pad", "crop", "pack_bin", "unpack_bin", "pack_ilv", "unpack_ilv", "save_bin", "read_bin"]

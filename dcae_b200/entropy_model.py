@@ -341,6 +341,106 @@ class EntropySliceLoop:
             self._tables_key = key
         return self._tables
 
+    # ---- the opt-in interleaved y format ilv1 coded on the GPU (include/dcae_rans.h, csrc/rans_gpu.cu) ------------
+    def _device_tables(self, gc):
+        """Device copies of the coder tables, uploaded once per table version (same key as `_coder_tables`)."""
+        key = (id(gc), gc._quantized_cdf.data_ptr(), gc._quantized_cdf._version)
+        if getattr(self, "_dev_tables_key", None) != key:
+            q, ln, off = (t.to(self.device) for t in self._coder_tables(gc))
+            self._dev_tables = (q, ln, off, _lib.CoderTables(q.data_ptr(), q.shape[1], ln.data_ptr(), off.data_ptr(), q.shape[0]))
+            self._dev_tables_key = key
+        return self._dev_tables[3]
+
+    def compress_to_strings_interleaved(self, y, latent_scales, latent_means, gc, lanes: int = 32) -> dict:
+        """Like `compress_to_string`, in the ilv1 format and with the coder on the GPU: one y string per image, its five
+        slices coded on `lanes` interleaved rANS states (1, 2, 4, 8, 16 or 32) by `dcae_ilv_encode`, straight from the
+        device symbols / indexes of `compress`.  One small copy of the segment sizes, then one copy of the strings.
+        -> dict(y_strings: list of B bytes, y_hat: device tensor)."""
+        out = self.compress(y, latent_scales, latent_means)
+        return {"y_strings": self.encode_symbols_interleaved(out["symbols"], out["indexes"], gc, lanes), "y_hat": out["y_hat"]}
+
+    def encode_symbols_interleaved(self, sym, idx, gc, lanes: int = 32) -> list:
+        """The coder alone: device int32 symbols / indexes [5, B, 64, h, w] (coder order) -> B ilv1 strings."""
+        if sym.dim() != 5 or sym.shape[0] != NUM_SLICES or sym.shape[2] != SLICE_CH or idx.shape != sym.shape:
+            raise ValueError("symbols / indexes: expected int32 [5, B, 64, h, w]")
+        sym, idx = sym.to(self.device, torch.int32).contiguous(), idx.to(self.device, torch.int32).contiguous()
+        _, B, _, h, w = sym.shape
+        lib, s = self.lib, self._stream()
+        tables = self._device_tables(gc)
+        cap = int(lib.dcae_ilv_encode_max_bytes(B, h, w, lanes))
+        if cap < 0:
+            raise ValueError(f"lanes must be 1, 2, 4, 8, 16 or 32 (got {lanes})")
+        scratch = torch.empty(int(lib.dcae_ilv_encode_scratch_bytes(B, h, w, lanes)) + 8, dtype=torch.uint8, device=self.device)
+        buf = torch.empty(max(cap, 4), dtype=torch.uint8, device=self.device)
+        sizes = torch.empty(B, NUM_SLICES, dtype=torch.int32, device=self.device)
+        status = torch.empty(B, dtype=torch.int32, device=self.device)
+        a = _lib.IlvEncArgs(sym.data_ptr(), idx.data_ptr(), B, h, w, lanes, tables, (scratch.data_ptr() + 7) // 8 * 8,
+                            scratch.numel() - 8, sizes.data_ptr(), buf.data_ptr(), buf.numel(), status.data_ptr())
+        with torch.cuda.device(self.device):
+            _lib.check(lib.dcae_ilv_encode(C.byref(a), s), "dcae_ilv_encode")
+        host_sizes, host_status = sizes.cpu(), status.cpu()
+        self._raise_on_status(host_status, "encode")
+        lengths = (24 + host_sizes.to(torch.int64).sum(1)).tolist()
+        data = buf[: sum(lengths)].cpu().numpy().tobytes()
+        strings, pos = [], 0
+        for n in lengths:
+            strings.append(data[pos: pos + n])
+            pos += n
+        return strings
+
+    def decompress_from_strings_interleaved(self, y_strings, latent_scales, latent_means, gc) -> dict:
+        """Inverse of `compress_to_strings_interleaved`: the B strings go to the device in one copy, then every slice is
+        decoded by `dcae_ilv_decode` on the stream, between `dcae_slice_loop_indexes` and `dcae_slice_loop_decode`,
+        with no host sync until the per-image status words are read once at the end.  A malformed or corrupt string
+        raises DcaeError.  -> dict(y_hat, indexes)."""
+        B, _, h, w = latent_scales.shape
+        decode_slice, finish = self._ilv_decoder(y_strings, B, h, w, gc)
+        out = self.decompress(latent_scales, latent_means, decode_slice)
+        finish()
+        return out
+
+    def decode_symbols_interleaved(self, y_strings, idx, gc) -> torch.Tensor:
+        """The coder alone: B ilv1 strings + device int32 indexes [5, B, 64, h, w] -> symbols [5, B, 64, h, w]."""
+        _, B, _, h, w = idx.shape
+        decode_slice, finish = self._ilv_decoder(y_strings, B, h, w, gc)
+        out = torch.stack([decode_slice(i, idx[i].to(self.device, torch.int32).contiguous()).clone() for i in range(NUM_SLICES)])
+        finish()
+        return out
+
+    def _ilv_decoder(self, y_strings, B, h, w, gc):
+        """(decode_slice(i, indexes [B, 64, h, w]) -> symbols, finish()) over the B strings, uploaded in one copy."""
+        if len(y_strings) != B:
+            raise ValueError(f"{len(y_strings)} y strings for a batch of {B}")
+        bounds, chunks, pos = [], [], 0
+        for st in y_strings:
+            st = bytes(st)
+            bounds += [pos, pos + len(st)]
+            pad = -len(st) % 4                                     # every string starts 4-byte aligned
+            chunks.append(st + b"\0" * pad)
+            pos += len(st) + pad
+        blob = torch.frombuffer(bytearray(b"".join(chunks) or b"\0\0\0\0"), dtype=torch.uint8)
+        dev_blob = blob.to(self.device)
+        dev_bounds = torch.tensor(bounds or [0], dtype=torch.int64).to(self.device)
+        status = torch.zeros(B, dtype=torch.int32, device=self.device)
+        sym = torch.empty(B, SLICE_CH, h, w, dtype=torch.int32, device=self.device)
+        tables = self._device_tables(gc)
+
+        def decode_slice(i, idx):
+            a = _lib.IlvDecArgs(dev_blob.data_ptr(), dev_bounds.data_ptr(), idx.data_ptr(), i, B, h, w, tables,
+                                sym.data_ptr(), status.data_ptr())
+            with torch.cuda.device(self.device):
+                _lib.check(self.lib.dcae_ilv_decode(C.byref(a), self._stream()), "dcae_ilv_decode")
+            return sym
+
+        return decode_slice, lambda: self._raise_on_status(status.cpu(), "decode")
+
+    @staticmethod
+    def _raise_on_status(status, what):
+        bad = [(b, int(v)) for b, v in enumerate(status.tolist()) if v]
+        if bad:
+            b, v = bad[0]
+            raise _lib.DcaeError(f"ilv1 {what}: image {b}: {_lib.ILV_STATUS.get(v, v)} ({len(bad)} of {len(status)} images failed)")
+
     # ---- DCAE.decompress slice loop -------------------------------------------------------------
     def decompress(self, latent_scales, latent_means,
                    decode_slice: Callable[[int, torch.Tensor], torch.Tensor]):

@@ -339,6 +339,52 @@ int dcae_pack_symbols(const int32_t* symbols, const int32_t* indexes, int64_t n,
                       unsigned long long* overflow_count, void* stream);
 
 /* --------------------------------------------------------------------------------------------
+ * The y range coder on the GPU, in the opt-in interleaved format ilv1 (include/dcae_rans.h describes it; the default
+ * reference format stays with the host coder).  One string per image; the bytes equal dcae_rans_ilv_encode's.
+ * The coder tables are device copies of GaussianConditional's quantized_cdf [n_cdfs, cdf_stride], cdf_length and
+ * offset (int32), uploaded once per table version.
+ * ------------------------------------------------------------------------------------------*/
+typedef struct {
+  const int32_t* cdfs; int32_t cdf_stride;
+  const int32_t* cdf_sizes;
+  const int32_t* offsets;
+  int32_t n_cdfs;
+} dcae_coder_tables;
+/* per-image status words written by the coder kernels: 0 = ok */
+enum { DCAE_ILV_OK = 0, DCAE_ILV_E_HEADER = 1, DCAE_ILV_E_CORRUPT = 2, DCAE_ILV_E_INDEX = 3, DCAE_ILV_E_TABLE = 4 };
+/* Encode: one warp per (image, slice), two phases (count the words, then code and store them at their final place), no
+ * atomics.  symbols / indexes: int32 [5, B, 64, h, w], the coder order of dcae_slice_loop_store.  Outputs:
+ * sizes [B, 5] (u32 bytes of each segment; image b's string is 24 + the sum of its five), the B strings back to back
+ * from out[0], and status [B] (DCAE_ILV_E_INDEX / _TABLE for an index or table row the coder cannot use).
+ * out: 4-byte aligned, out_capacity >= dcae_ilv_encode_max_bytes; scratch: 8-byte aligned, >= _scratch_bytes. */
+typedef struct {
+  const int32_t* symbols; const int32_t* indexes;
+  int32_t B, h, w, lanes;                 /* lanes: 1, 2, 4, 8, 16 or 32 */
+  dcae_coder_tables tables;
+  void* scratch; size_t scratch_bytes;
+  uint32_t* sizes;
+  uint8_t* out; int64_t out_capacity;
+  int32_t* status;
+} dcae_ilv_enc_args;
+size_t dcae_ilv_encode_scratch_bytes(int32_t B, int32_t h, int32_t w, int32_t lanes);
+int64_t dcae_ilv_encode_max_bytes(int32_t B, int32_t h, int32_t w, int32_t lanes);
+int dcae_ilv_encode(const dcae_ilv_enc_args* a, void* stream);
+/* Decode slice `slice` of B images: one warp per image.  Image b's string is strings[bounds[2b] .. bounds[2b + 1])
+ * (start 4-byte aligned); indexes: int32 [B, 64, h, w] (dcae_slice_loop_indexes), symbols: int32 [B, 64, h, w] out
+ * (dcae_slice_loop_decode's input).  Every read is checked against the string and its segment.  A malformed or corrupt
+ * string sets status[b] (DCAE_ILV_E_HEADER / _CORRUPT / _INDEX / _TABLE), writes 0 for the image's symbols and skips the
+ * image in later slices; status must be zero before slice 0 and is read by the host once, after the last slice. */
+typedef struct {
+  const uint8_t* strings; const int64_t* bounds;
+  const int32_t* indexes;
+  int32_t slice, B, h, w;
+  dcae_coder_tables tables;
+  int32_t* symbols;
+  int32_t* status;
+} dcae_ilv_dec_args;
+int dcae_ilv_decode(const dcae_ilv_dec_args* a, void* stream);
+
+/* --------------------------------------------------------------------------------------------
  * The channel-slice loop (dcae.py:638-670 forward, :713-753 compress, :878-906 decompress).
  * Packed weights of one slice i.  Dense weights are dcae_weight (row-major [N, K]); packing rules
  * (done by dcae_b200/weights.py from a reference state dict):

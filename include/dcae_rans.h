@@ -66,6 +66,27 @@ int dcae_rans_decoder_set_stream(dcae_rans_decoder* d, const uint8_t* bytes, int
 int dcae_rans_decoder_decode_stream(dcae_rans_decoder* d, const void* indexes, int32_t indexes_type, int64_t n,
                                     const dcae_rans_tables* t, int32_t* out);
 
+/* ---- ilv1: the interleaved y-stream format, one string per image (opt-in; the reference format above is the default) --
+ * The same steps as the coder above (same tables, sentinel and 4-bit bypass, same per-step arithmetic); only the
+ * assignment of symbols to states and the order of the words differ, so that up to 32 lanes decode in parallel.
+ *   string  = u8 version (1), u8 L (lanes: 1, 2, 4, 8, 16 or 32), u16 0, u32 bytes of segment s (s = 0..4), segments
+ *   segment = L final states (u64, lane order), then one shared stream of u32 words      (all fields little-endian)
+ * Symbol j of a slice (the [64, h, w] slice of one image flattened) is coded by lane j % L at step j / L.  The words
+ * are in the order the decoder consumes them: step ascending, then sub-operation ascending (0 = the symbol, then the
+ * bypass count and digit steps), then lane ascending; only lanes whose step renormalises take a word.  With L = 1 a
+ * segment is byte-identical to what dcae_rans_encoder_flush writes for the slice.  Cost: 4 + 5 (4 + 8 L) bytes per
+ * image (the reference format: 8).  csrc/rans_gpu.cu (libdcae_b200.so) codes the same bytes on the GPU.
+ *
+ * symbols / indexes / out: int32 [5, n] (slice-major, n symbols per slice).  _encode writes the string into out and
+ * returns its length (<= dcae_rans_ilv_max_bytes(n, lanes)), or a negative code if it does not fit `capacity`.
+ * _decode: DCAE_RANS_E_STREAM for a malformed, truncated or corrupt string (a segment must also end with every word
+ * consumed and every lane back in its initial state), DCAE_RANS_E_INVALID for bad arguments or indexes. */
+int64_t dcae_rans_ilv_max_bytes(int64_t n, int32_t lanes);
+int64_t dcae_rans_ilv_encode(const int32_t* symbols, const int32_t* indexes, int64_t n, int32_t lanes,
+                             const dcae_rans_tables* t, uint8_t* out, int64_t capacity);
+int dcae_rans_ilv_decode(const uint8_t* bytes, int64_t n_bytes, const int32_t* indexes, int64_t n,
+                         const dcae_rans_tables* t, int32_t* out);
+
 /* ---- compressai._CXX.pmf_to_quantized_cdf (used by GaussianConditional.update(), dcae.py:616-621) --------- */
 /* pmf [n] (non-negative, finite) -> cdf [n + 1] with cdf[0] = 0, cdf[n] = 2^precision, strictly increasing. */
 int dcae_pmf_to_quantized_cdf(const float* pmf, int32_t n, int32_t precision, int32_t* cdf);
