@@ -66,10 +66,7 @@ dict_attention_tcgen05_kernel(const __grid_constant__ CUtensorMap map_q, const _
     mbar_init(smem_u32(&o_full), 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_slot)), "r"(512) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (warp == 1) tmem_alloc<1>(smem_u32(&tmem_base_slot), 512);
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
@@ -283,9 +280,7 @@ dict_attention_tcgen05_kernel(const __grid_constant__ CUtensorMap map_q, const _
 
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
-  if (warp == 1) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(512) : "memory");
-  }
+  if (warp == 1) tmem_dealloc<1>(tmem, 512);
 }
 
 }  // namespace
@@ -308,21 +303,21 @@ int dict_attention_tcgen05(const float* q, int64_t q_ld, const dcae_dict_kv* kv,
     cuuint64_t dims[2] = {(cuuint64_t)q_ld, (cuuint64_t)T};
     cuuint64_t str[1] = {(cuuint64_t)q_ld * 4};
     cuuint32_t box[2] = {AT_HD, AT_M};
-    DCAE_TRY(encode_map(&mq, q, 2, dims, str, box));
+    DCAE_TRY(encode_map(&mq, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, q, 2, dims, str, box));
   }
   {
     cuuint64_t dims[2] = {AT_HD, (cuuint64_t)AT_HEADS * AT_ND};
     cuuint64_t str[1] = {AT_HD * 4};
     cuuint32_t box[2] = {AT_HD, AT_ND};
-    DCAE_TRY(encode_map(&mkh, kv->Kh_hi, 2, dims, str, box));
-    if (passes == 3) DCAE_TRY(encode_map(&mkl, kv->Kh_lo, 2, dims, str, box)); else mkl = mkh;
+    DCAE_TRY(encode_map(&mkh, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, kv->Kh_hi, 2, dims, str, box));
+    if (passes == 3) DCAE_TRY(encode_map(&mkl, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, kv->Kh_lo, 2, dims, str, box)); else mkl = mkh;
   }
   {
     cuuint64_t dims[2] = {AT_ND, (cuuint64_t)AT_HEADS * AT_HD};
     cuuint64_t str[1] = {AT_ND * 4};
     cuuint32_t box[2] = {32, AT_HD};
-    DCAE_TRY(encode_map(&mvh, kv->Vt_hi, 2, dims, str, box));
-    if (passes == 3) DCAE_TRY(encode_map(&mvl, kv->Vt_lo, 2, dims, str, box)); else mvl = mvh;
+    DCAE_TRY(encode_map(&mvh, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, kv->Vt_hi, 2, dims, str, box));
+    if (passes == 3) DCAE_TRY(encode_map(&mvl, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, kv->Vt_lo, 2, dims, str, box)); else mvl = mvh;
   }
   static std::once_flag once;
   static cudaError_t attr_err = cudaSuccess;

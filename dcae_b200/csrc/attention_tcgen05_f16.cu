@@ -65,24 +65,6 @@ __device__ __forceinline__ long long af_timed_wait(uint32_t bar, uint32_t parity
   return clock64() - t0;
 }
 
-__device__ __forceinline__ void mma_f16_ss(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void mma_f16_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  // A operand from TMEM: 128 lanes x 8 columns per K = 16 step (two fp16 per 32-bit column), B from shared memory
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-
 template <bool DBG>
 __global__ void __launch_bounds__(AF_THREADS, 1)
 dict_attention_f16_kernel(const __grid_constant__ CUtensorMap map_qh, const __grid_constant__ CUtensorMap map_ql,
@@ -112,10 +94,7 @@ dict_attention_f16_kernel(const __grid_constant__ CUtensorMap map_qh, const __gr
     }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_slot)), "r"(512) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (warp == 1) tmem_alloc<1>(smem_u32(&tmem_base_slot), 512);
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
@@ -163,9 +142,8 @@ dict_attention_f16_kernel(const __grid_constant__ CUtensorMap map_qh, const __gr
   } else if (warp == 1) {
     {
       // ===================== MMA issuer (warp-uniform, one elected lane issues) =====================
-      // D = F32 (bit 4), A = B = F16 (format 0), K-major, N >> 3 at bit 17, M >> 4 at bit 24
-      const uint32_t idesc_s = (1u << 4) | ((uint32_t)(AF_ND >> 3) << 17) | ((uint32_t)(AF_M >> 4) << 24);
-      const uint32_t idesc_o = (1u << 4) | ((uint32_t)(AF_HD >> 3) << 17) | ((uint32_t)(AF_M >> 4) << 24);
+      const uint32_t idesc_s = make_idesc_f16(AF_M, AF_ND);     // S: N = 128
+      const uint32_t idesc_o = make_idesc_f16(AF_M, AF_HD);     // O: N = 32
       long long w_full = 0, w_p = 0, w_of = 0;
       const long long t_mma0 = clock64();
       auto issue_s = [&](int g) {                                 // S(g) -> buffer g & 1
@@ -180,9 +158,9 @@ dict_attention_f16_kernel(const __grid_constant__ CUtensorMap map_qh, const __gr
             const uint32_t ko = (uint32_t)((g & 1) * 2 + k) * 32;    // this head's 32 dims inside the pair's 128-byte rows
             const uint64_t q_hi = make_smem_desc(sb + ko), q_lo = make_smem_desc(sb + OFF_QL + ko);
             const uint64_t k_hi = make_smem_desc(sb + OFF_KH + ko), k_lo = make_smem_desc(sb + OFF_KL + ko);
-            mma_f16_ss(d, q_lo, k_hi, idesc_s, k != 0);
-            mma_f16_ss(d, q_hi, k_lo, idesc_s, 1);
-            mma_f16_ss(d, q_hi, k_hi, idesc_s, 1);
+            mma_f16(d, q_lo, k_hi, idesc_s, k != 0);
+            mma_f16(d, q_hi, k_lo, idesc_s, 1);
+            mma_f16(d, q_hi, k_hi, idesc_s, 1);
           }
           mma_commit(smem_u32(&s_full[g & 1]));
         }
@@ -326,30 +304,7 @@ dict_attention_f16_kernel(const __grid_constant__ CUtensorMap map_qh, const __gr
 
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
-  if (warp == 1) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(512) : "memory");
-  }
-}
-
-int encode_f16_2d(CUtensorMap* m, const void* base, uint64_t inner, uint64_t rows, uint64_t row_bytes, uint32_t box_inner,
-                  uint32_t box_rows) {
-  EncodeTiledFn enc = get_encode();
-  if (!enc) {
-    set_error("cuTensorMapEncodeTiled is not available from the driver");
-    return DCAE_E_CUDA;
-  }
-  cuuint64_t dims[2] = {inner, rows};
-  cuuint64_t str[1] = {row_bytes};
-  cuuint32_t box[2] = {box_inner, box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void*>(base), dims, str, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled(attention f16) failed with CUresult %d (dims %llu x %llu)", (int)r, (unsigned long long)inner,
-              (unsigned long long)rows);
-    return DCAE_E_CUDA;
-  }
-  return DCAE_OK;
+  if (warp == 1) tmem_dealloc<1>(tmem, 512);
 }
 
 }  // namespace
@@ -369,13 +324,29 @@ int dict_attention_tcgen05_f16(const dcae_planes* q16, const dcae_dict_kv* kv, i
   p.tiles = (int)((T + AF_M - 1) / AF_M);
   p.k_descale = kv->k_descale; p.v_descale = kv->v_descale;
   CUtensorMap mqh, mql, mkh, mkl, mvh, mvl;
-  const uint64_t D = (uint64_t)AF_HEADS * AF_HD;
-  DCAE_TRY(encode_f16_2d(&mqh, q16->hi, D, (uint64_t)T, (uint64_t)q16->ld * 2, 64, AF_M));
-  DCAE_TRY(encode_f16_2d(&mql, q16->lo, D, (uint64_t)T, (uint64_t)q16->ld * 2, 64, AF_M));
-  DCAE_TRY(encode_f16_2d(&mkh, kv->K16_hi, D, AF_ND, D * 2, 64, AF_ND));
-  DCAE_TRY(encode_f16_2d(&mkl, kv->K16_lo, D, AF_ND, D * 2, 64, AF_ND));
-  DCAE_TRY(encode_f16_2d(&mvh, kv->Vt16_hi, AF_ND, D, AF_ND * 2, 64, 64));
-  DCAE_TRY(encode_f16_2d(&mvl, kv->Vt16_lo, AF_ND, D, AF_ND * 2, 64, 64));
+  const cuuint64_t D = (cuuint64_t)AF_HEADS * AF_HD;
+  constexpr CUtensorMapDataType F16 = CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
+  {
+    cuuint64_t dims[2] = {D, (cuuint64_t)T};
+    cuuint64_t str[1] = {(cuuint64_t)q16->ld * 2};
+    cuuint32_t box[2] = {64, AF_M};
+    DCAE_TRY(encode_map(&mqh, F16, q16->hi, 2, dims, str, box));
+    DCAE_TRY(encode_map(&mql, F16, q16->lo, 2, dims, str, box));
+  }
+  {
+    cuuint64_t dims[2] = {D, AF_ND};
+    cuuint64_t str[1] = {D * 2};
+    cuuint32_t box[2] = {64, AF_ND};
+    DCAE_TRY(encode_map(&mkh, F16, kv->K16_hi, 2, dims, str, box));
+    DCAE_TRY(encode_map(&mkl, F16, kv->K16_lo, 2, dims, str, box));
+  }
+  {
+    cuuint64_t dims[2] = {AF_ND, D};
+    cuuint64_t str[1] = {AF_ND * 2};
+    cuuint32_t box[2] = {64, 64};
+    DCAE_TRY(encode_map(&mvh, F16, kv->Vt16_hi, 2, dims, str, box));
+    DCAE_TRY(encode_map(&mvl, F16, kv->Vt16_lo, 2, dims, str, box));
+  }
   const size_t smem = (size_t)AF_STAGES * AF_STAGE + 1024;
   static std::once_flag once;
   static cudaError_t attr_err = cudaSuccess;

@@ -146,7 +146,6 @@ bool profiling_on();
 int gemm_simt(const dcae_operand* a, const dcae_weight* w, const dcae_epilogue* e, cudaStream_t s);
 int gemm_tcgen05(const dcae_operand* a, const dcae_weight* w, const dcae_epilogue* e, int passes, cudaStream_t s);
 int gemm_tcgen05_f16x3(const dcae_operand* a, const dcae_weight* w, const dcae_epilogue* e, int passes, cudaStream_t s);
-int gemm_tcgen05_2cta(const dcae_operand* a, const dcae_weight* w, const dcae_epilogue* e, int passes, int bn, cudaStream_t s);
 int dict_attention_tcgen05(const float* q, int64_t q_ld, const dcae_dict_kv* kv, int64_t T, float* out, int64_t out_ld,
                            dcae_planes out16, int passes, cudaStream_t s);
 int dict_attention_tcgen05_f16(const dcae_planes* q16, const dcae_dict_kv* kv, int64_t T, float* out, int64_t out_ld,

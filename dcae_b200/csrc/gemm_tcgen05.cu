@@ -15,6 +15,13 @@
 // * warp 0 = TMA producer, warp 1 = TMEM owner + MMA issuer, warps 2..5 = split warps, then the
 //   epilogue (tcgen05.ld 32x32b -> bias / addend / GELU / 0.5 tanh / scaled residual -> st.global).
 //
+// Thread-block-pair variant (tcgen05 cta_group::2, 3-pass only).  With one CTA per tile the 3-pass mainloop
+// needs ~58 B/clk/SM from L2 (A + B_hi + B_lo per k-block) and only 2-3 stages fit in shared memory; the sweep
+// in profiles/r01/gemm_knobs_v2.jsonl shows it starving.  Two CTAs (one SM pair) compute a 256-token x BN tile
+// with M = 256 MMAs issued by the leader CTA: each CTA loads its own 128-token A tile and only HALF of the
+// weight tile (BN/2 rows), so the weight traffic and its shared-memory footprint are halved (BN = 256: 64 KB
+// per stage -> 3 stages, 31 B/clk/SM) while the MMA instruction does twice the work per issue.
+//
 // Every mbarrier wait is bounded: a protocol bug traps instead of hanging the GPU.
 #include <cuda.h>
 
@@ -34,7 +41,6 @@ constexpr int MAX_STAGES = 8;
 constexpr int A_BYTES = BM * BK * 4;   // 16 KB
 constexpr int NTHREADS = 512;     // 16 warps, see the role table at the kernel
 constexpr int NDRAIN = 256;       // drain/epilogue threads (warps 8..15)
-constexpr int MAX_GROUPS = 8;     // 16-column groups per drain thread: BN/2 <= 128
 constexpr int REGS_CTRL = 40, REGS_SPLIT = 64, REGS_DRAIN = 200;   // 128*40 + 128*64 + 256*200 <= 65536
 constexpr int CHUNK_MMAS = 96;    // longest TMEM accumulation chain (RZ bias ~1.75e-8 per MMA)
 constexpr uint32_t SMEM_LIMIT = 227 * 1024;
@@ -45,13 +51,14 @@ struct TcParams {
   int cblk_per_tap;          // (k0 + k1) / 32
   int col0, k0, col1;
   int taps;
-  int B, h, w, TH, TW, tw_shift, tiles_x, tiles_y;
+  int B, h, w;
+  TokenTiling tt;
   int BN, stages, tmem_cols;
-  int n_tiles_n, total_tiles, chunk_kb;
-  uint32_t stage_bytes, b_bytes;
+  int n_tiles_n, total_tiles, chunk_kb;   // total_tiles: of CTAs, or of pairs (256 tokens x BN each)
+  uint32_t stage_bytes, b_bytes;          // b_bytes: this CTA's weight rows (a pair's CTA holds BN/2) x 128 B
 };
 
-// Persistent kernel: grid = min(#tiles, #SMs); each CTA walks tiles t = blockIdx.x + i * gridDim.x in
+// Persistent kernel: grid = min(#tiles, #SMs) CTAs (or pairs); each walks its tiles in
 // (token-tile major, n-tile minor) order so that CTAs running together share A tiles through L2.
 //
 // Accuracy: the tensor core's fp32 accumulator rounds toward zero, which biases a long accumulation
@@ -64,27 +71,39 @@ struct TcParams {
 // Warps: 0 = TMA producer, 1 = TMEM owner + MMA issuer, 2-3 idle, 4-7 = split warps (3-pass mode),
 // 8-15 = drain/epilogue (two warps per TMEM lane quarter, half of the BN columns each).
 // Registers are re-balanced with setmaxnreg: the drain warps hold BN/2 running sums per thread.
-template <int PASSES>
-__global__ void __launch_bounds__(NTHREADS, 1)
-gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_bh,
-                    const __grid_constant__ CUtensorMap map_bl, const TcParams p) {
+//
+// PAIR: the MMA warp of the leader CTA issues for both CTAs.  Barriers (S stages): full[S] local (the CTA's own
+// A tile landed; single CTA: its weights too), b_full[S] in the leader (weights of both CTAs), ready[S] in the
+// leader (256 split threads of both CTAs), empty[S] and tmem_full[2] in both CTAs (multicast tcgen05.commit),
+// tmem_empty[2] in the leader (512 drain threads).
+template <bool PAIR, int PASSES>
+__device__ __forceinline__ void gemm_tf32_body(const CUtensorMap& map_a, const CUtensorMap& map_bh, const CUtensorMap& map_bl,
+                                               const TcParams& p) {
+  static_assert(!PAIR || PASSES == 3, "the pair kernel runs the 3-pass mode only");
   extern __shared__ uint8_t smem_raw[];
-  __shared__ __align__(8) uint64_t full_bar[MAX_STAGES], ready_bar[MAX_STAGES], empty_bar[MAX_STAGES];
+  __shared__ __align__(8) uint64_t full_bar[MAX_STAGES], b_full[PAIR ? MAX_STAGES : 1], ready_bar[MAX_STAGES], empty_bar[MAX_STAGES];
   __shared__ __align__(8) uint64_t tmem_full_bar[2], tmem_empty_bar[2];
   __shared__ uint32_t tmem_base_slot;
 
-  const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0), lane = threadIdx.x & 31;   // warp: provably uniform
+  const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0), lane = threadIdx.x & 31;   // warp, rank: provably uniform
+  const uint32_t rank = PAIR ? __shfl_sync(0xffffffffu, cluster_ctarank(), 0) : 0u;
+  const bool leader = rank == 0;
+  // a persistent worker (a CTA, or a pair) walks tiles first_tile(), + tile_stride(), ...  Both are re-read at every
+  // use: held in registers across the kernel, they cost the single-CTA kernel 100 bytes of spill stores.
+  auto first_tile = [] { return PAIR ? (int)(blockIdx.x >> 1) : (int)blockIdx.x; };
+  auto tile_stride = [] { return PAIR ? (int)(gridDim.x >> 1) : (int)gridDim.x; };
   const uint32_t smem0 = (smem_u32(smem_raw) + 1023u) & ~1023u;   // SWIZZLE_128B atoms need 1024-B alignment
 
   if (threadIdx.x == 0) {
     for (int s = 0; s < p.stages; ++s) {
       mbar_init(smem_u32(&full_bar[s]), 1);
-      mbar_init(smem_u32(&ready_bar[s]), 128);
+      if (PAIR) mbar_init(smem_u32(&b_full[s]), 1);
+      mbar_init(smem_u32(&ready_bar[s]), PAIR ? 256 : 128);
       mbar_init(smem_u32(&empty_bar[s]), 1);
     }
     for (int b = 0; b < 2; ++b) {
       mbar_init(smem_u32(&tmem_full_bar[b]), 1);
-      mbar_init(smem_u32(&tmem_empty_bar[b]), NDRAIN);
+      mbar_init(smem_u32(&tmem_empty_bar[b]), PAIR ? 2 * NDRAIN : NDRAIN);
     }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
@@ -93,12 +112,10 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
     asm volatile("prefetch.tensormap [%0];" ::"l"(&map_bh) : "memory");
     if (PASSES == 3) asm volatile("prefetch.tensormap [%0];" ::"l"(&map_bl) : "memory");
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_slot)), "r"(p.tmem_cols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (warp == 1) tmem_alloc<PAIR ? 2 : 1>(smem_u32(&tmem_base_slot), p.tmem_cols);
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
+  if (PAIR) cluster_sync_all();     // the peer's barriers exist before anything signals them
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
   const uint32_t tmem_base = tmem_base_slot;
 
@@ -108,13 +125,14 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
   const uint32_t off_bl = off_bh + p.b_bytes;
   const int n_chunks = (p.KB + p.chunk_kb - 1) / p.chunk_kb;
 
+  // tile -> this CTA's token tile (b, y0, x0) and the tile's first output column n0
   auto tile_coords = [&](int t, int& b, int& y0, int& x0, int& n0) {
     const int nt = t % p.n_tiles_n;
-    int mt = t / p.n_tiles_n;
-    const int tile_x = mt % p.tiles_x; mt /= p.tiles_x;
-    const int tile_y = mt % p.tiles_y;
-    b = mt / p.tiles_y;
-    x0 = tile_x * p.TW; y0 = tile_y * p.TH; n0 = nt * p.BN;
+    int mt = PAIR ? (t / p.n_tiles_n) * 2 + (int)rank : t / p.n_tiles_n;   // b may reach B for a pair's odd tail tile:
+    const int tile_x = mt % p.tt.tiles_x; mt /= p.tt.tiles_x;                 // TMA zero-fills, the epilogue skips it
+    const int tile_y = mt % p.tt.tiles_y;
+    b = mt / p.tt.tiles_y;
+    x0 = tile_x * p.tt.TW; y0 = tile_y * p.tt.TH; n0 = nt * p.BN;
   };
 
   if (warp < 4) {
@@ -123,7 +141,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
       // ===================== TMA producer (warp-uniform; one elected lane issues, see elect_one) =====================
       int stage = 0;
       uint32_t phase = 0;
-      for (int t = blockIdx.x; t < p.total_tiles; t += gridDim.x) {
+      for (int t = first_tile(); t < p.total_tiles; t += tile_stride()) {
         int b, y0, x0, n0;
         tile_coords(t, b, y0, x0, n0);
         for (int kb = 0; kb < p.KB; ++kb) {
@@ -136,32 +154,51 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
           int dy = 0, dx = 0;
           if (p.taps == 9) { dy = tap / 3 - 1; dx = tap % 3 - 1; }
           if (elect_one()) {
-            mbar_expect_tx(fb, A_BYTES + (PASSES == 3 ? 2 : 1) * p.b_bytes);
-            tma_load_4d(sbase, &map_a, fb, col, x0 + dx, y0 + dy, b);
-            tma_load_2d(sbase + off_bh, &map_bh, fb, kb * BK, n0);
-            if (PASSES == 3) tma_load_2d(sbase + off_bl, &map_bl, fb, kb * BK, n0);
+            if (PAIR) {
+              const uint32_t bf = smem_u32(&b_full[stage]);
+              const int nrow = n0 + (int)rank * (p.BN >> 1);
+              mbar_expect_tx(fb, A_BYTES);
+              tma_load_4d(sbase, &map_a, fb, col, x0 + dx, y0 + dy, b);
+              if (leader) mbar_expect_tx(bf, 4 * p.b_bytes);            // hi + lo halves of both CTAs
+              tma_load_2d_2sm(sbase + off_bh, &map_bh, bf, kb * BK, nrow);
+              tma_load_2d_2sm(sbase + off_bl, &map_bl, bf, kb * BK, nrow);
+            } else {
+              mbar_expect_tx(fb, A_BYTES + (PASSES == 3 ? 2 : 1) * p.b_bytes);
+              tma_load_4d(sbase, &map_a, fb, col, x0 + dx, y0 + dy, b);
+              tma_load_2d(sbase + off_bh, &map_bh, fb, kb * BK, n0);
+              if (PASSES == 3) tma_load_2d(sbase + off_bl, &map_bl, fb, kb * BK, n0);
+            }
           }
           __syncwarp();
           if (++stage == p.stages) { stage = 0; phase ^= 1; }
         }
       }
-    } else if (warp == 1) {
-      // ===================== MMA issuer (warp-uniform; one elected lane issues) =====================
-      const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(p.BN >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
+    } else if (warp == 1 && leader) {
+      // ===================== MMA issuer (the leader CTA of a pair; warp-uniform, one elected lane issues) =====================
+      const uint32_t idesc = make_idesc_tf32((PAIR ? 2 : 1) * BM, p.BN);
       int stage = 0;
       uint32_t phase = 0, gchunk = 0;
-      for (int t = blockIdx.x; t < p.total_tiles; t += gridDim.x) {
+      for (int t = first_tile(); t < p.total_tiles; t += tile_stride()) {
         for (int ck = 0; ck < n_chunks; ++ck, ++gchunk) {
           const uint32_t buf = gchunk & 1;
-          mbar_wait(smem_u32(&tmem_empty_bar[buf]), ((gchunk >> 1) & 1) ^ 1);   // drained by the epilogue warps
+          if (PAIR) mbar_wait_cluster(smem_u32(&tmem_empty_bar[buf]), ((gchunk >> 1) & 1) ^ 1);   // drained by the epilogue warps
+          else mbar_wait(smem_u32(&tmem_empty_bar[buf]), ((gchunk >> 1) & 1) ^ 1);
           asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
           const uint32_t tmem_acc = tmem_base + buf * (uint32_t)p.BN;
           const int kb_end = min(p.KB, (ck + 1) * p.chunk_kb);
           for (int kb = ck * p.chunk_kb; kb < kb_end; ++kb) {
-            mbar_wait(smem_u32(PASSES == 3 ? &ready_bar[stage] : &full_bar[stage]), phase);
+            if (PAIR) {
+              mbar_wait_cluster(smem_u32(&ready_bar[stage]), phase);
+              mbar_wait_cluster(smem_u32(&b_full[stage]), phase);
+            } else {
+              mbar_wait(smem_u32(PASSES == 3 ? &ready_bar[stage] : &full_bar[stage]), phase);
+            }
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
             const uint32_t sbase = smem0 + stage * p.stage_bytes;
             const uint32_t first = (kb == ck * p.chunk_kb) ? 0u : 1u;
+            auto mma = [&](uint64_t a, uint64_t b, uint32_t accumulate) {
+              if (PAIR) mma_tf32_2sm(tmem_acc, a, b, idesc, accumulate); else mma_tf32(tmem_acc, a, b, idesc, accumulate);
+            };
             if (elect_one()) {
 #pragma unroll
               for (int k = 0; k < BK / UMMA_K; ++k) {
@@ -171,19 +208,22 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
                 if (PASSES == 3) {
                   const uint64_t a_lo = make_smem_desc(sbase + off_al + koff);
                   const uint64_t b_lo = make_smem_desc(sbase + off_bl + koff);
-                  mma_tf32(tmem_acc, a_lo, b_hi, idesc, first | (uint32_t)(k != 0));
-                  mma_tf32(tmem_acc, a_hi, b_lo, idesc, 1);
-                  mma_tf32(tmem_acc, a_hi, b_hi, idesc, 1);
+                  mma(a_lo, b_hi, first | (uint32_t)(k != 0));
+                  mma(a_hi, b_lo, 1);
+                  mma(a_hi, b_hi, 1);
                 } else {
-                  mma_tf32(tmem_acc, a_hi, b_hi, idesc, first | (uint32_t)(k != 0));
+                  mma(a_hi, b_hi, first | (uint32_t)(k != 0));
                 }
               }
-              mma_commit(smem_u32(&empty_bar[stage]));       // frees the smem slot once these MMAs retire
+              // frees the smem slot (of both CTAs) once these MMAs retire
+              if (PAIR) mma_commit_2sm(smem_u32(&empty_bar[stage])); else mma_commit(smem_u32(&empty_bar[stage]));
             }
             __syncwarp();
             if (++stage == p.stages) { stage = 0; phase ^= 1; }
           }
-          if (elect_one()) mma_commit(smem_u32(&tmem_full_bar[buf]));       // this chain is complete
+          if (elect_one()) {        // this chain is complete (a pair: both CTAs drain their half)
+            if (PAIR) mma_commit_2sm(smem_u32(&tmem_full_bar[buf])); else mma_commit(smem_u32(&tmem_full_bar[buf]));
+          }
           __syncwarp();
         }
       }
@@ -191,11 +231,11 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
   } else if (warp < 8) {
     asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(REGS_SPLIT));
     if (PASSES == 3) {
-      // ===================== split warps: a -> (a_hi in place, a_lo) =====================
+      // ===================== split warps: own A tile -> (a_hi in place, a_lo) =====================
       const int st = threadIdx.x - 128;   // 0..127
       int stage = 0;
       uint32_t phase = 0;
-      for (int t = blockIdx.x; t < p.total_tiles; t += gridDim.x) {
+      for (int t = first_tile(); t < p.total_tiles; t += tile_stride()) {
         for (int kb = 0; kb < p.KB; ++kb) {
           mbar_wait(smem_u32(&full_bar[stage]), phase);
           const uint32_t sbase = smem0 + stage * p.stage_bytes;
@@ -211,21 +251,22 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
             asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(sbase + off_al + off), "f"(lo.x), "f"(lo.y), "f"(lo.z), "f"(lo.w) : "memory");
           }
           asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic-proxy writes -> visible to the MMA (async proxy)
-          mbar_arrive(smem_u32(&ready_bar[stage]));
+          if (PAIR) mbar_arrive_cluster(smem_u32(&ready_bar[stage]), 0);      // the leader's barrier counts both CTAs
+          else mbar_arrive(smem_u32(&ready_bar[stage]));
           if (++stage == p.stages) { stage = 0; phase ^= 1; }
         }
       }
     }
   } else {
     asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(REGS_DRAIN));
-    // ===================== drain + epilogue warps =====================
+    // ===================== drain + epilogue warps (own 128 rows) =====================
     const int quarter = warp & 3;                  // TMEM lane quarter this warp may touch
     const int half = (warp - 8) >> 2;              // even / odd 32-column blocks
     uint32_t gchunk = 0;
-    for (int t = blockIdx.x; t < p.total_tiles; t += gridDim.x) {
+    for (int t = first_tile(); t < p.total_tiles; t += tile_stride()) {
       EpiTile et;
       tile_coords(t, et.b, et.y0, et.x0, et.n0);
-      et.B = p.B; et.h = p.h; et.w = p.w; et.tw_shift = p.tw_shift; et.N = p.N; et.BN = p.BN;
+      et.B = p.B; et.h = p.h; et.w = p.w; et.tw_shift = p.tt.tw_shift; et.N = p.N; et.BN = p.BN;
       float acc[EPI_BLOCKS * 32];
       for (int ck = 0; ck < n_chunks; ++ck, ++gchunk) {
         const uint32_t buf = gchunk & 1;
@@ -233,7 +274,8 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
         drain_chunk(acc, tmem_base + ((uint32_t)(quarter * 32) << 16) + buf * (uint32_t)p.BN, half, p.BN, ck == 0);
         asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        mbar_arrive(smem_u32(&tmem_empty_bar[buf]));   // the MMA warp may start the next chain in this buffer
+        // the MMA warp may start the next chain in this buffer
+        if (PAIR) mbar_arrive_cluster(smem_u32(&tmem_empty_bar[buf]), 0); else mbar_arrive(smem_u32(&tmem_empty_bar[buf]));
       }
       // ---- epilogue of this tile (overlaps the next tile's mainloop) ----
       epilogue_store(acc, p.e, et, quarter, half, lane);
@@ -242,25 +284,27 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
 
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
-  if (warp == 1) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(p.tmem_cols) : "memory");
-  }
+  if (PAIR) cluster_sync_all();     // neither CTA may free TMEM / exit while the pair still uses its smem or TMEM
+  if (warp == 1) tmem_dealloc<PAIR ? 2 : 1>(tmem_base, p.tmem_cols);
+}
+
+template <int PASSES>
+__global__ void __launch_bounds__(NTHREADS, 1)
+gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_bh,
+                    const __grid_constant__ CUtensorMap map_bl, const TcParams p) {
+  gemm_tf32_body<false, PASSES>(map_a, map_bh, map_bl, p);
+}
+
+template <int PASSES>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1)
+gemm_tcgen05_2cta_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_bh,
+                         const __grid_constant__ CUtensorMap map_bl, const TcParams p) {
+  gemm_tf32_body<true, PASSES>(map_a, map_bh, map_bl, p);
 }
 
 // ---------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------
-void pick_tile(int h, int w, int* TH, int* TW) {
-  // 128 tokens per tile as a TH x TW box inside one image; minimise the number of tiles
-  int best = 1 << 30;
-  for (int tw = 128; tw >= 1; tw >>= 1) {
-    const int th = 128 / tw;
-    const int tiles = ((h + th - 1) / th) * ((w + tw - 1) / tw);
-    // prefer wide-ish boxes (tw = 16) on ties: longer contiguous rows per TMA line group
-    if (tiles < best || (tiles == best && tw == 16)) { best = tiles; *TH = th; *TW = tw; }
-  }
-}
-
 int pick_bn(int N) {
   for (int bn = 256; bn >= 32; bn -= 32)
     if (N % bn == 0) return bn;
@@ -275,12 +319,6 @@ int gemm_tcgen05(const dcae_operand* a, const dcae_weight* w, const dcae_epilogu
   DCAE_REQUIRE(e->act_cols <= 0 || e->act_cols >= w->N || e->act_cols % 32 == 0, "gemm(tcgen05): act_cols must be a multiple of 32");
   const int64_t T = (int64_t)a->B * a->h * a->w;
   if (T == 0) return DCAE_OK;
-  // thread-block-pair kernel (gemm_tcgen05_2cta.cu).  Measured (profiles/r01/gemm_ab_v3.jsonl): it wins on long-K
-  // 3-pass layers (cc1: K = 8640..10944, +8 %) and loses on short K, where the extra cross-CTA handshakes are not amortised.
-  if (passes == 3 && w->K >= 4096) {
-    const int rc = gemm_tcgen05_2cta(a, w, e, passes, pick_bn(w->N), s);
-    if (rc != 1) return rc;
-  }
   TcParams p;
   p.e = *e;
   p.N = w->N;
@@ -289,18 +327,19 @@ int gemm_tcgen05(const dcae_operand* a, const dcae_weight* w, const dcae_epilogu
   p.col0 = a->col0; p.k0 = a->k0; p.col1 = a->col1;
   p.taps = a->taps;
   p.B = a->B; p.h = a->h; p.w = a->w;
-  pick_tile(a->h, a->w, &p.TH, &p.TW);
-  p.tw_shift = 0;
-  while ((1 << p.tw_shift) < p.TW) ++p.tw_shift;
-  p.tiles_x = (a->w + p.TW - 1) / p.TW;
-  p.tiles_y = (a->h + p.TH - 1) / p.TH;
+  p.tt = token_tiling(a->h, a->w);
   p.BN = pick_bn(w->N);
   DCAE_REQUIRE(p.BN > 0, "gemm(tcgen05): N=%d must be a multiple of 32", w->N);
+  const int m_tiles = p.tt.tiles_x * p.tt.tiles_y * a->B;
+  // The thread-block pair needs two token tiles and BN/2 weight rows per CTA, a multiple of 16 (pick_bn returns a
+  // multiple of 32).  Measured (profiles/r01/gemm_ab_v3.jsonl): it wins on long-K 3-pass layers (cc1: K = 8640..10944,
+  // +8 %) and loses on short K, where the extra cross-CTA handshakes are not amortised.
+  const bool pair = passes == 3 && w->K >= 4096 && p.BN % 32 == 0 && m_tiles >= 2;
   p.tmem_cols = 2 * p.BN <= 64 ? 64 : 2 * p.BN <= 128 ? 128 : 2 * p.BN <= 256 ? 256 : 512;   // two chain buffers
   p.n_tiles_n = w->N / p.BN;
-  p.total_tiles = p.n_tiles_n * p.tiles_x * p.tiles_y * a->B;
+  p.total_tiles = p.n_tiles_n * (pair ? (m_tiles + 1) / 2 : m_tiles);
   p.chunk_kb = (passes == 3) ? CHUNK_MMAS / 12 : p.KB;   // 3-pass: 12 MMAs per k-block; 1-pass: one chain
-  p.b_bytes = (uint32_t)p.BN * BK * 4;
+  p.b_bytes = (uint32_t)(pair ? p.BN / 2 : p.BN) * BK * 4;
   p.stage_bytes = (passes == 3) ? (2 * A_BYTES + 2 * p.b_bytes) : (A_BYTES + p.b_bytes);
   p.stages = (int)((SMEM_LIMIT - 2048) / p.stage_bytes);
   if (p.stages > MAX_STAGES) p.stages = MAX_STAGES;
@@ -312,29 +351,35 @@ int gemm_tcgen05(const dcae_operand* a, const dcae_weight* w, const dcae_epilogu
   {
     cuuint64_t dims[4] = {(cuuint64_t)a->ld, (cuuint64_t)a->w, (cuuint64_t)a->h, (cuuint64_t)a->B};
     cuuint64_t str[3] = {(cuuint64_t)a->ld * 4, (cuuint64_t)a->ld * 4 * a->w, (cuuint64_t)a->ld * 4 * a->w * a->h};
-    cuuint32_t box[4] = {BK, (cuuint32_t)p.TW, (cuuint32_t)p.TH, 1};
-    DCAE_TRY(encode_map(&map_a, a->base, 4, dims, str, box));
+    cuuint32_t box[4] = {BK, (cuuint32_t)p.tt.TW, (cuuint32_t)p.tt.TH, 1};
+    DCAE_TRY(encode_map(&map_a, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, a->base, 4, dims, str, box));
   }
   {
     cuuint64_t dims[2] = {(cuuint64_t)w->K, (cuuint64_t)w->N};
     cuuint64_t str[1] = {(cuuint64_t)w->K * 4};
-    cuuint32_t box[2] = {BK, (cuuint32_t)p.BN};
-    DCAE_TRY(encode_map(&map_bh, w->w_hi, 2, dims, str, box));
-    if (passes == 3) DCAE_TRY(encode_map(&map_bl, w->w_lo, 2, dims, str, box));
+    cuuint32_t box[2] = {BK, (cuuint32_t)(pair ? p.BN / 2 : p.BN)};
+    DCAE_TRY(encode_map(&map_bh, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, w->w_hi, 2, dims, str, box));
+    if (passes == 3) DCAE_TRY(encode_map(&map_bl, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, w->w_lo, 2, dims, str, box));
     else map_bl = map_bh;
   }
   static std::once_flag attr_once;
   static cudaError_t attr_err = cudaSuccess;
   std::call_once(attr_once, [] {
-    attr_err = cudaFuncSetAttribute(gemm_tcgen05_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_LIMIT - 1024);
-    if (attr_err == cudaSuccess)
-      attr_err = cudaFuncSetAttribute(gemm_tcgen05_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_LIMIT - 1024);
+    const void* kernels[3] = {(const void*)gemm_tcgen05_kernel<1>, (const void*)gemm_tcgen05_kernel<3>,
+                              (const void*)gemm_tcgen05_2cta_kernel<3>};
+    for (int i = 0; i < 3 && attr_err == cudaSuccess; ++i)
+      attr_err = cudaFuncSetAttribute(kernels[i], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_LIMIT - 1024);
   });
   DCAE_CUDA(attr_err);
-  const int ctas = p.total_tiles < num_sms() ? p.total_tiles : num_sms();
-  dim3 grid((unsigned)ctas);
-  if (passes == 3) gemm_tcgen05_kernel<3><<<grid, NTHREADS, smem, s>>>(map_a, map_bh, map_bl, p);
-  else gemm_tcgen05_kernel<1><<<grid, NTHREADS, smem, s>>>(map_a, map_bh, map_bl, p);
+  if (pair) {       // the pair kernel's cluster shape is fixed at compile time (__cluster_dims__)
+    const int max_pairs = num_sms() / 2;
+    const int pairs = p.total_tiles < max_pairs ? p.total_tiles : max_pairs;
+    gemm_tcgen05_2cta_kernel<3><<<dim3((unsigned)(2 * pairs)), NTHREADS, smem, s>>>(map_a, map_bh, map_bl, p);
+  } else {
+    const int ctas = p.total_tiles < num_sms() ? p.total_tiles : num_sms();
+    if (passes == 3) gemm_tcgen05_kernel<3><<<dim3((unsigned)ctas), NTHREADS, smem, s>>>(map_a, map_bh, map_bl, p);
+    else gemm_tcgen05_kernel<1><<<dim3((unsigned)ctas), NTHREADS, smem, s>>>(map_a, map_bh, map_bl, p);
+  }
   DCAE_LAUNCH_CHECK();
   return DCAE_OK;
 }

@@ -45,7 +45,8 @@ struct F16Params {
   dcae_epilogue e;
   int N, KB;                 // KB = taps * (Kp / 64)
   int cblk_per_tap, taps;
-  int B, h, w, TH, TW, tw_shift, tiles_x, tiles_y;
+  int B, h, w;
+  TokenTiling tt;
   int BN, stages, tmem_cols;
   int n_tiles_n, total_tiles, chunk_kb;
   float descale;
@@ -82,15 +83,6 @@ __device__ __forceinline__ void drain_chunk_f16(float* acc, uint32_t taddr, int 
       }
     }
   }
-}
-
-__device__ __forceinline__ void mma_f16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
 }
 
 __device__ __forceinline__ void tma_store_4d(const CUtensorMap* map, uint32_t src, int c0, int c1, int c2, int c3) {
@@ -220,37 +212,10 @@ __global__ void __launch_bounds__(256) split_f16_weight_kernel(const float* __re
   }
 }
 
-__device__ __forceinline__ void mma_f16_2sm(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void mbar_wait_cl(uint32_t bar, uint32_t parity) {   // cluster-scope acquire (peer CTA wrote / signalled)
-  uint32_t done = 0, spins = 0;
-  uint64_t t0 = 0;
-  while (true) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.b32 %0, 1, 0, p;\n\t}"
-        : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-    if (done) break;
-    if ((++spins & 1023u) == 0) {
-      uint64_t now;
-      asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now));
-      if (t0 == 0) t0 = now;
-      else if (now - t0 > 2000000000ull) __trap();
-    }
-  }
-}
-
 // debug-only: wait and report the cycles spent blocked (0 when the barrier was already complete)
 __device__ __forceinline__ long long timed_wait(uint32_t bar, uint32_t parity, bool cl) {
   const long long t0 = clock64();
-  if (cl) mbar_wait_cl(bar, parity); else mbar_wait(bar, parity);
+  if (cl) mbar_wait_cluster(bar, parity); else mbar_wait(bar, parity);
   return clock64() - t0;
 }
 
@@ -299,15 +264,7 @@ __device__ __forceinline__ void gemm_f16x3_body(const CUtensorMap& map_ah, const
     asm volatile("prefetch.tensormap [%0];" ::"l"(&map_bh) : "memory");
     asm volatile("prefetch.tensormap [%0];" ::"l"(&map_bl) : "memory");
   }
-  if (warp == 1) {
-    if (PAIR) {
-      asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_slot)), "r"(p.tmem_cols) : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    } else {
-      asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_slot)), "r"(p.tmem_cols) : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-  }
+  if (warp == 1) tmem_alloc<PAIR ? 2 : 1>(smem_u32(&tmem_base_slot), p.tmem_cols);
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
   if (PAIR) cluster_sync_all();     // the peer's barriers exist before anything signals them
@@ -322,10 +279,10 @@ __device__ __forceinline__ void gemm_f16x3_body(const CUtensorMap& map_ah, const
   auto tile_coords = [&](int t, int& b, int& y0, int& x0, int& n0) {
     const int nt = t % p.n_tiles_n;
     int mt = PAIR ? (t / p.n_tiles_n) * 2 + (int)rank : t / p.n_tiles_n;   // b may reach B for a pair's odd tail tile
-    const int tile_x = mt % p.tiles_x; mt /= p.tiles_x;
-    const int tile_y = mt % p.tiles_y;
-    b = mt / p.tiles_y;
-    x0 = tile_x * p.TW; y0 = tile_y * p.TH; n0 = nt * p.BN;
+    const int tile_x = mt % p.tt.tiles_x; mt /= p.tt.tiles_x;
+    const int tile_y = mt % p.tt.tiles_y;
+    b = mt / p.tt.tiles_y;
+    x0 = tile_x * p.tt.TW; y0 = tile_y * p.tt.TH; n0 = nt * p.BN;
   };
 
   if (warp < 4) {
@@ -372,9 +329,8 @@ __device__ __forceinline__ void gemm_f16x3_body(const CUtensorMap& map_ah, const
       if (DBG && lane == 0) p.dbg[blockIdx.x * 24 + 0] = (unsigned long long)w_empty;
     } else if (warp == 1 && leader) {
       // ===================== MMA issuer (the leader CTA of a pair; warp-uniform, one elected lane issues) =====================
-      // D = F32 (bit 4), A = B = F16 (format 0), K-major, N >> 3 at bit 17, M >> 4 at bit 24
-      const uint32_t idesc = (1u << 4) | ((uint32_t)(p.BN >> 3) << 17) | ((uint32_t)(((PAIR ? 2 : 1) * BM) >> 4) << 24);
-      const uint32_t idesc2 = (1u << 4) | ((uint32_t)((2 * p.BN) >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);   // fuse_b: N = 2 BN
+      const uint32_t idesc = make_idesc_f16((PAIR ? 2 : 1) * BM, p.BN);
+      const uint32_t idesc2 = make_idesc_f16(BM, 2 * p.BN);   // fuse_b: N = 2 BN
       int stage = 0;
       uint32_t phase = 0, gchunk = 0;
       long long w_full = 0, w_tmem = 0, n_kb = 0, n_tiles = 0;
@@ -385,14 +341,14 @@ __device__ __forceinline__ void gemm_f16x3_body(const CUtensorMap& map_ah, const
         for (int ck = 0; ck < n_chunks; ++ck, ++gchunk) {
           const uint32_t buf = gchunk & 1;
           if (DBG) w_tmem += timed_wait(smem_u32(&tmem_empty_bar[buf]), ((gchunk >> 1) & 1) ^ 1, PAIR);
-          else if (PAIR) mbar_wait_cl(smem_u32(&tmem_empty_bar[buf]), ((gchunk >> 1) & 1) ^ 1);
+          else if (PAIR) mbar_wait_cluster(smem_u32(&tmem_empty_bar[buf]), ((gchunk >> 1) & 1) ^ 1);
           else mbar_wait(smem_u32(&tmem_empty_bar[buf]), ((gchunk >> 1) & 1) ^ 1);
           asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
           const uint32_t tmem_acc = tmem_base + buf * (uint32_t)(p.fuse_b ? 2 * p.BN : p.BN);
           const int kb_end = min(p.KB, (ck + 1) * p.chunk_kb);
           for (int kb = ck * p.chunk_kb; kb < kb_end; ++kb) {
             if (DBG) { w_full += timed_wait(smem_u32(&full_bar[stage]), phase, PAIR); ++n_kb; }
-            else if (PAIR) mbar_wait_cl(smem_u32(&full_bar[stage]), phase);
+            else if (PAIR) mbar_wait_cluster(smem_u32(&full_bar[stage]), phase);
             else mbar_wait(smem_u32(&full_bar[stage]), phase);
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
             const uint32_t sbase = smem0 + stage * p.stage_bytes;
@@ -449,7 +405,7 @@ __device__ __forceinline__ void gemm_f16x3_body(const CUtensorMap& map_ah, const
     for (int t = unit; t < p.total_tiles; t += nunits) {
       EpiTile et;
       tile_coords(t, et.b, et.y0, et.x0, et.n0);
-      et.B = p.B; et.h = p.h; et.w = p.w; et.tw_shift = p.tw_shift; et.N = p.N; et.BN = p.BN;
+      et.B = p.B; et.h = p.h; et.w = p.w; et.tw_shift = p.tt.tw_shift; et.N = p.N; et.BN = p.BN;
       float acc[NB * 32];
       float bias_l[NB], rs_l[NB];          // column (block g, lane) of bias / res_scale, see finalize_block
 #pragma unroll
@@ -479,7 +435,7 @@ __device__ __forceinline__ void gemm_f16x3_body(const CUtensorMap& map_ah, const
       const dcae_epilogue& e = p.e;
       const int act_cols = (e.act_cols <= 0 || e.act_cols > p.N) ? p.N : e.act_cols;
       const int row = quarter * 32 + lane;
-      const int yy = et.y0 + (row >> p.tw_shift), xx = et.x0 + (row & ((1 << p.tw_shift) - 1));
+      const int yy = et.y0 + (row >> p.tt.tw_shift), xx = et.x0 + (row & ((1 << p.tt.tw_shift) - 1));
       const bool row_ok = yy < p.h && xx < p.w && et.b < p.B;
       const int64_t token = ((int64_t)et.b * p.h + yy) * p.w + xx;
       const uint32_t stg = stg_base + (uint32_t)half * STG_BYTES;
@@ -547,10 +503,7 @@ __device__ __forceinline__ void gemm_f16x3_body(const CUtensorMap& map_ah, const
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
   if (PAIR) cluster_sync_all();     // neither CTA may free TMEM / exit while the pair still uses its smem or TMEM
-  if (warp == 1) {
-    if (PAIR) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(p.tmem_cols) : "memory");
-    else asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(p.tmem_cols) : "memory");
-  }
+  if (warp == 1) tmem_dealloc<PAIR ? 2 : 1>(tmem_base, p.tmem_cols);
   if (DBG && threadIdx.x == 32) {
     unsigned long long gt;
     asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt));
@@ -577,34 +530,6 @@ gemm_f16x3_pair_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_
                        const __grid_constant__ CUtensorMap map_ol, const __grid_constant__ CUtensorMap map_oha,
                        const __grid_constant__ CUtensorMap map_ola, const F16Params p) {
   gemm_f16x3_body<true, DBG, NB>(map_ah, map_al, map_bh, map_bl, map_o32, map_oh, map_ol, map_oha, map_ola, p);
-}
-
-int encode_map_f16(CUtensorMap* m, const void* base, int rank, const cuuint64_t* dims, const cuuint64_t* strides_bytes,
-                   const cuuint32_t* box, CUtensorMapSwizzle swz = CU_TENSOR_MAP_SWIZZLE_128B) {
-  EncodeTiledFn enc = get_encode();
-  if (!enc) {
-    set_error("cuTensorMapEncodeTiled is not available from the driver");
-    return DCAE_E_CUDA;
-  }
-  cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, (cuuint32_t)rank, const_cast<void*>(base), dims, strides_bytes, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled(f16) failed with CUresult %d (rank %d, dims %llu %llu, box %u %u)", (int)r, rank,
-              (unsigned long long)dims[0], (unsigned long long)dims[1], box[0], box[1]);
-    return DCAE_E_CUDA;
-  }
-  return DCAE_OK;
-}
-
-void pick_tile16(int h, int w, int* TH, int* TW) {
-  int best = 1 << 30;
-  for (int tw = 128; tw >= 1; tw >>= 1) {
-    const int th = 128 / tw;
-    const int tiles = ((h + th - 1) / th) * ((w + tw - 1) / tw);
-    if (tiles < best || (tiles == best && tw == 16)) { best = tiles; *TH = th; *TW = tw; }
-  }
 }
 
 inline int pad64(int v) { return (v + 63) / 64 * 64; }
@@ -643,12 +568,8 @@ int gemm_tcgen05_f16x3(const dcae_operand* a, const dcae_weight* w, const dcae_e
   p.cblk_per_tap = Kp / BK16;
   p.KB = a->taps * p.cblk_per_tap;
   p.B = a->B; p.h = a->h; p.w = a->w;
-  pick_tile16(a->h, a->w, &p.TH, &p.TW);
-  p.tw_shift = 0;
-  while ((1 << p.tw_shift) < p.TW) ++p.tw_shift;
-  p.tiles_x = (a->w + p.TW - 1) / p.TW;
-  p.tiles_y = (a->h + p.TH - 1) / p.TH;
-  const int m_tiles = p.tiles_x * p.tiles_y * a->B;
+  p.tt = token_tiling(a->h, a->w);
+  const int m_tiles = p.tt.tiles_x * p.tt.tiles_y * a->B;
   // A/B sweeps (profiles/r01/gemm_f16_pair_ab.jsonl, layer_times_bn_pair_sweep3.log): pairs win where the mainloop is
   // long or wide (cc1, proj, fc1, the K = 2 016 conv layers); everything else runs single-CTA with BN <= 128 so that
   // the fused [b_hi; b_lo] MMA applies (N = 320 -> 128 + 128 + 64 ragged beats 2 x 160 by 20 %, N = 224 likewise).
@@ -701,40 +622,40 @@ int gemm_tcgen05_f16x3(const dcae_operand* a, const dcae_weight* w, const dcae_e
   CUtensorMap map_ah, map_al, map_bh, map_bl, map_o32, map_oh, map_ol, map_oha, map_ola;
   {
     // output boxes {32 columns, TW, TH, 1}; dims[0] = N clips a ragged last block, (w, h) clip ragged token tiles
-    cuuint32_t box[4] = {32, (cuuint32_t)p.TW, (cuuint32_t)p.TH, 1};
+    cuuint32_t box[4] = {32, (cuuint32_t)p.tt.TW, (cuuint32_t)p.tt.TH, 1};
     cuuint64_t dims[4] = {(cuuint64_t)w->N, (cuuint64_t)a->w, (cuuint64_t)a->h, (cuuint64_t)a->B};
     if (p.has_o32) {
       DCAE_REQUIRE(aligned16(e->out) && e->out_ld % 4 == 0, "gemm(f16x3): fp32 output must be 16-byte aligned with ld %% 4 == 0");
       cuuint64_t str[3] = {(cuuint64_t)e->out_ld * 4, (cuuint64_t)e->out_ld * 4 * a->w, (cuuint64_t)e->out_ld * 4 * a->w * a->h};
-      DCAE_TRY(encode_map(&map_o32, e->out, 4, dims, str, box));
+      DCAE_TRY(encode_map(&map_o32, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, e->out, 4, dims, str, box));
     }
     if (p.has_o16) {
       DCAE_REQUIRE(aligned16(e->out16.hi) && aligned16(e->out16.lo) && e->out16.ld % 8 == 0, "gemm(f16x3): output planes must be 16-byte aligned with ld %% 8 == 0");
       cuuint64_t str[3] = {(cuuint64_t)e->out16.ld * 2, (cuuint64_t)e->out16.ld * 2 * a->w, (cuuint64_t)e->out16.ld * 2 * a->w * a->h};
-      DCAE_TRY(encode_map_f16(&map_oh, e->out16.hi, 4, dims, str, box, CU_TENSOR_MAP_SWIZZLE_64B));
-      DCAE_TRY(encode_map_f16(&map_ol, e->out16.lo, 4, dims, str, box, CU_TENSOR_MAP_SWIZZLE_64B));
+      DCAE_TRY(encode_map(&map_oh, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, e->out16.hi, 4, dims, str, box, CU_TENSOR_MAP_SWIZZLE_64B));
+      DCAE_TRY(encode_map(&map_ol, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, e->out16.lo, 4, dims, str, box, CU_TENSOR_MAP_SWIZZLE_64B));
     }
     if (p.has_o16a) {
       DCAE_REQUIRE(aligned16(e->out16_act.hi) && aligned16(e->out16_act.lo) && e->out16_act.ld % 8 == 0, "gemm(f16x3): out16_act planes must be 16-byte aligned with ld %% 8 == 0");
       cuuint64_t str[3] = {(cuuint64_t)e->out16_act.ld * 2, (cuuint64_t)e->out16_act.ld * 2 * a->w, (cuuint64_t)e->out16_act.ld * 2 * a->w * a->h};
-      DCAE_TRY(encode_map_f16(&map_oha, e->out16_act.hi, 4, dims, str, box, CU_TENSOR_MAP_SWIZZLE_64B));
-      DCAE_TRY(encode_map_f16(&map_ola, e->out16_act.lo, 4, dims, str, box, CU_TENSOR_MAP_SWIZZLE_64B));
+      DCAE_TRY(encode_map(&map_oha, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, e->out16_act.hi, 4, dims, str, box, CU_TENSOR_MAP_SWIZZLE_64B));
+      DCAE_TRY(encode_map(&map_ola, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, e->out16_act.lo, 4, dims, str, box, CU_TENSOR_MAP_SWIZZLE_64B));
     }
   }
   {
     // dims[0] = Kp: a window that is not a multiple of 64 wide over-reads into the next columns (zero weights there)
     cuuint64_t dims[4] = {(cuuint64_t)Kp, (cuuint64_t)a->w, (cuuint64_t)a->h, (cuuint64_t)a->B};
     cuuint64_t str[3] = {(cuuint64_t)ldp * 2, (cuuint64_t)ldp * 2 * a->w, (cuuint64_t)ldp * 2 * a->w * a->h};
-    cuuint32_t box[4] = {BK16, (cuuint32_t)p.TW, (cuuint32_t)p.TH, 1};
-    DCAE_TRY(encode_map_f16(&map_ah, hi, 4, dims, str, box));
-    DCAE_TRY(encode_map_f16(&map_al, lo, 4, dims, str, box));
+    cuuint32_t box[4] = {BK16, (cuuint32_t)p.tt.TW, (cuuint32_t)p.tt.TH, 1};
+    DCAE_TRY(encode_map(&map_ah, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, hi, 4, dims, str, box));
+    DCAE_TRY(encode_map(&map_al, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, lo, 4, dims, str, box));
   }
   {
     cuuint64_t dims[2] = {(cuuint64_t)w->K16, (cuuint64_t)w->N};
     cuuint64_t str[1] = {(cuuint64_t)w->K16 * 2};
     cuuint32_t box[2] = {BK16, (cuuint32_t)(pair ? p.BN / 2 : p.BN)};
-    DCAE_TRY(encode_map_f16(&map_bh, w->w16_hi, 2, dims, str, box));
-    DCAE_TRY(encode_map_f16(&map_bl, w->w16_lo, 2, dims, str, box));
+    DCAE_TRY(encode_map(&map_bh, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, w->w16_hi, 2, dims, str, box));
+    DCAE_TRY(encode_map(&map_bl, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, w->w16_lo, 2, dims, str, box));
   }
   if (!p.has_o32) map_o32 = map_bh;       // unused by the kernel
   if (!p.has_o16) { map_oh = map_bh; map_ol = map_bh; }

@@ -41,6 +41,27 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
     }
   }
 }
+// the same wait with cluster-scope acquire: the data guarded by the barrier was written (or signalled) by the peer CTA
+__device__ __forceinline__ void mbar_wait_cluster(uint32_t bar, uint32_t parity) {
+  uint32_t done = 0, spins = 0;
+  uint64_t t0 = 0;
+  while (true) {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
+        "selp.b32 %0, 1, 0, p;\n\t}"
+        : "=r"(done)
+        : "r"(bar), "r"(parity)
+        : "memory");
+    if (done) break;
+    if ((++spins & 1023u) == 0) {
+      uint64_t now;
+      asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now));
+      if (t0 == 0) t0 = now;
+      else if (now - t0 > 2000000000ull) __trap();
+    }
+  }
+}
 __device__ __forceinline__ void tma_load_4d(uint32_t dst, const CUtensorMap* map, uint32_t bar, int c0, int c1, int c2, int c3) {
   asm volatile(
       "cp.async.bulk.tensor.4d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
@@ -77,6 +98,14 @@ __device__ __forceinline__ void mma_tf32(uint32_t tmem_d, uint64_t adesc, uint64
       "{\n\t.reg .pred p;\n\t"
       "setp.ne.b32 p, %4, 0;\n\t"
       "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
+      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+__device__ __forceinline__ void mma_f16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
       ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
@@ -134,6 +163,15 @@ __device__ __forceinline__ void mma_tf32_ts(uint32_t tmem_d, uint32_t tmem_a, ui
       ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+__device__ __forceinline__ void mma_f16_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+  // A operand from TMEM: 128 lanes x 8 columns per K = 16 step (two fp16 per 32-bit column), B from shared memory
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
+      ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 __device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t (&r)[16]) {
   asm volatile(
       "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], "
@@ -180,15 +218,47 @@ __device__ __forceinline__ void mma_tf32_2sm(uint32_t tmem_d, uint64_t adesc, ui
       ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+__device__ __forceinline__ void mma_f16_2sm(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
+      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 // commit: one arrival on the barrier at this offset in BOTH CTAs of the pair once all prior MMAs retire
 __device__ __forceinline__ void mma_commit_2sm(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
                ::"r"(bar), "h"((uint16_t)3) : "memory");
 }
 
+// TMEM allocation by one whole warp (CG = 1: this CTA; CG = 2: the same columns in both CTAs of the pair).  The
+// base address is written to the shared-memory word at `slot`.
+template <int CG>
+__device__ __forceinline__ void tmem_alloc(uint32_t slot, uint32_t ncols) {
+  static_assert(CG == 1 || CG == 2, "cta_group is 1 or 2");
+  if (CG == 1) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(slot), "r"(ncols) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+  } else {
+    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(slot), "r"(ncols) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+  }
+}
+template <int CG>
+__device__ __forceinline__ void tmem_dealloc(uint32_t base, uint32_t ncols) {
+  static_assert(CG == 1 || CG == 2, "cta_group is 1 or 2");
+  if (CG == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(base), "r"(ncols) : "memory");
+  else asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(base), "r"(ncols) : "memory");
+}
+
 __device__ __forceinline__ uint32_t make_idesc_tf32(int M, int N) {
   // D = F32 (bits 4-5), A = B = TF32 (bits 7-9, 10-12), both K-major, N >> 3 at bit 17, M >> 4 at bit 24
   return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
+}
+__device__ __forceinline__ uint32_t make_idesc_f16(int M, int N) {
+  // D = F32 (bits 4-5), A = B = F16 (format 0), both K-major, N >> 3 at bit 17, M >> 4 at bit 24
+  return (1u << 4) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
 
 // ---- drain + epilogue shared by the GEMM kernels ---------------------------------------------------
@@ -215,30 +285,21 @@ __device__ __forceinline__ void warp_transpose32(float* r, int lane) {
 
 // acc (+)= the chain partial sitting in TMEM at taddr (this warp's lane quarter, start of the chain buffer).
 // Both tcgen05.ld of a 32-column block are in flight per wait (more would spill next to the 128 running sums).
-template <int NB = EPI_BLOCKS>
 __device__ __forceinline__ void drain_chunk(float* acc, uint32_t taddr, int half, int BN, bool first) {
 #pragma unroll
-  for (int gg = 0; gg < NB; gg += 1) {
+  for (int g = 0; g < EPI_BLOCKS; ++g) {
+    const int blk = 2 * g + half;
     uint32_t raw[32];
-#pragma unroll
-    for (int g = gg; g < gg + 1; ++g) {
-      const int blk = 2 * g + half;
-      if (blk * 32 < BN) {                      // warp-uniform
-        tmem_ld16_nowait(taddr + blk * 32, raw + (g - gg) * 32);
-        tmem_ld16_nowait(taddr + blk * 32 + 16, raw + (g - gg) * 32 + 16);
-      }
+    if (blk * 32 < BN) {                        // warp-uniform
+      tmem_ld16_nowait(taddr + blk * 32, raw);
+      tmem_ld16_nowait(taddr + blk * 32 + 16, raw + 16);
     }
     tmem_ld_wait();
+    if (blk * 32 < BN) {
 #pragma unroll
-    for (int g = gg; g < gg + 1; ++g) {
-      const int blk = 2 * g + half;
-      if (blk * 32 < BN) {
-#pragma unroll
-        for (int j = 0; j < 32; ++j) {
-          const int i = g * 32 + j;
-          const float v = __uint_as_float(raw[(g - gg) * 32 + j]);
-          acc[i] = first ? v : __fadd_rn(acc[i], v);
-        }
+      for (int j = 0; j < 32; ++j) {
+        const float v = __uint_as_float(raw[j]);
+        acc[g * 32 + j] = first ? v : __fadd_rn(acc[g * 32 + j], v);
       }
     }
   }
@@ -337,25 +398,51 @@ EncodeTiledFn get_encode() {
   return fn;
 }
 
-int encode_map(CUtensorMap* m, const void* base, int rank, const cuuint64_t* dims, const cuuint64_t* strides_bytes,
-               const cuuint32_t* box) {
+// rank-1..5 tiled map of `dtype` elements; dims / box innermost first, strides_bytes for dims 1..rank-1
+int encode_map(CUtensorMap* m, CUtensorMapDataType dtype, const void* base, int rank, const cuuint64_t* dims,
+               const cuuint64_t* strides_bytes, const cuuint32_t* box, CUtensorMapSwizzle swizzle = CU_TENSOR_MAP_SWIZZLE_128B) {
   EncodeTiledFn enc = get_encode();
   if (!enc) {
     set_error("cuTensorMapEncodeTiled is not available from the driver");
     return DCAE_E_CUDA;
   }
   cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, (cuuint32_t)rank, const_cast<void*>(base), dims, strides_bytes, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  CUresult r = enc(m, dtype, (cuuint32_t)rank, const_cast<void*>(base), dims, strides_bytes, box, estr,
+                   CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled failed with CUresult %d (rank %d, dims %llu %llu, box %u %u)", (int)r, rank,
-              (unsigned long long)dims[0], (unsigned long long)dims[1], box[0], box[1]);
+    set_error("cuTensorMapEncodeTiled failed with CUresult %d (data type %d, rank %d, dims %llu %llu, box %u %u)", (int)r,
+              (int)dtype, rank, (unsigned long long)dims[0], (unsigned long long)dims[1], box[0], box[1]);
     return DCAE_E_CUDA;
   }
   return DCAE_OK;
 }
 
+// ---- host: token tiling of the GEMMs ----
+// 128 tokens per tile as a TH x TW box inside one image; minimise the number of tiles
+void pick_tile(int h, int w, int* TH, int* TW) {
+  int best = 1 << 30;
+  for (int tw = 128; tw >= 1; tw >>= 1) {
+    const int th = 128 / tw;
+    const int tiles = ((h + th - 1) / th) * ((w + tw - 1) / tw);
+    // prefer wide-ish boxes (tw = 16) on ties: longer contiguous rows per TMA line group
+    if (tiles < best || (tiles == best && tw == 16)) { best = tiles; *TH = th; *TW = tw; }
+  }
+}
+
+// token tile t_x + tiles_x * t_y covers rows [t_y * TH, +TH) and columns [t_x * TW, +TW) of an image; tile row r is
+// image row r >> tw_shift, column r & (TW - 1)
+struct TokenTiling {
+  int TH, TW, tw_shift, tiles_x, tiles_y;
+};
+TokenTiling token_tiling(int h, int w) {
+  TokenTiling t;
+  pick_tile(h, w, &t.TH, &t.TW);
+  t.tw_shift = 0;
+  while ((1 << t.tw_shift) < t.TW) ++t.tw_shift;
+  t.tiles_x = (w + t.TW - 1) / t.TW;
+  t.tiles_y = (h + t.TH - 1) / t.TH;
+  return t;
+}
 
 }  // namespace
 }  // namespace dcae
