@@ -1,7 +1,5 @@
 // C ABI glue + the host-side plan of the channel-slice loop
 // (/root/reference/models/dcae.py:638-670 forward, :713-753 compress, :878-906 decompress).
-#include <nvtx3/nvToolsExt.h>
-#include <stdlib.h>
 #include <stdarg.h>
 #include <string.h>
 
@@ -39,16 +37,7 @@ cudaEvent_t take_event() {
 }
 }  // namespace
 
-// DCAE_NVTX=1: every public operator call is an NVTX range named after its kernel family (header-only NVTX v3; a no-op when no
-// tool is attached), so that `ncu --nvtx --nvtx-include "gemm/"` or a timeline tool can select the launches of one family.
-static const bool g_nvtx = [] { const char* v = getenv("DCAE_NVTX"); return v && atoi(v) != 0; }();
-static const char* const kFamilyNames[DCAE_PROF_FAMILIES] = {"gemm", "attention", "gc", "other"};
-
-ProfileScope::ProfileScope(int family, double work, void* s) : slot(-1), stream(s), nvtx(false) {
-  if (g_nvtx && family >= 0 && family < DCAE_PROF_FAMILIES) {
-    nvtxRangePushA(kFamilyNames[family]);
-    nvtx = true;
-  }
+ProfileScope::ProfileScope(int family, double work, void* s) : slot(-1), stream(s) {
   if (!g_prof_on) return;
   ProfRec r{family, work, take_event(), take_event()};
   cudaEventRecord(r.a, (cudaStream_t)stream);
@@ -57,7 +46,6 @@ ProfileScope::ProfileScope(int family, double work, void* s) : slot(-1), stream(
 }
 ProfileScope::~ProfileScope() {
   if (slot >= 0) cudaEventRecord(g_prof[slot].b, (cudaStream_t)stream);
-  if (nvtx) nvtxRangePop();
 }
 bool profiling_on() { return g_prof_on; }
 

@@ -30,7 +30,6 @@
 #include "tc_common.cuh"
 
 #include <mutex>
-#include <vector>
 
 namespace dcae {
 
@@ -56,16 +55,8 @@ struct AfParams {
   int64_t T;
   int tiles;
   float k_descale, v_descale;
-  unsigned long long* dbg;   // DCAE_F16_DBG=1: per-CTA role counters (8 u64 each)
 };
 
-__device__ __forceinline__ long long af_timed_wait(uint32_t bar, uint32_t parity) {
-  const long long t0 = clock64();
-  mbar_wait(bar, parity);
-  return clock64() - t0;
-}
-
-template <bool DBG>
 __global__ void __launch_bounds__(AF_THREADS, 1)
 dict_attention_f16_kernel(const __grid_constant__ CUtensorMap map_qh, const __grid_constant__ CUtensorMap map_ql,
                           const __grid_constant__ CUtensorMap map_kh, const __grid_constant__ CUtensorMap map_kl,
@@ -114,13 +105,12 @@ dict_attention_f16_kernel(const __grid_constant__ CUtensorMap map_qh, const __gr
   if (warp == 0) {
     {
       // ===================== TMA producer: one stage per head pair (warp-uniform, one elected lane issues) =====================
-      long long w_empty = 0;
       for (int pr = 0; pr < total / 2; ++pr) {
         const int stage = pr % AF_STAGES;
         const uint32_t phase = (pr / AF_STAGES) & 1;
         const int gp = (int)blockIdx.x + pr * (int)gridDim.x;
         const int tile = gp / HP, hp = gp % HP;
-        if (DBG) w_empty += af_timed_wait(smem_u32(&empty_bar[stage]), phase ^ 1); else mbar_wait(smem_u32(&empty_bar[stage]), phase ^ 1);
+        mbar_wait(smem_u32(&empty_bar[stage]), phase ^ 1);
         const uint32_t sb = smem0 + stage * AF_STAGE;
         const uint32_t fb = smem_u32(&full_bar[stage]);
         if (elect_one()) {
@@ -137,18 +127,15 @@ dict_attention_f16_kernel(const __grid_constant__ CUtensorMap map_qh, const __gr
         }
         __syncwarp();
       }
-      if (DBG && lane == 0) p.dbg[blockIdx.x * 8 + 0] = (unsigned long long)w_empty;
     }
   } else if (warp == 1) {
     {
       // ===================== MMA issuer (warp-uniform, one elected lane issues) =====================
       const uint32_t idesc_s = make_idesc_f16(AF_M, AF_ND);     // S: N = 128
       const uint32_t idesc_o = make_idesc_f16(AF_M, AF_HD);     // O: N = 32
-      long long w_full = 0, w_p = 0, w_of = 0;
-      const long long t_mma0 = clock64();
       auto issue_s = [&](int g) {                                 // S(g) -> buffer g & 1
         const int pr = g >> 1, stage = pr % AF_STAGES;
-        if ((g & 1) == 0) { if (DBG) w_full += af_timed_wait(smem_u32(&full_bar[stage]), (pr / AF_STAGES) & 1); else mbar_wait(smem_u32(&full_bar[stage]), (pr / AF_STAGES) & 1); }
+        if ((g & 1) == 0) mbar_wait(smem_u32(&full_bar[stage]), (pr / AF_STAGES) & 1);
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
         const uint32_t sb = smem0 + stage * AF_STAGE;
         const uint32_t d = tmem + TF_SP + (uint32_t)(g & 1) * 128;
@@ -170,8 +157,8 @@ dict_attention_f16_kernel(const __grid_constant__ CUtensorMap map_qh, const __gr
       for (int g = 0; g < total; ++g) {
         const int b = g & 1, pr = g >> 1, stage = pr % AF_STAGES;
         const uint32_t sb = smem0 + stage * AF_STAGE;
-        if (DBG) w_p += af_timed_wait(smem_u32(&p_ready[b]), (g >> 1) & 1); else mbar_wait(smem_u32(&p_ready[b]), (g >> 1) & 1);
-        if (g >= 2) { if (DBG) w_of += af_timed_wait(smem_u32(&o_free[b]), ((g >> 1) & 1) ^ 1); else mbar_wait(smem_u32(&o_free[b]), ((g >> 1) & 1) ^ 1); }      // O(g-2) has been read back
+        mbar_wait(smem_u32(&p_ready[b]), (g >> 1) & 1);
+        if (g >= 2) mbar_wait(smem_u32(&o_free[b]), ((g >> 1) & 1) ^ 1);      // O(g-2) has been read back
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
         const uint32_t pa = tmem + TF_SP + (uint32_t)b * 128;                  // P_hi words at +0, P_lo words at +64
         const uint32_t od = tmem + TF_O + (uint32_t)b * 32;
@@ -190,11 +177,6 @@ dict_attention_f16_kernel(const __grid_constant__ CUtensorMap map_qh, const __gr
         }
         __syncwarp();
         if (g + 2 < total) issue_s(g + 2);                                      // overwrites P(g): in order behind PV(g)
-      }
-      if (DBG && lane == 0) {
-        unsigned long long* d = p.dbg + blockIdx.x * 8;
-        d[1] = (unsigned long long)w_full; d[2] = (unsigned long long)w_p; d[3] = (unsigned long long)w_of;
-        d[4] = (unsigned long long)(clock64() - t_mma0); d[5] = (unsigned long long)total;
       }
     }
   } else {
@@ -236,15 +218,13 @@ dict_attention_f16_kernel(const __grid_constant__ CUtensorMap map_qh, const __gr
         }
       }
     };
-    long long w_s = 0;
-    const long long t_sm0 = clock64();
     int last = -1;
     for (int g = group; g < total; g += AF_GROUPS) {
       const int b = g & 1;                                 // == group: each group keeps to its own S/P and O buffers
       const int head = (((int)blockIdx.x + (g >> 1) * (int)gridDim.x) % HP) * 2 + b;
       // softmax(sim * scale) = 2^(t - max t) / sum, t = acc * (k_descale * scale * log2 e)
       const float sc = __ldg(p.head_scale + head) * p.k_descale * 1.4426950408889634f;
-      if (DBG) w_s += af_timed_wait(smem_u32(&s_full[b]), (g >> 1) & 1); else mbar_wait(smem_u32(&s_full[b]), (g >> 1) & 1);
+      mbar_wait(smem_u32(&s_full[b]), (g >> 1) & 1);
       asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
       float s[HC];
       {
@@ -295,10 +275,6 @@ dict_attention_f16_kernel(const __grid_constant__ CUtensorMap map_qh, const __gr
     if (last >= 0) {
       row_sync();
       write_out(last);
-    }
-    if (DBG && warp == 2 && lane == 0) {
-      p.dbg[blockIdx.x * 8 + 6] = (unsigned long long)w_s;
-      p.dbg[blockIdx.x * 8 + 7] = (unsigned long long)(clock64() - t_sm0);
     }
   }
 
@@ -351,34 +327,12 @@ int dict_attention_tcgen05_f16(const dcae_planes* q16, const dcae_dict_kv* kv, i
   static std::once_flag once;
   static cudaError_t attr_err = cudaSuccess;
   std::call_once(once, [] {
-    attr_err = cudaFuncSetAttribute(dict_attention_f16_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, AF_STAGES * AF_STAGE + 1024);
-    if (attr_err == cudaSuccess)
-      attr_err = cudaFuncSetAttribute(dict_attention_f16_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, AF_STAGES * AF_STAGE + 1024);
+    attr_err = cudaFuncSetAttribute(dict_attention_f16_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, AF_STAGES * AF_STAGE + 1024);
   });
   DCAE_CUDA(attr_err);
   const int ctas = p.tiles * (AF_HEADS / 2) < num_sms() ? p.tiles * (AF_HEADS / 2) : num_sms();
-  static const bool dbg_on = getenv("DCAE_F16_DBG") != nullptr;
-  p.dbg = nullptr;
-  if (!dbg_on) {
-    dict_attention_f16_kernel<false><<<ctas, AF_THREADS, smem, s>>>(mqh, mql, mkh, mkl, mvh, mvl, p);
-    DCAE_LAUNCH_CHECK();
-    return DCAE_OK;
-  }
-  // debug only: synchronous launch with per-CTA role counters, summary on stderr
-  DCAE_CUDA(cudaMalloc(&p.dbg, (size_t)ctas * 8 * sizeof(unsigned long long)));
-  DCAE_CUDA(cudaMemsetAsync(p.dbg, 0, (size_t)ctas * 8 * sizeof(unsigned long long), s));
-  dict_attention_f16_kernel<true><<<ctas, AF_THREADS, smem, s>>>(mqh, mql, mkh, mkl, mvh, mvl, p);
+  dict_attention_f16_kernel<<<ctas, AF_THREADS, smem, s>>>(mqh, mql, mkh, mkl, mvh, mvl, p);
   DCAE_LAUNCH_CHECK();
-  std::vector<unsigned long long> hb((size_t)ctas * 8);
-  DCAE_CUDA(cudaStreamSynchronize(s));
-  DCAE_CUDA(cudaMemcpy(hb.data(), p.dbg, hb.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-  DCAE_CUDA(cudaFree(p.dbg));
-  double sum[8] = {0};
-  for (int c = 0; c < ctas; ++c)
-    for (int i = 0; i < 8; ++i) sum[i] += (double)hb[(size_t)c * 8 + i] / ctas;
-  fprintf(stderr, "[attdbg] T=%lld per CTA (cycles): head steps %.1f | mma total %.0f wait_full(stage) %.0f wait_p_ready %.0f wait_o_free %.0f | "
-                  "producer wait_empty %.0f | softmax total %.0f wait_s_full %.0f\n",
-          (long long)T, sum[5], sum[4], sum[1], sum[2], sum[3], sum[0], sum[7], sum[6]);
   return DCAE_OK;
 }
 

@@ -137,7 +137,6 @@ struct ProfileScope {
   ~ProfileScope();
   int slot;
   void* stream;
-  bool nvtx;
 };
 
 bool profiling_on();

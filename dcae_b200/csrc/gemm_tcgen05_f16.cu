@@ -16,11 +16,9 @@
 // fill), persistent CTAs, <= 96-MMA accumulation chains in two alternating TMEM buffers summed in fp32
 // registers (RZ-accumulator fix), epilogue overlapped with the next tile.
 #include <cuda_fp16.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 #include "tc_common.cuh"
-#include <vector>
 
 namespace dcae {
 
@@ -54,7 +52,6 @@ struct F16Params {
   int fuse_b;                // single CTA, BN <= 128: one N = 2 BN MMA covers a_hi x [b_hi; b_lo], see the MMA issuer
   int passes;                // 3 = hi/lo error-compensated (fp32-level accuracy); 1 = DCAE_MATH_F16: a_hi x b_hi only, lo planes never loaded
   uint32_t stage_bytes, b_bytes;
-  unsigned long long* dbg;   // DCAE_F16_DBG=1: per-CTA role counters (16 u64 each), see dump in the host wrapper
 };
 
 
@@ -212,19 +209,12 @@ __global__ void __launch_bounds__(256) split_f16_weight_kernel(const float* __re
   }
 }
 
-// debug-only: wait and report the cycles spent blocked (0 when the barrier was already complete)
-__device__ __forceinline__ long long timed_wait(uint32_t bar, uint32_t parity, bool cl) {
-  const long long t0 = clock64();
-  if (cl) mbar_wait_cluster(bar, parity); else mbar_wait(bar, parity);
-  return clock64() - t0;
-}
-
 // PAIR = false: one CTA per 128-token tile.  PAIR = true: thread-block pair (cta_group::2): the pair computes a
 // 256-token x BN tile with M = 256 MMAs issued by the leader; each CTA loads its own A planes and HALF of the weight
 // planes (BN/2 rows), TMA completion of both CTAs is credited to the leader's full barrier, tcgen05.commit is
 // multicast to both CTAs, the drain warps of both CTAs release the leader's TMEM-empty barrier.
 // NB = 32-column blocks per drain group and tile: 2 for BN <= 128 (64 accumulator registers), 4 up to BN = 256
-template <bool PAIR, bool DBG, int NB>
+template <bool PAIR, int NB>
 __device__ __forceinline__ void gemm_f16x3_body(const CUtensorMap& map_ah, const CUtensorMap& map_al, const CUtensorMap& map_bh,
                                                 const CUtensorMap& map_bl, const CUtensorMap& map_o32, const CUtensorMap& map_oh,
                                                 const CUtensorMap& map_ol, const CUtensorMap& map_oha, const CUtensorMap& map_ola,
@@ -236,12 +226,6 @@ __device__ __forceinline__ void gemm_f16x3_body(const CUtensorMap& map_ah, const
 
   const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0), lane = threadIdx.x & 31;   // warp: provably uniform
   const uint32_t smem0 = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  const long long t_entry = DBG ? clock64() : 0;
-  if (DBG && threadIdx.x == 32) {
-    unsigned long long gt;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt));
-    p.dbg[blockIdx.x * 24 + 16] = gt;
-  }
   const uint32_t rank = PAIR ? __shfl_sync(0xffffffffu, cluster_ctarank(), 0) : 0u;
   const bool leader = rank == 0;
   const int unit = PAIR ? (int)(blockIdx.x >> 1) : (int)blockIdx.x;          // which persistent worker (CTA or pair)
@@ -291,13 +275,11 @@ __device__ __forceinline__ void gemm_f16x3_body(const CUtensorMap& map_ah, const
       // ===================== TMA producer (warp-uniform; one elected lane issues) =====================
       int stage = 0;
       uint32_t phase = 0;
-      long long w_empty = 0;
       for (int t = unit; t < p.total_tiles; t += nunits) {
         int b, y0, x0, n0;
         tile_coords(t, b, y0, x0, n0);
         for (int kb = 0; kb < p.KB; ++kb) {
-          if (DBG) w_empty += timed_wait(smem_u32(&empty_bar[stage]), phase ^ 1, false);
-          else mbar_wait(smem_u32(&empty_bar[stage]), phase ^ 1);
+          mbar_wait(smem_u32(&empty_bar[stage]), phase ^ 1);
           const uint32_t sbase = smem0 + stage * p.stage_bytes;
           const uint32_t fb = smem_u32(&full_bar[stage]);
           const int tap = kb / p.cblk_per_tap;
@@ -326,30 +308,21 @@ __device__ __forceinline__ void gemm_f16x3_body(const CUtensorMap& map_ah, const
           if (++stage == p.stages) { stage = 0; phase ^= 1; }
         }
       }
-      if (DBG && lane == 0) p.dbg[blockIdx.x * 24 + 0] = (unsigned long long)w_empty;
     } else if (warp == 1 && leader) {
       // ===================== MMA issuer (the leader CTA of a pair; warp-uniform, one elected lane issues) =====================
       const uint32_t idesc = make_idesc_f16((PAIR ? 2 : 1) * BM, p.BN);
       const uint32_t idesc2 = make_idesc_f16(BM, 2 * p.BN);   // fuse_b: N = 2 BN
       int stage = 0;
       uint32_t phase = 0, gchunk = 0;
-      long long w_full = 0, w_tmem = 0, n_kb = 0, n_tiles = 0;
-      const long long t_start = clock64();
-      if (DBG && lane == 0) p.dbg[blockIdx.x * 24 + 12] = (unsigned long long)(t_start - t_entry);
       for (int t = unit; t < p.total_tiles; t += nunits) {
-        ++n_tiles;
         for (int ck = 0; ck < n_chunks; ++ck, ++gchunk) {
           const uint32_t buf = gchunk & 1;
-          if (DBG) w_tmem += timed_wait(smem_u32(&tmem_empty_bar[buf]), ((gchunk >> 1) & 1) ^ 1, PAIR);
-          else if (PAIR) mbar_wait_cluster(smem_u32(&tmem_empty_bar[buf]), ((gchunk >> 1) & 1) ^ 1);
-          else mbar_wait(smem_u32(&tmem_empty_bar[buf]), ((gchunk >> 1) & 1) ^ 1);
+          if (PAIR) mbar_wait_cluster(smem_u32(&tmem_empty_bar[buf]), ((gchunk >> 1) & 1) ^ 1); else mbar_wait(smem_u32(&tmem_empty_bar[buf]), ((gchunk >> 1) & 1) ^ 1);
           asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
           const uint32_t tmem_acc = tmem_base + buf * (uint32_t)(p.fuse_b ? 2 * p.BN : p.BN);
           const int kb_end = min(p.KB, (ck + 1) * p.chunk_kb);
           for (int kb = ck * p.chunk_kb; kb < kb_end; ++kb) {
-            if (DBG) { w_full += timed_wait(smem_u32(&full_bar[stage]), phase, PAIR); ++n_kb; }
-            else if (PAIR) mbar_wait_cluster(smem_u32(&full_bar[stage]), phase);
-            else mbar_wait(smem_u32(&full_bar[stage]), phase);
+            if (PAIR) mbar_wait_cluster(smem_u32(&full_bar[stage]), phase); else mbar_wait(smem_u32(&full_bar[stage]), phase);
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
             const uint32_t sbase = smem0 + stage * p.stage_bytes;
             const uint32_t first = (kb == ck * p.chunk_kb) ? 0u : 1u;
@@ -388,11 +361,6 @@ __device__ __forceinline__ void gemm_f16x3_body(const CUtensorMap& map_ah, const
           __syncwarp();
         }
       }
-      if (DBG && lane == 0) {
-        unsigned long long* d = p.dbg + blockIdx.x * 24;
-        d[1] = (unsigned long long)w_full; d[2] = (unsigned long long)w_tmem; d[3] = (unsigned long long)(clock64() - t_start);
-        d[4] = (unsigned long long)n_kb; d[5] = (unsigned long long)n_tiles;
-      }
     }
   } else {
     asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(REGS_DRAIN));
@@ -400,8 +368,6 @@ __device__ __forceinline__ void gemm_f16x3_body(const CUtensorMap& map_ah, const
     const int quarter = warp & 3;
     const int half = (warp - 4) >> 2;
     uint32_t gchunk = 0;
-    long long w_acc = 0, t_drain = 0, t_epi = 0, t_fin = 0, t_rd = 0, t_st = 0, t_b2 = 0;
-    const long long t_start = clock64();
     for (int t = unit; t < p.total_tiles; t += nunits) {
       EpiTile et;
       tile_coords(t, et.b, et.y0, et.x0, et.n0);
@@ -417,21 +383,17 @@ __device__ __forceinline__ void gemm_f16x3_body(const CUtensorMap& map_ah, const
       }
       for (int ck = 0; ck < n_chunks; ++ck, ++gchunk) {
         const uint32_t buf = gchunk & 1;
-        if (DBG) w_acc += timed_wait(smem_u32(&tmem_full_bar[buf]), (gchunk >> 1) & 1, false);
-        else mbar_wait(smem_u32(&tmem_full_bar[buf]), (gchunk >> 1) & 1);
-        const long long td0 = DBG ? clock64() : 0;
+        mbar_wait(smem_u32(&tmem_full_bar[buf]), (gchunk >> 1) & 1);
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
         drain_chunk_f16<NB>(acc, tmem_base + ((uint32_t)(quarter * 32) << 16) + buf * (uint32_t)(p.fuse_b ? 2 * p.BN : p.BN), half, p.BN, ck == 0, p.fuse_b != 0);
         asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
         if (PAIR) mbar_arrive_cluster(smem_u32(&tmem_empty_bar[buf]), 0); else mbar_arrive(smem_u32(&tmem_empty_bar[buf]));
-        if (DBG) t_drain += clock64() - td0;
       }
-      const long long te0 = DBG ? clock64() : 0;
       // ---- epilogue: registers -> swizzled staging -> TMA tensor store, one 32-column block at a time ----
       // A ROLLED loop with one copy of the body.  Fully unrolled (4 blocks x 3 activations x 3 outputs) the kernel was
       // 350 KB of straight-line SASS that each warp runs once per tile: instruction fetch, not arithmetic, set the
-      // epilogue time (every phase measured 10-20x its instruction count; DCAE_F16_DBG counters).  The accumulator
-      // registers need static indices, so the block's 32 values are selected into r[] first.
+      // epilogue time (every phase measured 10-20x its instruction count; role-counter logs under profiles/r01).  The
+      // accumulator registers need static indices, so the block's 32 values are selected into r[] first.
       const dcae_epilogue& e = p.e;
       const int act_cols = (e.act_cols <= 0 || e.act_cols > p.N) ? p.N : e.act_cols;
       const int row = quarter * 32 + lane;
@@ -452,9 +414,7 @@ __device__ __forceinline__ void gemm_f16x3_body(const CUtensorMap& map_ah, const
         const float bias_lane = bias_l[0], rs_lane = rs_l[0];
 #pragma unroll
         for (int j = 0; j < 32; ++j) r[j] *= p.descale;          // exact: power of two
-        const long long tf0 = DBG ? clock64() : 0;
         finalize_block(r, e, act, row_ok, token, nb0, bias_lane, rs_lane);
-        if (DBG) { r[0] += 0.f * __int_as_float(__float_as_int(r[31]) & 0); t_fin += clock64() - tf0; }
         // output o: 0 = fp32, 1 = fp16 planes, 2 = fp16 planes of act2(result), the next layer's GELU prologue.
         // One staging round each: wait until the previous store has read the buffer, stage, make the writes visible
         // to the async proxy, and let one thread issue the bulk store(s).
@@ -465,12 +425,9 @@ __device__ __forceinline__ void gemm_f16x3_body(const CUtensorMap& map_ah, const
 #pragma unroll
             for (int j = 0; j < 32; ++j) r[j] = gelu_fast(r[j]);
           }
-          long long c0 = DBG ? clock64() : 0, c1;
           if (issuer) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-          if (DBG) { c1 = clock64(); t_rd += c1 - c0; c0 = c1; }
           named_bar_sync(1 + half, 128);
           if (o == 0) stage_f32(r, row, stg); else stage_f16(r, row, stg);
-          if (DBG) { c1 = clock64(); t_st += c1 - c0; c0 = c1; }
           asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
           named_bar_sync(1 + half, 128);
           if (issuer) {
@@ -482,20 +439,12 @@ __device__ __forceinline__ void gemm_f16x3_body(const CUtensorMap& map_ah, const
             }
             asm volatile("cp.async.bulk.commit_group;" ::: "memory");
           }
-          if (DBG) { c1 = clock64(); t_b2 += c1 - c0; }
         }
 #pragma unroll
         for (int i = 0; i < (NB - 1) * 32; ++i) acc[i] = acc[i + 32];
 #pragma unroll
         for (int q = 0; q < NB - 1; ++q) { bias_l[q] = bias_l[q + 1]; rs_l[q] = rs_l[q + 1]; }
       }
-      if (DBG) t_epi += clock64() - te0;
-    }
-    if (DBG && warp == 4 && lane == 0) {
-      unsigned long long* d = p.dbg + blockIdx.x * 24;
-      d[6] = (unsigned long long)w_acc; d[7] = (unsigned long long)t_drain; d[8] = (unsigned long long)t_epi;
-      d[9] = (unsigned long long)(clock64() - t_start); d[10] = (unsigned long long)t_fin; d[11] = (unsigned long long)t_rd;
-      d[13] = (unsigned long long)t_st; d[15] = (unsigned long long)t_b2;
     }
     if (quarter == 0 && lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");   // all stores landed before exit
   }
@@ -504,32 +453,26 @@ __device__ __forceinline__ void gemm_f16x3_body(const CUtensorMap& map_ah, const
   __syncthreads();
   if (PAIR) cluster_sync_all();     // neither CTA may free TMEM / exit while the pair still uses its smem or TMEM
   if (warp == 1) tmem_dealloc<PAIR ? 2 : 1>(tmem_base, p.tmem_cols);
-  if (DBG && threadIdx.x == 32) {
-    unsigned long long gt;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt));
-    p.dbg[blockIdx.x * 24 + 17] = gt;
-    p.dbg[blockIdx.x * 24 + 14] = (unsigned long long)(clock64() - t_entry);
-  }
 }
 
-template <bool DBG, int NB>
+template <int NB>
 __global__ void __launch_bounds__(NTHREADS, 1)
 gemm_f16x3_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_constant__ CUtensorMap map_al,
                   const __grid_constant__ CUtensorMap map_bh, const __grid_constant__ CUtensorMap map_bl,
                   const __grid_constant__ CUtensorMap map_o32, const __grid_constant__ CUtensorMap map_oh,
                   const __grid_constant__ CUtensorMap map_ol, const __grid_constant__ CUtensorMap map_oha,
                   const __grid_constant__ CUtensorMap map_ola, const F16Params p) {
-  gemm_f16x3_body<false, DBG, NB>(map_ah, map_al, map_bh, map_bl, map_o32, map_oh, map_ol, map_oha, map_ola, p);
+  gemm_f16x3_body<false, NB>(map_ah, map_al, map_bh, map_bl, map_o32, map_oh, map_ol, map_oha, map_ola, p);
 }
 
-template <bool DBG, int NB>
+template <int NB>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1)
 gemm_f16x3_pair_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_constant__ CUtensorMap map_al,
                        const __grid_constant__ CUtensorMap map_bh, const __grid_constant__ CUtensorMap map_bl,
                        const __grid_constant__ CUtensorMap map_o32, const __grid_constant__ CUtensorMap map_oh,
                        const __grid_constant__ CUtensorMap map_ol, const __grid_constant__ CUtensorMap map_oha,
                        const __grid_constant__ CUtensorMap map_ola, const F16Params p) {
-  gemm_f16x3_body<true, DBG, NB>(map_ah, map_al, map_bh, map_bl, map_o32, map_oh, map_ol, map_oha, map_ola, p);
+  gemm_f16x3_body<true, NB>(map_ah, map_al, map_bh, map_bl, map_o32, map_oh, map_ol, map_oha, map_ola, p);
 }
 
 inline int pad64(int v) { return (v + 63) / 64 * 64; }
@@ -605,8 +548,6 @@ int gemm_tcgen05_f16x3(const dcae_operand* a, const dcae_weight* w, const dcae_e
   p.total_tiles = p.n_tiles_n * (pair ? (m_tiles + 1) / 2 : m_tiles);
   p.chunk_kb = CHUNK_MMAS / (passes == 1 ? 4 : p.fuse_b ? 8 : 12);      // accumulation chain per column: 1, 2 (fused) or 3 MMAs per K = 16 step, 4 steps per k-block
   p.descale = w->descale;
-  static const bool dbg_on = getenv("DCAE_F16_DBG") != nullptr;
-  p.dbg = nullptr;
   p.b_bytes = (uint32_t)(pair ? p.BN / 2 : p.BN) * BK16 * 2;     // a pair's CTA holds half of the weight rows
   p.stage_bytes = (passes == 3 ? 2 : 1) * (A16_BYTES + p.b_bytes);
   p.stages = (int)((SMEM_LIMIT - 2048 - 2 * STG_BYTES) / p.stage_bytes);
@@ -663,57 +604,20 @@ int gemm_tcgen05_f16x3(const dcae_operand* a, const dcae_weight* w, const dcae_e
   static std::once_flag attr_once;
   static cudaError_t attr_err = cudaSuccess;
   std::call_once(attr_once, [] {
-    const void* kernels[8] = {(const void*)gemm_f16x3_kernel<false, 2>, (const void*)gemm_f16x3_kernel<true, 2>,
-                              (const void*)gemm_f16x3_kernel<false, 4>, (const void*)gemm_f16x3_kernel<true, 4>,
-                              (const void*)gemm_f16x3_pair_kernel<false, 2>, (const void*)gemm_f16x3_pair_kernel<true, 2>,
-                              (const void*)gemm_f16x3_pair_kernel<false, 4>, (const void*)gemm_f16x3_pair_kernel<true, 4>};
-    for (int i = 0; i < 8 && attr_err == cudaSuccess; ++i)
+    const void* kernels[4] = {(const void*)gemm_f16x3_kernel<2>, (const void*)gemm_f16x3_kernel<4>,
+                              (const void*)gemm_f16x3_pair_kernel<2>, (const void*)gemm_f16x3_pair_kernel<4>};
+    for (int i = 0; i < 4 && attr_err == cudaSuccess; ++i)
       attr_err = cudaFuncSetAttribute(kernels[i], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_LIMIT - 1024);
   });
   DCAE_CUDA(attr_err);
   const int n_ctas = pair ? 2 * (p.total_tiles < num_sms() / 2 ? p.total_tiles : num_sms() / 2)
                           : (p.total_tiles < num_sms() ? p.total_tiles : num_sms());
-  if (dbg_on) {     // debug only: synchronous launch with per-CTA role counters, summary on stderr
-    DCAE_CUDA(cudaMalloc(&p.dbg, (size_t)n_ctas * 24 * sizeof(unsigned long long)));
-    DCAE_CUDA(cudaMemsetAsync(p.dbg, 0, (size_t)n_ctas * 24 * sizeof(unsigned long long), s));
-  }
   // the pair kernel's cluster shape is fixed at compile time (__cluster_dims__)
   const bool nb2 = p.BN <= 128;
-  decltype(&gemm_f16x3_kernel<false, 2>) kernel;
-  if (pair) kernel = dbg_on ? (nb2 ? gemm_f16x3_pair_kernel<true, 2> : gemm_f16x3_pair_kernel<true, 4>)
-                            : (nb2 ? gemm_f16x3_pair_kernel<false, 2> : gemm_f16x3_pair_kernel<false, 4>);
-  else kernel = dbg_on ? (nb2 ? gemm_f16x3_kernel<true, 2> : gemm_f16x3_kernel<true, 4>)
-                       : (nb2 ? gemm_f16x3_kernel<false, 2> : gemm_f16x3_kernel<false, 4>);
+  const auto kernel = pair ? (nb2 ? gemm_f16x3_pair_kernel<2> : gemm_f16x3_pair_kernel<4>)
+                           : (nb2 ? gemm_f16x3_kernel<2> : gemm_f16x3_kernel<4>);
   kernel<<<n_ctas, NTHREADS, smem, s>>>(map_ah, map_al, map_bh, map_bl, map_o32, map_oh, map_ol, map_oha, map_ola, p);
   DCAE_LAUNCH_CHECK();
-  if (dbg_on) {
-    std::vector<unsigned long long> hbuf((size_t)n_ctas * 24);
-    DCAE_CUDA(cudaStreamSynchronize(s));
-    DCAE_CUDA(cudaMemcpy(hbuf.data(), p.dbg, hbuf.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-    DCAE_CUDA(cudaFree(p.dbg));
-    double sum[16] = {0};
-    int nm = 0;
-    unsigned long long g0 = ~0ull, g1 = 0, g0max = 0, g1min = ~0ull;
-    for (int c = 0; c < n_ctas; ++c) {
-      const unsigned long long a0 = hbuf[(size_t)c * 24 + 16], a1 = hbuf[(size_t)c * 24 + 17];
-      if (a0 && a0 < g0) g0 = a0;
-      if (a0 > g0max) g0max = a0;
-      if (a1 > g1) g1 = a1;
-      if (a1 && a1 < g1min) g1min = a1;
-    }
-    for (int c = 0; c < n_ctas; ++c) {
-      if (hbuf[(size_t)c * 24 + 3] == 0 && pair) continue;        // non-leader CTA of a pair: no MMA thread
-      ++nm;
-      for (int i = 0; i < 16; ++i) sum[i] += (double)hbuf[(size_t)c * 24 + i];
-    }
-    const double inv = nm ? 1.0 / nm : 0.0;
-    fprintf(stderr,
-            "[f16dbg] N=%d K=%d taps=%d BN=%d stages=%d pair=%d outs=%d%d%d | per CTA (cycles): mma_total %.0f wait_full %.0f wait_tmem %.0f "
-            "kblocks %.0f tiles %.1f | producer wait_empty %.0f | drain total %.0f wait_acc %.0f tmem_ld %.0f epilogue %.0f (finalize %.0f wait_read %.0f bar+stage %.0f fence+bar+issue %.0f) | prologue %.0f cta_total %.0f | grid span %.1f us, entry skew %.1f us, exit skew %.1f us\n",
-            p.N, (int)Kp * p.taps, p.taps, p.BN, p.stages, (int)pair, p.has_o32, p.has_o16, p.has_o16a, sum[3] * inv, sum[1] * inv,
-            sum[2] * inv, sum[4] * inv, sum[5] * inv, sum[0] * inv, sum[9] * inv, sum[6] * inv, sum[7] * inv, sum[8] * inv, sum[10] * inv, sum[11] * inv, sum[13] * inv, sum[15] * inv, sum[12] * inv, sum[14] * inv,
-            (double)(g1 - g0) * 1e-3, (double)(g0max - g0) * 1e-3, (double)(g1 - g1min) * 1e-3);
-  }
   return DCAE_OK;
 }
 

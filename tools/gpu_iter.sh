@@ -16,5 +16,4 @@ run it_loop  900 python -m pytest tests/test_gpu_slice_loop.py -q -m gpu
 run it_bench 600 python bench.py --no-cpu-baseline
 run it_bench1 600 python bench.py --no-cpu-baseline --lanes 1
 run it_layers 300 python tools/layer_times.py
-run it_dbg 300 python tools/f16_dbg.py
 exit 0
