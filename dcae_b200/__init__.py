@@ -15,6 +15,8 @@ Public surface (mirrors the reference's operator interface for this path only):
                            window-attention backward kernel; dcae_b200/training.py)
   EntropyBottleneckModel, DCAEModel, dcae_rate_distortion_loss -- the trainable bottleneck (backward kernel
                            dcae_eb_backward) and the whole DCAE as one trainable module (dcae_b200/training.py)
+  ms_ssim, MSSSIMStatsFunction -- MS-SSIM with the library's forward and backward kernels (dcae_b200/msssim.py); the
+                           distortion of dcae_rate_distortion_loss(..., metric="ms-ssim")
   DCAECodec             -- the whole model (forward / compress / decompress / update, image <-> .bin container) from a reference state dict
   container             -- the reference's bitstream container and image padding (compress_and_decompress.py:48-148)
 """
@@ -36,6 +38,9 @@ def __getattr__(name):
                 "EntropyBottleneckFunction", "EntropyBottleneckModel", "DCAEModel", "dcae_rate_distortion_loss"):
         from . import training
         return getattr(training, name)
+    if name in ("ms_ssim", "MSSSIMStatsFunction"):
+        from . import msssim
+        return getattr(msssim, name)
     if name == "EntropyBottleneck":
         from .entropy_bottleneck import EntropyBottleneck
         return EntropyBottleneck

@@ -66,6 +66,18 @@ class EbBwdArgs(C.Structure):
                 ("grad_z", c_f32p), ("grad_params", c_f32p)]
 
 
+class MsssimArgs(C.Structure):
+    _fields_ = [("x", c_f32p), ("y", c_f32p), ("B", C.c_int32), ("C", C.c_int32), ("H", C.c_int32), ("W", C.c_int32),
+                ("data_range", C.c_float), ("scratch", C.c_void_p), ("scratch_bytes", C.c_size_t),
+                ("ssim", c_f32p), ("cs", c_f32p)]
+
+
+class MsssimBwdArgs(C.Structure):
+    _fields_ = [("x", c_f32p), ("y", c_f32p), ("B", C.c_int32), ("C", C.c_int32), ("H", C.c_int32), ("W", C.c_int32),
+                ("data_range", C.c_float), ("scratch", C.c_void_p), ("scratch_bytes", C.c_size_t),
+                ("grad_ssim", c_f32p), ("grad_cs", c_f32p), ("grad_x", c_f32p)]
+
+
 class CoderTables(C.Structure):
     _fields_ = [("cdfs", C.c_void_p), ("cdf_stride", C.c_int32), ("cdf_sizes", C.c_void_p), ("offsets", C.c_void_p),
                 ("n_cdfs", C.c_int32)]
@@ -157,6 +169,9 @@ SIGNATURES = {
     "dcae_gc_backward": (C.c_int, [C.POINTER(GcBwdArgs), _P]),
     "dcae_eb_fused": (C.c_int, [C.POINTER(EbArgs), _P]),
     "dcae_eb_backward": (C.c_int, [C.POINTER(EbBwdArgs), _P]),
+    "dcae_msssim_scratch_bytes": (C.c_size_t, [_I32, _I32, _I32, _I32]),
+    "dcae_msssim_forward": (C.c_int, [C.POINTER(MsssimArgs), _P]),
+    "dcae_msssim_backward": (C.c_int, [C.POINTER(MsssimBwdArgs), _P]),
     "dcae_gc_num_partials": (_I64, [_I64, _I64]),
     "dcae_reduce_partials": (C.c_int, [_P, _I64, _P, _P]),
     "dcae_op_gemm": (C.c_int, [C.POINTER(Operand), C.POINTER(Weight), C.POINTER(Epilogue), C.c_int, _P]),

@@ -40,6 +40,7 @@ from .entropy_bottleneck import EntropyBottleneck
 from .entropy_model import EntropySliceLoop, get_scale_table
 from .gaussian_conditional import GaussianConditional
 from .modules import HOT_PREFIXES
+from .msssim import ms_ssim
 from .params import init_entropy_params
 from .transforms import STACKS, TransformStack, init_transform_params, transform_param_shapes
 
@@ -304,13 +305,20 @@ def rate_distortion_loss(likelihoods: torch.Tensor, y_hat: torch.Tensor, target:
     return lmbda * 255 ** 2 * mse + bpp, bpp, mse
 
 
-def dcae_rate_distortion_loss(out: dict, target: torch.Tensor, lmbda: float = 0.013):
-    """train.py:82-88 with type='mse' for the whole model: bpp = sum over BOTH likelihood tensors (y and z) of
-    sum(log lik) / (-ln 2 * pixels), pixels = N * H * W of the image; loss = lmbda * 255^2 * mse(x_hat, target) + bpp.
-    -> (loss, bpp, mse)."""
+def dcae_rate_distortion_loss(out: dict, target: torch.Tensor, lmbda: float = 0.013, metric: str = "mse"):
+    """train.py:82-88 for the whole model: bpp = sum over BOTH likelihood tensors (y and z) of
+    sum(log lik) / (-ln 2 * pixels), pixels = N * H * W of the image.
+      metric="mse"      loss = lmbda * 255^2 * mse(x_hat, target) + bpp              -> (loss, bpp, mse)
+      metric="ms-ssim"  loss = lmbda * (1 - ms_ssim(x_hat, target, data_range=1)) + bpp  -> (loss, bpp, ms_ssim)
+    (the ms-ssim form of the TCM-lineage RateDistortionLoss; MS-SSIM on the library's kernels, dcae_b200/msssim.py)."""
+    if metric not in ("mse", "ms-ssim"):
+        raise ValueError(f"dcae_rate_distortion_loss: metric must be 'mse' or 'ms-ssim', got {metric!r}")
     N, _, H, W = target.shape
     pixels = N * H * W
     bpp = sum(torch.log(lik).sum() / (-_math.log(2) * pixels) for lik in out["likelihoods"].values())
+    if metric == "ms-ssim":
+        msssim = ms_ssim(out["x_hat"], target, data_range=1.0)
+        return lmbda * (1 - msssim) + bpp, bpp, msssim
     mse = F.mse_loss(out["x_hat"], target)
     return lmbda * 255 ** 2 * mse + bpp, bpp, mse
 

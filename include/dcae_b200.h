@@ -174,6 +174,37 @@ typedef struct {
 int dcae_eb_backward(const dcae_eb_bwd_args* a, void* stream);
 
 /* --------------------------------------------------------------------------------------------
+ * MS-SSIM statistics (the distortion of the ms-ssim rate-distortion loss): pytorch_msssim.ms_ssim v1.0 with its
+ * defaults -- 11-tap Gaussian window (sigma 1.5) as a valid separable correlation, C1 = (0.01 R)^2, C2 = (0.03 R)^2,
+ * 5 levels joined by avg_pool2d(2, 2, padding = (h % 2, w % 2), count_include_pad).  x, y: fp32 NCHW [B, C, H, W],
+ * min(H, W) > 160.  The forward writes the per-level means of the ssim and cs maps of each plane, ssim / cs [5, B, C]
+ * (level-major); the weighted product over the levels is left to the caller.  The backward takes dL/dssim and dL/dcs
+ * [5, B, C] and overwrites grad_x [B, C, H, W] = dL/dx (y gets no gradient).  Both take the same scratch, of at least
+ * dcae_msssim_scratch_bytes(B, C, H, W) bytes, 16-byte aligned: the forward leaves the pooled pyramid of x and y there
+ * and the backward reads it, so the backward must see the scratch of the forward on the same x and y.
+ * Deterministic, no atomics; a plane's results do not depend on the other planes.  No host synchronisation.
+ * ------------------------------------------------------------------------------------------*/
+typedef struct {
+  const float* x; const float* y;
+  int32_t B, C, H, W;
+  float data_range;                        /* R > 0 */
+  void* scratch; size_t scratch_bytes;
+  float* ssim; float* cs;                  /* [5, B, C] */
+} dcae_msssim_args;
+typedef struct {
+  const float* x; const float* y;
+  int32_t B, C, H, W;
+  float data_range;
+  void* scratch; size_t scratch_bytes;     /* as left by dcae_msssim_forward */
+  const float* grad_ssim; const float* grad_cs;   /* [5, B, C] */
+  float* grad_x;                           /* [B, C, H, W] */
+} dcae_msssim_bwd_args;
+/* scratch bytes for both directions; 0 for a shape they reject */
+size_t dcae_msssim_scratch_bytes(int32_t B, int32_t C, int32_t H, int32_t W);
+int dcae_msssim_forward(const dcae_msssim_args* a, void* stream);
+int dcae_msssim_backward(const dcae_msssim_bwd_args* a, void* stream);
+
+/* --------------------------------------------------------------------------------------------
  * Elementary token-major operators (each replaces one torch dispatch chain of dcae.py:300-509).
  * ------------------------------------------------------------------------------------------*/
 

@@ -1,12 +1,15 @@
 """One training step of the whole DCAE (train.py:165-179) at the crops of config #4 (8 and 16 crops of 256x256 per step).
 
-    python tools/dcae_train_step.py [--batches 8 16] [--rounds 5] [--iters 3] [--out profiles/r03/dcae_train_step.log]
+    python tools/dcae_train_step.py [--batches 8 16] [--rounds 5] [--iters 3] [--metric {mse,ms-ssim}]
+                                    [--out profiles/r03/dcae_train_step.log]
 
 1. Median step time (CUDA events; one warm-up step, then the median over rounds of `iters` steps) and peak memory
    (max_memory_allocated) of forward, main backward, aux backward and both Adam steps, two ways:
      library   dcae_b200.DCAEModel
      eager     the same graph in eager torch, fp32, TF32 off: transform_graph stacks, torch_graph.slice_loop with a torch
                Gaussian likelihood, and a torch entropy bottleneck
+   with the loss of --metric: mse (default) or ms-ssim (library: dcae_rate_distortion_loss(metric="ms-ssim") on the MS-SSIM
+   kernels; eager: the same loss with oracle/msssim.py's torch MS-SSIM).
 2. The entropy-bottleneck backward kernel alone (dcae_eb_backward) at the training shape of z and at 4 x 3840x2160
    (z = 4 x 192 x 60 x 34 after padding to multiples of 128), against torch autograd of the same likelihood.
 The device name and power limit are read in the same run and printed first.
@@ -28,6 +31,7 @@ from dcae_b200 import _lib, torch_graph, transform_graph  # noqa: E402
 from dcae_b200.modules import HOT_PREFIXES  # noqa: E402
 from oracle import entropy_bottleneck as oeb  # noqa: E402
 from oracle import gaussian_conditional as ogc  # noqa: E402
+from oracle import msssim as oms  # noqa: E402
 
 C = 192
 
@@ -82,7 +86,15 @@ def eager_aux_loss(P):
     return torch.abs(oeb.logits_cumulative(p, p["quantiles"]) - torch.tensor([-target, 0.0, target], device=p["quantiles"].device)).sum()
 
 
-def step_fn(kind, B, dev):
+def eager_ms_ssim_loss(out, target, lmbda=0.013):
+    """dcae_rate_distortion_loss(metric="ms-ssim") with the torch MS-SSIM of the oracle."""
+    bpp = sum(torch.log(lik).sum() / (-math.log(2) * target.shape[0] * target.shape[2] * target.shape[3])
+              for lik in out["likelihoods"].values())
+    msssim = oms.ms_ssim(out["x_hat"], target, data_range=1.0)
+    return lmbda * (1 - msssim) + bpp, bpp, msssim
+
+
+def step_fn(kind, B, dev, metric="mse"):
     from dcae_b200.training import DCAEModel, dcae_rate_distortion_loss
     model = DCAEModel(device=dev, seed=0).train()
     g = torch.Generator(device=dev).manual_seed(B)
@@ -101,11 +113,15 @@ def step_fn(kind, B, dev):
         run, aux_loss = (lambda: eager_forward(P, x, y_noise, z_noise)), (lambda: eager_aux_loss(P))
         del model
     opt, aux_opt = torch.optim.Adam(main, lr=1e-4), torch.optim.Adam(aux, lr=1e-3)
+    if kind == "eager" and metric == "ms-ssim":
+        loss_fn = eager_ms_ssim_loss
+    else:
+        loss_fn = lambda out, target: dcae_rate_distortion_loss(out, target, metric=metric)      # noqa: E731
 
     def fn():
         opt.zero_grad()
         aux_opt.zero_grad()
-        loss, _, _ = dcae_rate_distortion_loss(run(), x)
+        loss, _, _ = loss_fn(run(), x)
         loss.backward()
         opt.step()
         aux_loss().backward()
@@ -153,6 +169,7 @@ def main():
     ap.add_argument("--batches", type=int, nargs="+", default=[8, 16])
     ap.add_argument("--rounds", type=int, default=5)
     ap.add_argument("--iters", type=int, default=3)
+    ap.add_argument("--metric", choices=["mse", "ms-ssim"], default="mse")
     ap.add_argument("--out", default="")
     args = ap.parse_args()
     if not torch.cuda.is_available():
@@ -174,10 +191,10 @@ def main():
     for B in args.batches:
         parts = []
         for kind in ("library", "eager"):
-            t, mem = timed(step_fn(kind, B, dev), args.iters, args.rounds)
+            t, mem = timed(step_fn(kind, B, dev, args.metric), args.iters, args.rounds)
             parts.append(f"{kind} {t:.2f} ms {mem / 2**30:.2f} GiB")
             torch.cuda.empty_cache()
-        emit(f"train step (forward, main + aux backward, both Adam steps) B={B}x256x256: " + " | ".join(parts))
+        emit(f"train step (forward, main + aux backward, both Adam steps) B={B}x256x256, {args.metric} loss: " + " | ".join(parts))
     for row in eb_rows(dev, args.iters, args.rounds, args.batches):
         emit(row)
     if args.out:
